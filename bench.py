@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: NMF outer iterations / second, HALS and MU beta=1, 65536 x 8192, rank 64.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows M --cols N --rank R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows M --cols N --rank R] [--dump-outputs DIR]
 
 One "step" = one HALS outer iteration + one MU (beta=1) outer iteration (U update, V update, cost
 each), every one on its own resident factor state.  `value` = 2K / T outer iterations per second
@@ -51,7 +51,15 @@ def parse_args():
     p.add_argument("--no-parity-n1", action="store_true", help="skip the sharded-vs-single-GPU self-check (N > 1)")
     p.add_argument("--c3-parity-full", action="store_true",
                    help="run the single-GPU self-check of C3 also when the matrix has more than 2^31 elements")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what they computed as DIR/<name>.npy: per rule (hals, mu) the factors U "
+                        "(m x r) and V (r x n) and the costs of the timed iterations (see dump_outputs for the size cap)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 def ncu_traffic(phase):
@@ -354,6 +362,42 @@ def parity_vs_single_gpu(args, dev, world, rank, X_full, U0, V0_full, sharded_co
     return out
 
 
+DUMP_BYTES = 63 * 10 ** 6      # array data of --dump-outputs: with the .npy headers, the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of `arrays` (name -> float32 / float64 numpy array) as out_dir/<name>.npy.  If they add up to more
+    than DUMP_BYTES, every matrix keeps the same fraction of its longer axis (rows of U, columns of V), chosen by a fixed seed,
+    so that two runs with the same arguments write the same entries."""
+    os.makedirs(out_dir, exist_ok=True)
+    mats = sum(a.nbytes for a in arrays.values() if a.ndim == 2)
+    rest = sum(a.nbytes for a in arrays.values() if a.ndim != 2)
+    keep = min(1.0, (DUMP_BYTES - rest) / mats) if mats else 1.0
+    for name, a in arrays.items():
+        if keep < 1.0 and a.ndim == 2:
+            axis = 0 if a.shape[0] >= a.shape[1] else 1
+            idx = np.sort(np.random.RandomState(0).choice(a.shape[axis], max(1, int(a.shape[axis] * keep)), replace=False))
+            a = np.take(a, idx, axis=axis)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def timed_outputs(states, costs, fused, world):
+    """What a caller of the timed path receives for each rule: U (m x r), V (r x n) and the costs of the timed iterations.
+    Column-sharded runs gather the column blocks of V (every rank must call this)."""
+    import torch.distributed as dist
+    out = {}
+    for rule, st in states.items():
+        U, V = st.factors() if fused else (st.U, st.V)
+        V = V.cpu().numpy()
+        if world > 1:
+            blocks = [None] * world
+            dist.all_gather_object(blocks, V)
+            V = np.concatenate(blocks, axis=1)
+        out[f"{rule}_U"], out[f"{rule}_V"] = U.cpu().numpy(), V
+        out[f"{rule}_costs"] = np.asarray(costs[rule], dtype=np.float64)
+    return out
+
+
 def main():
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -444,6 +488,10 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms = float(t.item())
     value = 2.0 * args.steps / (total_ms / 1e3)
+    if args.dump_outputs:
+        outputs = timed_outputs(states, {"hals": c1, "mu": c2}, fused, world)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
 
     # ---- per-phase breakdown and roofline of the dominant kernel ----
     phases = {}
