@@ -40,6 +40,8 @@ typedef enum {
 /* flags of nnfac_hals_nnls */
 #define NNFAC_HALS_NORMALIZE 1u /* nnls.py:179-185 */
 #define NNFAC_HALS_NONZERO 2u   /* nnls.py:173-177 */
+#define NNFAC_HALS_NO_TC 4u     /* fp32: skip the tensor-core sweep (its step operand is a bf16 hi/lo split); the CUDA-core sweeps
+                                 * ignore this bit */
 
 typedef struct nnfac_ctx nnfac_ctx; /* per-device workspace + launch limits; not thread-safe.  Scratch shared by several
                                      * kernels is guarded: a call on another stream than the last user of the same
@@ -253,6 +255,16 @@ int nnfac_nmf_plan_create_in(nnfac_ctx* ctx, int64_t m, int64_t n, int r, void* 
 int nnfac_nmf_plan_bytes_sided(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, size_t* bytes);
 int nnfac_nmf_plan_create_sided(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, void* workspace, size_t workspace_bytes,
                                 void* stream, nnfac_nmf_plan** out);
+/* Plans with `planes` bf16 planes per value (every other create / bytes call means planes = 2):
+ *   2: hi + lo, 16 significant bits, products of 3 MMAs;
+ *   3: hi = RN(x), mid = RN(x - hi), lo = RN(x - hi - mid): hi + mid + lo == x for every finite fp32 x whose lo does not
+ *      underflow (above 2^128 - 2^119, where RN(x) would overflow bf16, hi is rounded toward zero instead), products of the six terms down to order 2^-16 (fp32 accumulation).  Rank <= 64; 6 bytes per element and
+ *      orientation.  Ingest (load_x*), set_factor, cross, fused (mode 1 after enable_f32, whose copies are then the caller's
+ *      values), reduce and info cover it; mu_finish, hals_solve, set_factor_gathered / _pulled, set_krao*, set_push and views
+ *      return NNFAC_ERR_UNSUPPORTED without writing anything (apply or solve on a copy, then set_factor). */
+int nnfac_nmf_plan_bytes_planes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, int planes, size_t* bytes);
+int nnfac_nmf_plan_create_planes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, int planes, void* workspace,
+                                 size_t workspace_bytes, void* stream, nnfac_nmf_plan** out);
 /* View plans: the unfolding of another mode of the C-order tensor whose mode-0 unfolding `base` holds (I_0 x rest, rest % 64 == 0),
  * addressed in place through TMA maps over the SAME planes -- the reference copies the tensor once per mode (ntf.py:309-311).
  * The tensor is read as (left, I, right); the view is the I x (left*right) unfolding of the middle axis: the last mode
@@ -269,7 +281,7 @@ int nnfac_nmf_plan_load_x(nnfac_nmf_plan* plan, const float* X, int64_t ldx, voi
  * upload of X with its ingest; call nnfac_nmf_plan_load_x_done once after the last slab. */
 int nnfac_nmf_plan_load_x_rows(nnfac_nmf_plan* plan, const float* Xrows, int64_t ldx, int64_t row0, int64_t rows, void* stream);
 int nnfac_nmf_plan_load_x_done(nnfac_nmf_plan* plan, void* stream);
-/* Optional fp32 copies of X and X^T (= hi + lo of the planes) in a caller-owned, 256-byte aligned workspace: the beta = 1
+/* Optional fp32 copies of X and X^T (= hi + lo of the planes; hi + mid + lo of a 3-plane plan, which needs them for mode 1) in a caller-owned, 256-byte aligned workspace: the beta = 1
  * fused pass then reads x from fp32 instead of reconstructing it from two bf16 planes (3 instructions per element fewer).
  * Call after the ingest; the workspace must outlive the plan. */
 int nnfac_nmf_plan_f32_bytes(const nnfac_nmf_plan* plan, size_t* bytes);

@@ -47,7 +47,7 @@ extern "C" int nnfac_hals_nnls(nnfac_ctx* ctx, int dtype, const void* UtM, int64
   if (r > 128 || force_general)       // beyond the specialised kernels (the reference has no rank limit)
     return nnfac_sweep_general(ctx, dtype, UtM, ld_utm, UtU, ld_utu, V, ld_v, r, n, maxiter, delta, sparsity, flags, result, st);
   const int rp = r <= 16 ? 16 : r <= 32 ? 32 : r <= 64 ? 64 : 128;
-  if (dtype == NNFAC_F32 && flags == 0) {
+  if (dtype == NNFAC_F32 && flags == 0) {   // (NNFAC_HALS_NO_TC makes flags != 0: no tensor-core sweep)
     // tensor-core blocked sweep when the shape fits (rank <= 64, n <= 512 columns per SM); NNFAC_SWEEP=fma disables it
     static const bool force_fma = getenv("NNFAC_SWEEP") && !strcmp(getenv("NNFAC_SWEEP"), "fma");
     if (!force_fma) {

@@ -230,4 +230,14 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
   lo = __float2bfloat16_rn(x - __bfloat162float(hi));
 }
 
+// Three planes: hi + mid + lo == x exactly for every finite x whose lo does not underflow bf16 (24 significant bits).  Above
+// 2^128 - 2^119 round-to-nearest would give hi = inf: hi is then rounded toward zero (the largest finite bf16) instead.
+__device__ __forceinline__ void split3_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& mid, __nv_bfloat16& lo) {
+  hi = __float2bfloat16_rn(x);
+  if (isinf(__bfloat162float(hi)) && isfinite(x)) hi = __float2bfloat16_rz(x);
+  const float r = x - __bfloat162float(hi);     // exact
+  mid = __float2bfloat16_rn(r);
+  lo = __float2bfloat16_rn(r - __bfloat162float(mid));
+}
+
 }  // namespace tc

@@ -42,14 +42,20 @@ constexpr int DRAIN = 2;             // stages per TMEM accumulation chain of th
 // Per padded rank RK (64 or 128).  RK = 128 (ranks 65..128, MODE_RES only): the factor slab of a stage is two 64-rank
 // atoms per plane (64 KiB stages, 3 of them), the contraction GEMM is 128 wide, and the rows of the aligned factor go
 // global -> registers -> tensor memory (no 64 KiB staging buffer); tensor memory: D1 2 x 64 | D2 2 x 128 | A1 128.
-template <int RK>
+//
+// PLANES = 3 (rank <= 64): X, the factor slabs and A1 are hi/mid/lo planes, every product is six MMAs (five for the ratio tile
+// of MU, which stays hi/lo).  Residual pass: stages of 3 x 16 KiB X + 3 x 8 KiB slab = 72 KiB, two of them after the 48 KiB A1
+// staging buffer.  beta = 1 (X from its fp32 copy): 56 KiB stages, three of them; tensor memory D1 2 x 64 | D2 2 x 64 | A1 96 |
+// Q 128 = 480 columns (ND1 = 2: three model-tile buffers would need 544).
+template <int RK, int PLANES = 2, bool XF32 = false>
 struct Cfg {
   static constexpr int KR = RK / 64;                                              // 64-rank atoms
   static constexpr uint32_t FK_BYTES = (uint32_t)KR * 64 * BK * sizeof(bf16);     // one plane of the slab: 64 columns of X x RK ranks
-  static constexpr uint32_t STAGE_BYTES = 2 * X_BYTES + 2 * FK_BYTES;             // 48 / 64 KiB
-  static constexpr int FSTAGES = RK == 64 ? 4 : 3;
-  static constexpr int ND1 = RK == 64 ? 3 : 2;   // model-tile buffers in tensor memory: the model GEMM runs up to ND1 - 1 stages ahead of the transform
-  static constexpr uint32_t A1_BYTES = RK == 64 ? 2 * X_BYTES : 0;
+  static constexpr uint32_t XB = (PLANES == 3 && !XF32 ? 3 : 2) * X_BYTES;        // X part of a stage (XF32: one fp32 tile = 2 x 16 KiB)
+  static constexpr uint32_t STAGE_BYTES = XB + PLANES * FK_BYTES;                 // 48 / 64 KiB (3 planes: 72 / 56 KiB)
+  static constexpr int FSTAGES = PLANES == 3 ? (XF32 ? 3 : 2) : RK == 64 ? 4 : 3;
+  static constexpr int ND1 = PLANES == 3 && XF32 ? 2 : RK == 64 ? 3 : 2;   // model-tile buffers in tensor memory: the model GEMM runs up to ND1 - 1 stages ahead of the transform
+  static constexpr uint32_t A1_BYTES = RK == 64 ? PLANES * X_BYTES : 0;
   static constexpr int CWD = RK / NSP;           // D2 columns per transform thread
   static constexpr size_t SMEM = A1_BYTES + (size_t)FSTAGES * STAGE_BYTES + 512;
 };
@@ -79,21 +85,40 @@ __device__ __forceinline__ float lg2_approx(float x) {   // MUFU.LG2 without the
   asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
+// g(q) = q ln q - q + 1 >= 0, so that KL(x | k) = k g(x / k) element by element: a sum of non-negative terms, accurate also when
+// x / k is within 1e-3 of 1 (series of g in d = q - 1 there; the cost of the 3-plane beta = 1 pass).  q = 0 (x = 0) gives 1.
+__device__ __forceinline__ float kl_g(float q) {
+  const float d = q - 1.f;
+  if (fabsf(d) < 0.0625f) {
+    float c = fmaf(d, -1.f / 42.f, 1.f / 30.f);
+    c = fmaf(d, c, -1.f / 20.f);
+    c = fmaf(d, c, 1.f / 12.f);
+    c = fmaf(d, c, -1.f / 6.f);
+    c = fmaf(d, c, 0.5f);
+    return d * d * c;
+  }
+  return fmaf(q, lg2_approx(q + 1e-30f) * 0.6931471805599453f, -d);
+}
 __device__ __forceinline__ float bf_lo(uint32_t w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
 
-template <int MODE, bool COST, bool XF32, int RK>
+// map_xm / map_fkm / map_a1m: the middle planes (PLANES = 3 only).
+template <int MODE, bool COST, bool XF32, int RK, int PLANES = 2>
 __global__ void __launch_bounds__(FUSED_THREADS, 1)
 tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constant__ CUtensorMap map_xl,
                 const __grid_constant__ CUtensorMap map_fkh, const __grid_constant__ CUtensorMap map_fkl,
                 const __grid_constant__ CUtensorMap map_a1h, const __grid_constant__ CUtensorMap map_a1l,
-                const FusedParams p) {
-  using C = Cfg<RK>;
+                const FusedParams p, const __grid_constant__ CUtensorMap map_xm, const __grid_constant__ CUtensorMap map_fkm,
+                const __grid_constant__ CUtensorMap map_a1m) {
+  using C = Cfg<RK, PLANES, PLANES == 3 && XF32>;
   static_assert(RK == 64 || (MODE == MODE_RES && !XF32), "rank 65..128: residual + cross-product pass only");
+  static_assert(PLANES == 2 || (RK == 64 && (MODE == MODE_RES) != XF32), "3 planes: rank <= 64; beta = 1 reads X from its fp32 copy");
   constexpr int FSTAGES = C::FSTAGES, ND1 = C::ND1, CWD = C::CWD;
-  constexpr uint32_t FK_BYTES = C::FK_BYTES, STAGE_BYTES = C::STAGE_BYTES, A1_BYTES = C::A1_BYTES;
+  // 3 planes: one stage per contraction chain (24 MMAs, as many as two stages of the 2-plane products), drained two stages late
+  constexpr int DRAIN_P = PLANES == 3 ? 1 : DRAIN;
+  constexpr uint32_t FK_BYTES = C::FK_BYTES, STAGE_BYTES = C::STAGE_BYTES, A1_BYTES = C::A1_BYTES, XB = C::XB;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* a1 = smem;                                   // [hi | lo]  (RK = 64 only)
+  uint8_t* a1 = smem;                                   // [hi | lo (| mid)]  (RK = 64 only)
   uint8_t* ring = smem + A1_BYTES;
   uint64_t* bars = reinterpret_cast<uint64_t*>(ring + (size_t)FSTAGES * STAGE_BYTES);
   uint64_t* full = bars;                 // [4]
@@ -117,6 +142,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
     tc::prefetch_tmap(&map_xh); tc::prefetch_tmap(&map_xl);
     tc::prefetch_tmap(&map_fkh); tc::prefetch_tmap(&map_fkl);
     if (RK == 64) { tc::prefetch_tmap(&map_a1h); tc::prefetch_tmap(&map_a1l); }
+    if (PLANES == 3) { if (!XF32) tc::prefetch_tmap(&map_xm); tc::prefetch_tmap(&map_fkm); tc::prefetch_tmap(&map_a1m); }
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < FSTAGES; ++s) { tc::mbar_init(&full[s], 1); tc::mbar_init(&empty[s], NWT + 1); }
@@ -132,8 +158,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
   __syncthreads();
   tc::tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // tensor-memory map (columns): D1 ND1 x 64 | D2 2 x RK | A1 hi RK/2 + lo RK/2 | Q 2 x (hi 32 + lo 32) (MU)  (512 in all)
-  const uint32_t D1 = tmem_base, D2 = tmem_base + 64 * ND1, A1T = D2 + 2 * RK, QT = A1T + RK;
+  // tensor-memory map (columns): D1 ND1 x 64 | D2 2 x RK | A1 hi RK/2 + lo RK/2 (+ mid RK/2) | Q 2 x (hi 32 + lo 32) (MU)  (512 in all)
+  const uint32_t D1 = tmem_base, D2 = tmem_base + 64 * ND1, A1T = D2 + 2 * RK, QT = A1T + PLANES * (RK / 2);
   const int S = p.stages_per_unit;
 
   if (warp == 0 && lane == 0) {
@@ -148,6 +174,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         tc::mbar_arrive_expect_tx(a1_full, A1_BYTES);
         tc::tma_load_2d_hint(a1, &map_a1h, a1_full, 0, row0, tc::kEvictLast);
         tc::tma_load_2d_hint(a1 + X_BYTES, &map_a1l, a1_full, 0, row0, tc::kEvictLast);
+        if (PLANES == 3) tc::tma_load_2d_hint(a1 + 2 * X_BYTES, &map_a1m, a1_full, 0, row0, tc::kEvictLast);
       }
       for (int ks = 0; ks < S; ++ks) {
         tc::mbar_wait(&empty[stage], phase ^ 1);
@@ -157,10 +184,12 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         // XF32: map_xh is the fp32 copy of X; the two 16 KiB halves of the tile are its columns [c, c+32) and [c+32, c+64)
         tc::tma_load_2d_hint(st, &map_xh, &full[stage], c, row0, tc::kEvictFirst);
         tc::tma_load_2d_hint(st + X_BYTES, XF32 ? &map_xh : &map_xl, &full[stage], XF32 ? c + 32 : c, row0, tc::kEvictFirst);
+        if (PLANES == 3 && !XF32) tc::tma_load_2d_hint(st + 2 * X_BYTES, &map_xm, &full[stage], c, row0, tc::kEvictFirst);
 #pragma unroll
         for (int kr = 0; kr < C::KR; ++kr) {   // 64 columns of X x 64 ranks per box
-          tc::tma_load_2d_hint(st + 2 * X_BYTES + kr * 8192, &map_fkh, &full[stage], kr * 64, c, tc::kEvictLast);
-          tc::tma_load_2d_hint(st + 2 * X_BYTES + FK_BYTES + kr * 8192, &map_fkl, &full[stage], kr * 64, c, tc::kEvictLast);
+          tc::tma_load_2d_hint(st + XB + kr * 8192, &map_fkh, &full[stage], kr * 64, c, tc::kEvictLast);
+          tc::tma_load_2d_hint(st + XB + FK_BYTES + kr * 8192, &map_fkl, &full[stage], kr * 64, c, tc::kEvictLast);
+          if (PLANES == 3) tc::tma_load_2d_hint(st + XB + 2 * FK_BYTES + kr * 8192, &map_fkm, &full[stage], kr * 64, c, tc::kEvictLast);
         }
         if (++stage == FSTAGES) { stage = 0; phase ^= 1; }
       }
@@ -182,8 +211,27 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         tc::tcgen05_fence_after();
         if (tc::elect_one()) {
           const uint32_t sb = tc::smem_u32(ring + (size_t)st1 * STAGE_BYTES);
-          const uint64_t fkh = tc::umma_desc_k_sw128(sb + 2 * X_BYTES), fkl = tc::umma_desc_k_sw128(sb + 2 * X_BYTES + FK_BYTES);
+          const uint64_t fkh = tc::umma_desc_k_sw128(sb + XB), fkl = tc::umma_desc_k_sw128(sb + XB + FK_BYTES);
           const uint32_t d = D1 + (uint32_t)b1 * 64;
+          if constexpr (PLANES == 3) {
+            // the five small products over the whole contraction first, the hi * hi ones last (truncating accumulation)
+            const uint64_t fkm = tc::umma_desc_k_sw128(sb + XB + 2 * FK_BYTES);
+            const uint32_t ah = A1T, al = A1T + RK / 2, am = A1T + RK;
+#pragma unroll
+            for (int k = 0; k < RK / UMMA_K; ++k) {
+              if (k < ksteps) {
+                const uint64_t bo = (uint64_t)((k & 3) * 2);
+                tc::umma_bf16_ts(d, al + 8 * k, fkh + bo, idesc1, k != 0);   // order 2^-16
+                tc::umma_bf16_ts(d, am + 8 * k, fkm + bo, idesc1, true);
+                tc::umma_bf16_ts(d, ah + 8 * k, fkl + bo, idesc1, true);
+                tc::umma_bf16_ts(d, am + 8 * k, fkh + bo, idesc1, true);     // order 2^-8
+                tc::umma_bf16_ts(d, ah + 8 * k, fkm + bo, idesc1, true);
+              }
+            }
+#pragma unroll
+            for (int k = 0; k < RK / UMMA_K; ++k)
+              if (k < ksteps) tc::umma_bf16_ts(d, ah + 8 * k, fkh + (uint64_t)((k & 3) * 2), idesc1, true);
+          } else {
 #pragma unroll
           for (int k = 0; k < RK / UMMA_K; ++k) {
             if (k < ksteps) {
@@ -192,6 +240,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
               tc::umma_bf16_ts(d, A1T + RK / 2 + 8 * k, fkh + bo, idesc1, true);
               tc::umma_bf16_ts(d, A1T + 8 * k, fkl + bo, idesc1, true);
             }
+          }
           }
           tc::umma_commit(&d1_full[b1]);
           if (i == S - 1) tc::umma_commit(a1t_free);
@@ -209,8 +258,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
     int b2 = 0; uint32_t b2_phase = 0;      // D2 buffer
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
       for (int j = 0; j < S; ++j) {
-        const bool chain_start = (j % DRAIN) == 0;
-        const bool chain_end = ((j + 1) % DRAIN) == 0 || j == S - 1;
+        const bool chain_start = (j % DRAIN_P) == 0;
+        const bool chain_end = ((j + 1) % DRAIN_P) == 0 || j == S - 1;
         tc::mbar_wait(&full[st2], ph2);
         if (MODE == MODE_MU) tc::mbar_wait(&q_ready[qb], qb_phase);
         if (chain_start) tc::mbar_wait(&d2_empty[b2], b2_phase ^ 1);
@@ -220,9 +269,37 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           const uint64_t xh = tc::umma_desc_k_sw128(sb), xl = tc::umma_desc_k_sw128(sb + X_BYTES);
           // B operand = the SAME 64-column slab of the other factor that the model GEMM reads K-major, addressed
           // MN-major here (rank contiguous = N, columns = K): no second copy of the factor travels through L2
-          const uint64_t fnh = tc::umma_desc_mn_sw128(sb + 2 * X_BYTES);
-          const uint64_t fnl = tc::umma_desc_mn_sw128(sb + 2 * X_BYTES + FK_BYTES);
+          const uint64_t fnh = tc::umma_desc_mn_sw128(sb + XB);
+          const uint64_t fnl = tc::umma_desc_mn_sw128(sb + XB + FK_BYTES);
           const uint32_t d = D2 + (uint32_t)b2 * RK;
+          if constexpr (PLANES == 3) {
+            // small products of the stage first, hi * hi last (see the model GEMM)
+            const uint64_t fnm = tc::umma_desc_mn_sw128(sb + XB + 2 * FK_BYTES);
+            const uint64_t xm = tc::umma_desc_k_sw128(sb + 2 * X_BYTES);
+#pragma unroll
+            for (int k = 0; k < BK / UMMA_K; ++k) {
+              const uint64_t ko = (uint64_t)(k * 2), kb = (uint64_t)(k * 128);
+              const bool acc0 = !(chain_start && k == 0);
+              if (MODE == MODE_MU) {
+                const uint32_t qa = QT + (uint32_t)qb * 64 + 8 * k;   // ratio tile: hi at qa, lo at qa + 32
+                tc::umma_bf16_ts(d, qa, fnl + kb, idesc2, acc0);        // order 2^-16
+                tc::umma_bf16_ts(d, qa + 32, fnm + kb, idesc2, true);
+                tc::umma_bf16_ts(d, qa, fnm + kb, idesc2, true);        // order 2^-8
+                tc::umma_bf16_ts(d, qa + 32, fnh + kb, idesc2, true);
+              } else {
+                tc::umma_bf16(d, xl + ko, fnh + kb, idesc2, acc0);      // order 2^-16
+                tc::umma_bf16(d, xm + ko, fnm + kb, idesc2, true);
+                tc::umma_bf16(d, xh + ko, fnl + kb, idesc2, true);
+                tc::umma_bf16(d, xm + ko, fnh + kb, idesc2, true);      // order 2^-8
+                tc::umma_bf16(d, xh + ko, fnm + kb, idesc2, true);
+              }
+            }
+#pragma unroll
+            for (int k = 0; k < BK / UMMA_K; ++k) {
+              if (MODE == MODE_MU) tc::umma_bf16_ts(d, QT + (uint32_t)qb * 64 + 8 * k, fnh + (uint64_t)(k * 128), idesc2, true);
+              else tc::umma_bf16(d, xh + (uint64_t)(k * 2), fnh + (uint64_t)(k * 128), idesc2, true);
+            }
+          } else {
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
             const uint64_t ko = (uint64_t)(k * 2);            // A (K-major): 16 bf16 = 32 B inside the 128 B row
@@ -237,6 +314,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
               tc::umma_bf16(d, xl + ko, fnh + kb, idesc2, true);
               tc::umma_bf16(d, xh + ko, fnl + kb, idesc2, true);
             }
+          }
           }
           tc::umma_commit(&empty[st2]);
           if (MODE == MODE_MU) tc::umma_commit(&q_free[qb]);
@@ -271,7 +349,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         a1_phase ^= 1;
         tc::tcgen05_fence_after();
 #pragma unroll
-        for (int pl = 0; pl < 2; ++pl) {
+        for (int pl = 0; pl < PLANES; ++pl) {
           uint32_t w[4 * NCHK];
 #pragma unroll
           for (int cc = 0; cc < NCHK; ++cc) {
@@ -390,6 +468,16 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
             const uint4 h4 = *reinterpret_cast<const uint4*>(xh + off);
             const uint4 l4 = *reinterpret_cast<const uint4*>(xl + off);
             const uint32_t hw[4] = {h4.x, h4.y, h4.z, h4.w}, lw[4] = {l4.x, l4.y, l4.z, l4.w};
+            if constexpr (PLANES == 3) {
+              // x = hi + (mid + lo): mid + lo is the exact remainder x - hi, so x is the caller's fp32 value (hi + mid can overflow
+              // near the largest float)
+              const uint4 m4 = *reinterpret_cast<const uint4*>(xl + X_BYTES + off);
+              const uint32_t mw[4] = {m4.x, m4.y, m4.z, m4.w};
+#pragma unroll
+              for (int w = 0; w < 4; ++w)
+                xv[w] = __fadd2_rn(make_float2(bf_lo(hw[w]), bf_hi(hw[w])),
+                                   __fadd2_rn(make_float2(bf_lo(mw[w]), bf_hi(mw[w])), make_float2(bf_lo(lw[w]), bf_hi(lw[w]))));
+            } else {
 #pragma unroll
             for (int w = 0; w < 4; ++w)
 #if FUSED_PACKED
@@ -397,6 +485,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #else
               xv[w] = make_float2(bf_lo(hw[w]) + bf_lo(lw[w]), bf_hi(hw[w]) + bf_hi(lw[w]));
 #endif
+            }
           }
 #if FUSED_PACKED
 #pragma unroll
@@ -482,17 +571,22 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           if (DEFER) {
 #pragma unroll
             for (int e = 0; e < 4 * NCHK; ++e) {
-              const float2 qt = __fadd2_rn(qs[DEFER ? e : 0], tiny2);
-              acc2 = __ffma2_rn(xs[DEFER ? e : 0], make_float2(lg2_approx(qt.x), lg2_approx(qt.y)), acc2);
+              if constexpr (PLANES == 3) {     // the KL terms themselves, k g(q): no cancellation against sum(x) - sum(k)
+                const float2 k2 = make_float2(__uint_as_float(kk[2 * e]), __uint_as_float(kk[2 * e + 1]));
+                acc2 = __ffma2_rn(k2, make_float2(kl_g(qs[DEFER ? e : 0].x), kl_g(qs[DEFER ? e : 0].y)), acc2);
+              } else {
+                const float2 qt = __fadd2_rn(qs[DEFER ? e : 0], tiny2);
+                acc2 = __ffma2_rn(xs[DEFER ? e : 0], make_float2(lg2_approx(qt.x), lg2_approx(qt.y)), acc2);
+              }
             }
             flush_cost();
           }
         }
         // drain with a lag of one more stage: chain (i-3)/2 ended with stage i-2, its GEMMs have retired by now, and
         // its TMEM buffer is only needed again by the chain that starts with stage i+1
-        if (i >= 3 && (i & 1)) { drain_chain(); ++drained; }
+        if (DRAIN_P == 2 ? (i >= 3 && (i & 1)) : i >= 2) { drain_chain(); ++drained; }
       }
-      for (; drained < (S + DRAIN - 1) / DRAIN; ++drained) drain_chain();
+      for (; drained < (S + DRAIN_P - 1) / DRAIN_P; ++drained) drain_chain();
       if (p.push_chunk > 0) {
         const int64_t row0 = (int64_t)tile * TILE_ROWS;
         const int q = (int)(row0 / p.push_chunk);                          // owner of these rows of U (warp-uniform)
@@ -538,13 +632,15 @@ struct PeerG {                      // PULL: slice s of the factor lives in p[s]
   unsigned long long seq;
 };
 
-template <bool APPLY, int RK, bool PULL>
+// PLANES = 3: the middle planes go to fm / rowm.
+template <bool APPLY, int RK, bool PULL, int PLANES = 2>
 __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restrict__ partial, int splits, int r, int r_pad, int64_t R,
                                                             int64_t ldp, const float* __restrict__ F_in, int64_t ld_in,
                                                             int64_t in_chunk, int64_t in_slab, const PeerG G,
                                                             const float* __restrict__ den, float floor_value, float* __restrict__ F_out,
                                                             int64_t ld_out, bf16* __restrict__ fh, bf16* __restrict__ fl, int64_t ld_plane,
-                                                            bf16* __restrict__ rowh, bf16* __restrict__ rowl) {
+                                                            bf16* __restrict__ rowh, bf16* __restrict__ rowl,
+                                                            bf16* __restrict__ fm = nullptr, bf16* __restrict__ rowm = nullptr) {
   __shared__ float tile[RK][33];
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   if (PULL && G.flags != nullptr) {
@@ -593,7 +689,13 @@ __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restr
       }
       if (F_out) F_out[(int64_t)k * ld_out + c] = f;
       bf16 h, l;
-      tc::split_bf16(f, h, l);
+      if constexpr (PLANES == 3) {
+        bf16 md;
+        tc::split3_bf16(f, h, md, l);
+        fm[(int64_t)k * ld_plane + c] = md;
+      } else {
+        tc::split_bf16(f, h, l);
+      }
       fh[(int64_t)k * ld_plane + c] = h;
       fl[(int64_t)k * ld_plane + c] = l;
     }
@@ -608,7 +710,13 @@ __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restr
       for (int h2 = 0; h2 < RK / 32; ++h2) {
         const int k = tx + 32 * h2;
         bf16 h, l;
-        tc::split_bf16(tile[k][i], h, l);
+        if constexpr (PLANES == 3) {
+          bf16 md;
+          tc::split3_bf16(tile[k][i], h, md, l);
+          rowm[cc * RK + k] = md;
+        } else {
+          tc::split_bf16(tile[k][i], h, l);
+        }
         rowh[cc * RK + k] = h;
         rowl[cc * RK + k] = l;
       }
@@ -641,13 +749,20 @@ __global__ void kl_cost_finish_kernel(const double* part, int n, const double* s
   }
 }
 
-// fp32 copy of a plane pair: out = hi + lo (exact: 16 significant bits), [rows x ld].
+// fp32 copy of a plane pair: out = hi + lo (exact: 16 significant bits), [rows x ld].  PLANES = 3: out = hi + (mid + lo),
+// the fp32 value the planes were split from (mid + lo is its exact remainder x - hi).
+template <int PLANES>
 __global__ void __launch_bounds__(256) planes_to_f32_kernel(const bf16* __restrict__ hi, const bf16* __restrict__ lo, int64_t count,
-                                                            float* __restrict__ out) {
+                                                            float* __restrict__ out, const bf16* __restrict__ mid) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x * 2;
   for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 2; i < count; i += stride) {
     const uint32_t h = *reinterpret_cast<const uint32_t*>(hi + i), l = *reinterpret_cast<const uint32_t*>(lo + i);
-    *reinterpret_cast<float2*>(out + i) = make_float2(bf_lo(h) + bf_lo(l), bf_hi(h) + bf_hi(l));
+    if constexpr (PLANES == 3) {
+      const uint32_t md = *reinterpret_cast<const uint32_t*>(mid + i);
+      *reinterpret_cast<float2*>(out + i) = make_float2(bf_lo(h) + (bf_lo(md) + bf_lo(l)), bf_hi(h) + (bf_hi(md) + bf_hi(l)));
+    } else {
+      *reinterpret_cast<float2*>(out + i) = make_float2(bf_lo(h) + bf_lo(l), bf_hi(h) + bf_hi(l));
+    }
   }
 }
 
@@ -663,6 +778,12 @@ static int finish_factor(nnfac_nmf_plan* p, int which, bool apply, const float* 
   bf16* rl = p->fused_ok ? p->rowp_l[which] : nullptr;
   PeerG none;
   memset(&none, 0, sizeof(none));
+  if (p->planes == 3) {     // plain install only (the writers that would apply or pull refuse a 3-plane plan)
+    factor_finish_kernel<false, 64, false, 3><<<grid, 256, 0, st>>>(nullptr, 0, p->r, p->r_pad, len, 0, F_in, ld_in, in_chunk, in_slab,
+        none, nullptr, 0.f, F_out, ld_out, cs->fh, cs->fl, cs->ld, rh, rl, cs->fm, p->rowp_m[which]);
+    NNFAC_LAUNCH_CHECK(p->ctx);
+    return NNFAC_OK;
+  }
 #define NNFAC_FINISH(RKV)                                                                                                          \
   do {                                                                                                                             \
     if (pulled)                                                                                                                    \
@@ -685,8 +806,9 @@ static int finish_factor(nnfac_nmf_plan* p, int which, bool apply, const float* 
 extern "C" {
 
 // fp32 copies of X for the beta = 1 fused pass (see nnfac_nmf_plan::xf): `workspace` (256-byte aligned, caller-owned,
-// >= nnfac_nmf_plan_f32_bytes) receives X and X^T as fp32; call after the ingest.  Optional: without it the pass
-// reconstructs x = hi + lo from the bf16 planes.
+// >= nnfac_nmf_plan_f32_bytes) receives X and X^T as fp32; call after the ingest.  Optional for 2-plane plans: without it
+// the pass reconstructs x = hi + lo from the bf16 planes.  A 3-plane plan's beta = 1 pass needs it; its copies are the
+// caller's fp32 values (hi + mid + lo).
 int nnfac_nmf_plan_f32_bytes(const nnfac_nmf_plan* p, size_t* bytes) {
   NNFAC_ARG(p && bytes, "nnfac_nmf_plan_f32_bytes: NULL argument");
   size_t tot = 0;
@@ -709,7 +831,8 @@ int nnfac_nmf_plan_enable_f32(nnfac_nmf_plan* p, void* workspace, size_t workspa
     p->xf[i] = (float*)base;
     const int64_t count = s->R * s->ld;                       // ld is a multiple of 64: pairs never straddle rows
     base += (((size_t)count * sizeof(float)) + 255) & ~(size_t)255;
-    planes_to_f32_kernel<<<p->ctx->sm_count * 16, 256, 0, st>>>(s->xh, s->xl, count, p->xf[i]);
+    if (p->planes == 3) planes_to_f32_kernel<3><<<p->ctx->sm_count * 16, 256, 0, st>>>(s->xh, s->xl, count, p->xf[i], s->xm);
+    else planes_to_f32_kernel<2><<<p->ctx->sm_count * 16, 256, 0, st>>>(s->xh, s->xl, count, p->xf[i], nullptr);
     NNFAC_LAUNCH_CHECK(p->ctx);
     const int rc = make_map_f32(&p->map_xf[i], p->xf[i], s->R, s->C, s->ld);
     if (rc) return rc;
@@ -735,6 +858,7 @@ int nnfac_nmf_plan_set_factor_gathered(nnfac_nmf_plan* p, int which, const float
   NNFAC_ARG(p && G && Ft_out && chunk > 0 && (which == 0 || which == 1), "nnfac_nmf_plan_set_factor_gathered: bad argument");
   const int64_t len = which == 0 ? p->m : p->n;
   NNFAC_ARG(ld_out >= len, "nnfac_nmf_plan_set_factor_gathered: leading dimension too small");
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_set_factor_gathered: writes two planes, the plan has %d", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   return finish_factor(p, which, false, G, chunk, chunk, (int64_t)p->r * chunk, nullptr, 0.f, Ft_out, ld_out, (cudaStream_t)stream);
 }
 
@@ -749,6 +873,7 @@ int nnfac_nmf_plan_set_factor_pulled(nnfac_nmf_plan* p, int which, const nnfac_x
                                      int64_t ld_out, void* stream) {
   NNFAC_ARG(p && x && Ft_out && chunk > 0 && pitch >= chunk && (which == 0 || which == 1), "nnfac_nmf_plan_set_factor_pulled: bad argument");
   NNFAC_ARG(!p->base, "nnfac_nmf_plan_set_factor_pulled: not available on a view plan");
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_set_factor_pulled: writes two planes, the plan has %d", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   const int64_t len = which == 0 ? p->m : p->n;
   const int world = nnfac_xchg_world(x);
   NNFAC_ARG(ld_out >= len && (int64_t)world * chunk >= len, "nnfac_nmf_plan_set_factor_pulled: %d slices of %lld columns do not cover %lld",
@@ -761,13 +886,14 @@ int nnfac_nmf_plan_set_factor_pulled(nnfac_nmf_plan* p, int which, const nnfac_x
 
 // HALS solve of factor `which` (nnls.py:24-198, deterministic rule) that also installs the result in the plan:
 // F_out = hals_nnls_acc(UtM, UtU, F_in) and every operand plane of F_out, written by the sweep kernel itself.
-// Returns NNFAC_ERR_UNSUPPORTED (no error text) when the shape is outside the tensor-core sweep's envelope; the caller
-// then runs nnfac_hals_nnls + nnfac_nmf_plan_set_factor.
+// Returns NNFAC_ERR_UNSUPPORTED (no error text) when the shape is outside the tensor-core sweep's envelope, or for a 3-plane plan
+// (the sweep writes two planes); the caller then runs nnfac_hals_nnls + nnfac_nmf_plan_set_factor.
 int nnfac_nmf_plan_hals_solve(nnfac_nmf_plan* p, int which, const float* UtM, int64_t ld_utm, const float* UtU, int64_t ld_utu,
                               const float* F_in, int64_t ld_in, float* F_out, int64_t ld_out, int maxiter, double delta,
                               double sparsity, double* result, void* stream) {
   NNFAC_ARG(p && UtU && F_in && F_out && result && (which == 0 || which == 1), "nnfac_nmf_plan_hals_solve: bad argument");
   NNFAC_ARG(!p->base, "nnfac_nmf_plan_hals_solve: not available on a view plan");
+  if (p->planes != 2) return NNFAC_ERR_UNSUPPORTED;
   const int64_t len = which == 0 ? p->m : p->n;
   NNFAC_ARG((!UtM || ld_utm >= len) && ld_in >= len && ld_out >= len && ld_utu >= p->r, "nnfac_nmf_plan_hals_solve: leading dimension too small");
   // UtM == NULL: the right-hand side is what the last X pass over side `which` left in the plan as split-K partials
@@ -800,6 +926,7 @@ int nnfac_nmf_plan_set_push(nnfac_nmf_plan* p, const nnfac_xchg* x, int64_t inbo
   NNFAC_ARG(p, "nnfac_nmf_plan_set_push: NULL plan");
   if (!x) { p->push_chunk = 0; return NNFAC_OK; }
   NNFAC_ARG(!p->base && p->fused_ok, "nnfac_nmf_plan_set_push: needs a plan with the fused pass");
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_set_push: not available on a 3-plane plan"); return NNFAC_ERR_UNSUPPORTED; }
   const int world = nnfac_xchg_world(x);
   const int splits = p->side[0].cp.splits;
   NNFAC_ARG(chunk > 0 && chunk % TILE_ROWS == 0 && (int64_t)world * chunk >= p->m && inbox_off >= 0,
@@ -859,6 +986,7 @@ int nnfac_nmf_plan_mu_finish(nnfac_nmf_plan* p, int which, const float* F_in, in
   const int64_t len = which == 0 ? p->m : p->n;
   NNFAC_ARG(ld_in >= len && ld_out >= len, "nnfac_nmf_plan_mu_finish: leading dimension too small");
   if (!p->fused_ok) { nnfac_set_error("nnfac_nmf_plan_mu_finish: rank %d > 128 is not covered by the fused pass", p->r); return NNFAC_ERR_UNSUPPORTED; }
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_mu_finish: writes two planes, the plan has %d (apply + set_factor)", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   return finish_factor(p, which, true, F_in, ld_in, 0, 0, den, (float)floor_value, F_out, ld_out, (cudaStream_t)stream);
 }
 
@@ -872,6 +1000,7 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
   NNFAC_ARG((p->sides >> side) & 1, "nnfac_nmf_plan_fused: this plan keeps no planes of side %d", side);
   if (!p->fused_ok) { nnfac_set_error("nnfac_nmf_plan_fused: not covered by the fused pass (rank %d > 128, or a view plan)", p->r); return NNFAC_ERR_UNSUPPORTED; }
   if (mode == 1 && p->rk != 64) { nnfac_set_error("nnfac_nmf_plan_fused: the beta = 1 pass covers rank <= 64 (rank %d)", p->r); return NNFAC_ERR_UNSUPPORTED; }
+  if (mode == 1 && p->planes == 3 && !p->xf_ready) { nnfac_set_error("nnfac_nmf_plan_fused: the beta = 1 pass of a 3-plane plan reads X from its fp32 copies (nnfac_nmf_plan_enable_f32)"); return NNFAC_ERR_UNSUPPORTED; }
   Side* s = &p->side[side];
   NNFAC_ARG(!out || ld_out >= s->R, "nnfac_nmf_plan_fused: leading dimension too small");
   cudaStream_t st = (cudaStream_t)stream;
@@ -893,9 +1022,22 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
     const size_t smem = Cfg<RKV>::SMEM;                                                                                       \
     NNFAC_CUDA(cudaFuncSetAttribute(tc_fused_kernel<M, C, XF, RKV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     tc_fused_kernel<M, C, XF, RKV><<<s->grid, FUSED_THREADS, smem, st>>>(MAPH, MAPL, p->map_row_b_h[other],                  \
-        p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp);                                               \
+        p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp, MAPH, p->map_row_b_h[other],                  \
+        p->map_row_a_h[side]);                                                                                                \
   } while (0)
-  if (mode == 0 && p->rk == 128) NNFAC_LAUNCH_FUSED(MODE_RES, true, false, 128, s->map_xh, s->map_xl);
+#define NNFAC_LAUNCH_FUSED3(M, C, XF, MAPH, MAPL)                                                                                \
+  do {                                                                                                                        \
+    const size_t smem = Cfg<64, 3, XF>::SMEM;                                                                                 \
+    NNFAC_CUDA(cudaFuncSetAttribute(tc_fused_kernel<M, C, XF, 64, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    tc_fused_kernel<M, C, XF, 64, 3><<<s->grid, FUSED_THREADS, smem, st>>>(MAPH, MAPL, p->map_row_b_h[other],                \
+        p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp, s->map_xm, p->map_row_b_m[other],             \
+        p->map_row_a_m[side]);                                                                                                \
+  } while (0)
+  if (p->planes == 3) {
+    if (mode == 0) NNFAC_LAUNCH_FUSED3(MODE_RES, true, false, s->map_xh, s->map_xl);
+    else if (fp.want_cost) NNFAC_LAUNCH_FUSED3(MODE_MU, true, true, p->map_xf[side], p->map_xf[side]);
+    else NNFAC_LAUNCH_FUSED3(MODE_MU, false, true, p->map_xf[side], p->map_xf[side]);
+  } else if (mode == 0 && p->rk == 128) NNFAC_LAUNCH_FUSED(MODE_RES, true, false, 128, s->map_xh, s->map_xl);
   else if (mode == 0) NNFAC_LAUNCH_FUSED(MODE_RES, true, false, 64, s->map_xh, s->map_xl);
   else if (p->xf_ready) {   // beta = 1: X only travels through registers -> read its fp32 copy
     if (fp.want_cost) NNFAC_LAUNCH_FUSED(MODE_MU, true, true, 64, p->map_xf[side], p->map_xf[side]);
@@ -905,13 +1047,14 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
     else NNFAC_LAUNCH_FUSED(MODE_MU, false, false, 64, s->map_xh, s->map_xl);
   }
 #undef NNFAC_LAUNCH_FUSED
+#undef NNFAC_LAUNCH_FUSED3
   NNFAC_LAUNCH_CHECK(p->ctx);
   if (out) {      // out == NULL: the split partials stay in the plan for nnfac_nmf_plan_mu_finish
     nnfac_reduce_partials(p->partial, fp.splits, p->r, p->r_pad, s->R, fp.ld_partial, out, ld_out, p->ctx->sm_count, st);
     NNFAC_LAUNCH_CHECK(p->ctx);
   }
   if (cost_out && fp.want_cost) {
-    if (mode == 0)
+    if (mode == 0 || p->planes == 3)     // 3 planes, mode 1: the pass summed the KL terms themselves
       sum_cost_parts_kernel<<<1, 32, 0, st>>>(p->cost_part, s->grid, cost_out);
     else
       kl_cost_finish_kernel<<<1, 32, 0, st>>>(p->cost_part, s->grid, p->sums, cost_out);

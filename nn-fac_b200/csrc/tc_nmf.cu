@@ -16,22 +16,31 @@
 namespace {
 using namespace tcplan;
 
-// ---- ingest: fp32 -> bf16 hi/lo planes ----------------------------------------------------------
+// ---- ingest: fp32 -> bf16 hi/lo planes (PLANES = 3: hi/mid/lo, `mid` is the middle plane) ------------------------------
+template <int PLANES>
 __global__ void split_planes_kernel(const float* __restrict__ in, int64_t ld_in, int64_t rows, int64_t cols,
-                                    bf16* __restrict__ hi, bf16* __restrict__ lo, int64_t ld_out) {
+                                    bf16* __restrict__ hi, bf16* __restrict__ lo, int64_t ld_out, bf16* __restrict__ mid) {
   const int64_t total = rows * cols;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = i / cols, c = i % cols;
     bf16 h, l;
-    tc::split_bf16(in[r * ld_in + c], h, l);
+    if constexpr (PLANES == 3) {
+      bf16 md;
+      tc::split3_bf16(in[r * ld_in + c], h, md, l);
+      mid[r * ld_out + c] = md;
+    } else {
+      tc::split_bf16(in[r * ld_in + c], h, l);
+    }
     hi[r * ld_out + c] = h;
     lo[r * ld_out + c] = l;
   }
 }
 
-// out planes hold in^T: hiT/loT are [cols x rows] with leading dimension ld_out
+// out planes hold in^T: hiT/loT (/midT) are [cols x rows] with leading dimension ld_out
+template <int PLANES>
 __global__ void split_planes_transposed_kernel(const float* __restrict__ in, int64_t ld_in, int64_t rows, int64_t cols,
-                                               bf16* __restrict__ hiT, bf16* __restrict__ loT, int64_t ld_out) {
+                                               bf16* __restrict__ hiT, bf16* __restrict__ loT, int64_t ld_out,
+                                               bf16* __restrict__ midT) {
   __shared__ float tile[32][33];
   const int64_t c0 = (int64_t)blockIdx.x * 32, r0 = (int64_t)blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -43,7 +52,13 @@ __global__ void split_planes_transposed_kernel(const float* __restrict__ in, int
     const int64_t c = c0 + i, r = r0 + threadIdx.x;
     if (r < rows && c < cols) {
       bf16 h, l;
-      tc::split_bf16(tile[threadIdx.x][i], h, l);
+      if constexpr (PLANES == 3) {
+        bf16 md;
+        tc::split3_bf16(tile[threadIdx.x][i], h, md, l);
+        midT[c * ld_out + r] = md;
+      } else {
+        tc::split_bf16(tile[threadIdx.x][i], h, l);
+      }
       hiT[c * ld_out + r] = h;
       loT[c * ld_out + r] = l;
     }
@@ -54,16 +69,18 @@ __global__ void split_planes_transposed_kernel(const float* __restrict__ in, int
 // 1: the planes hold X^T -- contraction index = plane row, the 128 output rows of a tile are contiguous in memory -- and the
 // tile is an MN-major UMMA operand (two 64-wide M blocks per plane, each a 64 x 64 TMA box): the LAST mode of a C-order tensor;
 // 2: as 0 through a 3-D map, k-block b = (slab b / kb_per_slab, offset 64 (b % kb_per_slab)): a MIDDLE mode.
-template <int MAX_RPAD, int AMODE>
+// PLANES = 3 (AMODE 0 only): X and the factor as hi/mid/lo planes (map_xm / map_fm: the middle ones), six MMAs per k step.
+template <int MAX_RPAD, int AMODE, int PLANES>
 __global__ void __launch_bounds__(NTHREADS, 1)
 tc_cross_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constant__ CUtensorMap map_xl,
                 const __grid_constant__ CUtensorMap map_fh, const __grid_constant__ CUtensorMap map_fl,
-                const CrossParams p) {
+                const CrossParams p, const __grid_constant__ CUtensorMap map_xm, const __grid_constant__ CUtensorMap map_fm) {
+  static_assert(PLANES == 2 || (PLANES == 3 && AMODE == 0 && MAX_RPAD == 64), "3 planes: rank <= 64, rows K-major");
   extern __shared__ __align__(1024) uint8_t smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t x_bytes = TILE_ROWS * BK * sizeof(bf16);        // 16 KiB
   const uint32_t f_bytes = (uint32_t)p.r_pad * BK * sizeof(bf16);
-  const uint32_t stage_bytes = 2 * x_bytes + 2 * f_bytes;
+  const uint32_t stage_bytes = PLANES * (x_bytes + f_bytes);   // [X planes | factor planes], plane order hi, lo(, mid)
   uint8_t* ring = smem;
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)p.num_stages * stage_bytes);
   uint64_t* empty = full + p.num_stages;
@@ -76,6 +93,7 @@ tc_cross_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 
   if (warp == 0 && lane == 0) {
     tc::prefetch_tmap(&map_xh); tc::prefetch_tmap(&map_xl); tc::prefetch_tmap(&map_fh); tc::prefetch_tmap(&map_fl);
+    if (PLANES == 3) { tc::prefetch_tmap(&map_xm); tc::prefetch_tmap(&map_fm); }
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < p.num_stages; ++s) { tc::mbar_init(&full[s], 1); tc::mbar_init(&empty[s], 1); }
@@ -103,6 +121,7 @@ tc_cross_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         if (AMODE == 0) {
           tc::tma_load_2d_hint(st, &map_xh, &full[stage], c, row0, tc::kEvictFirst);
           tc::tma_load_2d_hint(st + x_bytes, &map_xl, &full[stage], c, row0, tc::kEvictFirst);
+          if (PLANES == 3) tc::tma_load_2d_hint(st + 2 * x_bytes, &map_xm, &full[stage], c, row0, tc::kEvictFirst);
         } else if (AMODE == 1) {
 #pragma unroll
           for (int mb = 0; mb < 2; ++mb) {             // M block mb: output rows row0 + 64 mb .. + 63, contraction rows c .. c + 63
@@ -114,8 +133,9 @@ tc_cross_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           tc::tma_load_3d_hint(st, &map_xh, &full[stage], off, row0, slab, tc::kEvictFirst);
           tc::tma_load_3d_hint(st + x_bytes, &map_xl, &full[stage], off, row0, slab, tc::kEvictFirst);
         }
-        tc::tma_load_2d_hint(st + 2 * x_bytes, &map_fh, &full[stage], c, 0, tc::kEvictLast);
-        tc::tma_load_2d_hint(st + 2 * x_bytes + f_bytes, &map_fl, &full[stage], c, 0, tc::kEvictLast);
+        tc::tma_load_2d_hint(st + PLANES * x_bytes, &map_fh, &full[stage], c, 0, tc::kEvictLast);
+        tc::tma_load_2d_hint(st + PLANES * x_bytes + f_bytes, &map_fl, &full[stage], c, 0, tc::kEvictLast);
+        if (PLANES == 3) tc::tma_load_2d_hint(st + 3 * x_bytes + 2 * f_bytes, &map_fm, &full[stage], c, 0, tc::kEvictLast);
         if (++stage == p.num_stages) { stage = 0; phase ^= 1; }
       }
     }
@@ -138,6 +158,29 @@ tc_cross_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           tc::tcgen05_fence_after();
           if (tc::elect_one()) {
             const uint32_t st = tc::smem_u32(ring + (size_t)stage * stage_bytes);
+            if constexpr (PLANES == 3) {
+              // the five small products of the whole stage first, then the four hi*hi: the truncating adds of the small terms
+              // then act on a partial sum 2^8 smaller than the result
+              const uint32_t fb = st + 3 * x_bytes;
+#pragma unroll
+              for (int k = 0; k < BK / UMMA_K; ++k) {
+                const uint32_t koff = k * UMMA_K * sizeof(bf16);
+                const uint64_t xh = tc::umma_desc_k_sw128(st + koff), xl = tc::umma_desc_k_sw128(st + x_bytes + koff);
+                const uint64_t xm = tc::umma_desc_k_sw128(st + 2 * x_bytes + koff);
+                const uint64_t fh = tc::umma_desc_k_sw128(fb + koff), fl = tc::umma_desc_k_sw128(fb + f_bytes + koff);
+                const uint64_t fm = tc::umma_desc_k_sw128(fb + 2 * f_bytes + koff);
+                tc::umma_bf16(d, xl, fh, idesc, (ks != ks0) || (k != 0));   // order 2^-16
+                tc::umma_bf16(d, xm, fm, idesc, true);
+                tc::umma_bf16(d, xh, fl, idesc, true);
+                tc::umma_bf16(d, xm, fh, idesc, true);                      // order 2^-8
+                tc::umma_bf16(d, xh, fm, idesc, true);
+              }
+#pragma unroll
+              for (int k = 0; k < BK / UMMA_K; ++k) {
+                const uint32_t koff = k * UMMA_K * sizeof(bf16);
+                tc::umma_bf16(d, tc::umma_desc_k_sw128(st + koff), tc::umma_desc_k_sw128(fb + koff), idesc, true);
+              }
+            } else {
 #pragma unroll
             for (int k = 0; k < BK / UMMA_K; ++k) {
               const uint32_t koff = k * UMMA_K * sizeof(bf16);   // 32 B inside the 128 B swizzle row
@@ -149,6 +192,7 @@ tc_cross_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
               tc::umma_bf16(d, xh, fh, idesc, (ks != ks0) || (k != 0));
               tc::umma_bf16(d, xl, fh, idesc, true);
               tc::umma_bf16(d, xh, fl, idesc, true);
+            }
             }
             tc::umma_commit(&empty[stage]);                      // frees the smem slot when the MMAs retire
             if (ks == ks1 - 1) tc::umma_commit(&acc_full[acc]);  // chain result ready for the epilogue
@@ -237,7 +281,7 @@ namespace {
 
 int64_t round_up(int64_t a, int64_t b) { return (a + b - 1) / b * b; }
 
-void choose_partition(int sm, int64_t R, int64_t C, int r_pad, Side* s) {
+void choose_partition(int sm, int64_t R, int64_t C, int r_pad, int planes, Side* s) {
   const int64_t tiles = ceil_div64(R, TILE_ROWS), kblocks = ceil_div64(C, BK);
   int best_s = 1;
   double best_eff = -1.0;
@@ -257,22 +301,24 @@ void choose_partition(int sm, int64_t R, int64_t C, int r_pad, Side* s) {
   s->cp.tiles = (int)tiles;
   s->cp.amode = 0;
   s->cp.kb_per_slab = 1;
-  // factor planes of this side: r_pad x ld, hi + lo.  When they do not fit L2 comfortably, order the units split-major
-  s->cp.split_major = ((size_t)r_pad * (size_t)round_up(C, 64) * 4 > ((size_t)32 << 20) && tiles <= sm) ? 1 : 0;
-  const size_t stage_bytes = 2 * (size_t)TILE_ROWS * BK * 2 + 2 * (size_t)r_pad * BK * 2;
+  // factor planes of this side: r_pad x ld, `planes` of them.  When they do not fit L2 comfortably, order the units split-major
+  s->cp.split_major = ((size_t)r_pad * (size_t)round_up(C, 64) * 2 * planes > ((size_t)32 << 20) && tiles <= sm) ? 1 : 0;
+  const size_t stage_bytes = (size_t)planes * ((size_t)TILE_ROWS * BK * 2 + (size_t)r_pad * BK * 2);
   int stages = (int)((200 * 1024) / stage_bytes);
   if (stages > 6) stages = 6;
   if (stages < 2) stages = 2;
   s->cp.num_stages = stages;
-  s->cp.drain = 2;
+  s->cp.drain = planes == 3 ? 1 : 2;    // 3 planes: 24 MMAs per stage already
   s->cp.ld_partial = round_up(R, TILE_ROWS);
   s->smem = (size_t)stages * stage_bytes + (2 * stages + 4) * sizeof(uint64_t) + 16;
   s->grid = s->cp.num_units < sm ? s->cp.num_units : sm;
 }
 
-// Sum of hi + lo over an [rows x cols] plane pair: per-block fp64 partials (rows are dealt round-robin to the blocks).
+// Sum of hi + lo (+ mid) over an [rows x cols] plane pair (triple): per-block fp64 partials (rows are dealt round-robin to the
+// blocks).
+template <int PLANES>
 __global__ void __launch_bounds__(256) plane_total_kernel(const bf16* __restrict__ hi, const bf16* __restrict__ lo, int64_t ld,
-                                                          int64_t rows, int64_t cols, double* part) {
+                                                          int64_t rows, int64_t cols, double* part, const bf16* __restrict__ mid) {
   __shared__ double sh[33];
   double s = 0.0;
   for (int64_t r = blockIdx.x; r < rows; r += gridDim.x) {
@@ -281,7 +327,10 @@ __global__ void __launch_bounds__(256) plane_total_kernel(const bf16* __restrict
     float t = 0.f;
     int cnt = 0;
     for (int64_t c = threadIdx.x; c < cols; c += 256) {
-      t += __bfloat162float(h[c]) + __bfloat162float(l[c]);
+      if constexpr (PLANES == 3)
+        t += __bfloat162float(h[c]) + (__bfloat162float(mid[r * ld + c]) + __bfloat162float(l[c]));
+      else
+        t += __bfloat162float(h[c]) + __bfloat162float(l[c]);
       if (++cnt == 16) { s += (double)t; t = 0.f; cnt = 0; }
     }
     s += (double)t;
@@ -344,13 +393,13 @@ __global__ void __launch_bounds__(256) krao_row_planes_kernel(const float* __res
 
 void nnfac_split_planes(const float* in, int64_t ld_in, int64_t rows, int64_t cols, __nv_bfloat16* hi, __nv_bfloat16* lo,
                         int64_t ld_out, int grid, cudaStream_t st) {
-  split_planes_kernel<<<grid, 256, 0, st>>>(in, ld_in, rows, cols, hi, lo, ld_out);
+  split_planes_kernel<2><<<grid, 256, 0, st>>>(in, ld_in, rows, cols, hi, lo, ld_out, nullptr);
 }
 
 void nnfac_split_planes_transposed(const float* in, int64_t ld_in, int64_t rows, int64_t cols, __nv_bfloat16* hiT,
                                    __nv_bfloat16* loT, int64_t ld_out, cudaStream_t st) {
   dim3 g((unsigned)ceil_div64(cols, 32), (unsigned)ceil_div64(rows, 32)), b(32, 8);
-  split_planes_transposed_kernel<<<g, b, 0, st>>>(in, ld_in, rows, cols, hiT, loT, ld_out);
+  split_planes_transposed_kernel<2><<<g, b, 0, st>>>(in, ld_in, rows, cols, hiT, loT, ld_out, nullptr);
 }
 
 void nnfac_reduce_partials(const float* partial, int splits, int r, int r_pad, int64_t R, int64_t ld_partial, float* out,
@@ -369,24 +418,26 @@ void nnfac_reduce_partials_chunked(const float* partial, int splits, int r, int 
                                                        (int64_t)r * (chunk + tail_cols), slabs, tail, ld_tail, tail_cols);
 }
 
-// every variant of the cross-product kernel: padded rank <= 64 / <= 128 x addressing mode of the X operand
+// every variant of the cross-product kernel: padded rank <= 64 / <= 128 x addressing mode of the X operand (+ the 3-plane one)
 template <int AMODE>
 static cudaError_t cross_set_smem(int r_pad, size_t smem) {
-  return r_pad <= 64 ? cudaFuncSetAttribute(tc_cross_kernel<64, AMODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                     : cudaFuncSetAttribute(tc_cross_kernel<128, AMODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  return r_pad <= 64 ? cudaFuncSetAttribute(tc_cross_kernel<64, AMODE, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                     : cudaFuncSetAttribute(tc_cross_kernel<128, AMODE, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 }
-static cudaError_t cross_prepare(const Side* s, int r_pad) {
+static cudaError_t cross_prepare(const Side* s, int r_pad, int planes) {
+  if (planes == 3) return cudaFuncSetAttribute(tc_cross_kernel<64, 0, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem);
   return s->cp.amode == 0 ? cross_set_smem<0>(r_pad, s->smem) : s->cp.amode == 1 ? cross_set_smem<1>(r_pad, s->smem) : cross_set_smem<2>(r_pad, s->smem);
 }
 template <int AMODE>
 static void cross_launch_mode(const Side* s, const CrossParams& cp, int r_pad, cudaStream_t st) {
   if (r_pad <= 64)
-    tc_cross_kernel<64, AMODE><<<s->grid, NTHREADS, s->smem, st>>>(s->map_xh, s->map_xl, s->map_fh, s->map_fl, cp);
+    tc_cross_kernel<64, AMODE, 2><<<s->grid, NTHREADS, s->smem, st>>>(s->map_xh, s->map_xl, s->map_fh, s->map_fl, cp, s->map_xh, s->map_fh);
   else
-    tc_cross_kernel<128, AMODE><<<s->grid, NTHREADS, s->smem, st>>>(s->map_xh, s->map_xl, s->map_fh, s->map_fl, cp);
+    tc_cross_kernel<128, AMODE, 2><<<s->grid, NTHREADS, s->smem, st>>>(s->map_xh, s->map_xl, s->map_fh, s->map_fl, cp, s->map_xh, s->map_fh);
 }
-static void cross_launch(const Side* s, const CrossParams& cp, int r_pad, cudaStream_t st) {
-  if (cp.amode == 0) cross_launch_mode<0>(s, cp, r_pad, st);
+static void cross_launch(const Side* s, const CrossParams& cp, int r_pad, int planes, cudaStream_t st) {
+  if (planes == 3) tc_cross_kernel<64, 0, 3><<<s->grid, NTHREADS, s->smem, st>>>(s->map_xh, s->map_xl, s->map_fh, s->map_fl, cp, s->map_xm, s->map_fm);
+  else if (cp.amode == 0) cross_launch_mode<0>(s, cp, r_pad, st);
   else if (cp.amode == 1) cross_launch_mode<1>(s, cp, r_pad, st);
   else cross_launch_mode<2>(s, cp, r_pad, st);
 }
@@ -403,22 +454,26 @@ int nnfac_nmf_plan_destroy(nnfac_nmf_plan* p) {
 // Every device buffer of a plan is carved out of ONE allocation (256-byte aligned pieces): either the caller's
 // workspace (`buffer`, at least nnfac_nmf_plan_bytes() bytes -- e.g. a block of a caching allocator, so that repeated
 // factorisations of same-shaped data never reach cudaMalloc / cudaFree) or one cudaMalloc owned by the plan.
-static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, void* buffer, size_t buffer_bytes, cudaStream_t st,
-                      nnfac_nmf_plan** out, size_t* bytes_out) {
-  NNFAC_ARG(ctx && m > 0 && n > 0 && r > 0 && sides >= 1 && sides <= 3, "nnfac_nmf_plan_create: bad argument");
+static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, int planes, void* buffer, size_t buffer_bytes,
+                      cudaStream_t st, nnfac_nmf_plan** out, size_t* bytes_out) {
+  NNFAC_ARG(ctx && m > 0 && n > 0 && r > 0 && sides >= 1 && sides <= 3 && (planes == 2 || planes == 3), "nnfac_nmf_plan_create: bad argument");
   if (r > 128) { nnfac_set_error("nnfac_nmf_plan_create: rank %d > 128 is not covered by the tensor-core path", r); return NNFAC_ERR_UNSUPPORTED; }
+  if (planes == 3 && r > 64) { nnfac_set_error("nnfac_nmf_plan_create: 3-plane plans cover rank <= 64 (rank %d)", r); return NNFAC_ERR_UNSUPPORTED; }
   if (m >= (1ll << 31) - 256 || n >= (1ll << 31) - 256) { nnfac_set_error("nnfac_nmf_plan_create: dimension too large"); return NNFAC_ERR_UNSUPPORTED; }
   nnfac_nmf_plan* p = (nnfac_nmf_plan*)calloc(1, sizeof(nnfac_nmf_plan));
   if (!p) return NNFAC_ERR_ALLOC;
   p->ctx = ctx; p->m = m; p->n = n; p->r = r;
   p->sides = sides;
+  p->planes = planes;
   p->r_pad = (int)round_up(r, 16);
   p->rk = p->r_pad <= 64 ? 64 : 128;
   p->fused_ok = 1;                       // rank <= 128: residual pass; the beta = 1 pass needs rk == 64
   // ---- sizes ----
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-  size_t o_xh[2], o_xl[2], o_fh[2], o_fl[2], o_rh[2] = {0, 0}, o_rl[2] = {0, 0}, xb[2], fb[2], rb[2] = {0, 0};
+  size_t o_xh[2], o_xl[2], o_fh[2], o_fl[2], o_xm[2], o_fm[2], o_rh[2] = {0, 0}, o_rl[2] = {0, 0}, o_rm[2] = {0, 0}, xb[2], fb[2],
+         rb[2] = {0, 0};
+  const size_t mid = planes == 3 ? 1 : 0;    // the middle planes exist in 3-plane plans only
   size_t partial_bytes = 0;
   for (int i = 0; i < 2; ++i) {
     Side* s = &p->side[i];
@@ -428,7 +483,8 @@ static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, vo
     xb[i] = (sides >> i) & 1 ? (size_t)s->R * s->ld * sizeof(bf16) : 0;     // an absent side keeps no planes of X
     fb[i] = (size_t)p->r_pad * s->ld * sizeof(bf16);
     o_xh[i] = take(xb[i]); o_xl[i] = take(xb[i]); o_fh[i] = take(fb[i]); o_fl[i] = take(fb[i]);
-    choose_partition(ctx->sm_count, s->R, s->C, p->r_pad, s);
+    o_xm[i] = take(mid * xb[i]); o_fm[i] = take(mid * fb[i]);
+    choose_partition(ctx->sm_count, s->R, s->C, p->r_pad, planes, s);
     const size_t pb = (size_t)s->cp.splits * p->r_pad * s->cp.ld_partial * sizeof(float);
     if (((sides >> i) & 1) && pb > partial_bytes) partial_bytes = pb;
   }
@@ -436,7 +492,7 @@ static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, vo
   if (p->fused_ok)
     for (int i = 0; i < 2; ++i) {
       rb[i] = (size_t)(i == 0 ? m : n) * p->rk * sizeof(bf16);
-      o_rh[i] = take(rb[i]); o_rl[i] = take(rb[i]);
+      o_rh[i] = take(rb[i]); o_rl[i] = take(rb[i]); o_rm[i] = take(mid * rb[i]);
     }
   const size_t o_cost = take(sizeof(double) * 2048);
   if (bytes_out) *bytes_out = off;
@@ -470,8 +526,14 @@ static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, vo
     if (!rc) rc = make_map(&s->map_xl, s->xl, s->R, s->C, s->ld, TILE_ROWS);
     if (!rc) rc = make_map(&s->map_fh, s->fh, p->r_pad, s->C, s->ld, p->r_pad);
     if (!rc) rc = make_map(&s->map_fl, s->fl, p->r_pad, s->C, s->ld, p->r_pad);
+    if (planes == 3) {
+      s->xm = (bf16*)(base + o_xm[i]); s->fm = (bf16*)(base + o_fm[i]);
+      cudaMemsetAsync(s->fm, 0, fb[i], st);
+      if (!rc) rc = make_map(&s->map_xm, s->xm, s->R, s->C, s->ld, TILE_ROWS);
+      if (!rc) rc = make_map(&s->map_fm, s->fm, p->r_pad, s->C, s->ld, p->r_pad);
+    }
     if (rc) { nnfac_nmf_plan_destroy(p); return rc; }
-    cudaError_t e = cross_prepare(s, p->r_pad);
+    cudaError_t e = cross_prepare(s, p->r_pad, planes);
     if (e != cudaSuccess) { nnfac_set_error("cudaFuncSetAttribute(smem=%zu): %s", s->smem, cudaGetErrorString(e)); nnfac_nmf_plan_destroy(p); return NNFAC_ERR_CUDA; }
   }
   p->partial = (float*)(base + o_partial);
@@ -487,6 +549,12 @@ static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, vo
       if (!rc) rc = make_map(&p->map_row_a_l[i], p->rowp_l[i], len, p->rk, p->rk, TILE_ROWS);
       if (!rc) rc = make_map(&p->map_row_b_h[i], p->rowp_h[i], len, p->rk, p->rk, 64);
       if (!rc) rc = make_map(&p->map_row_b_l[i], p->rowp_l[i], len, p->rk, p->rk, 64);
+      if (planes == 3) {
+        p->rowp_m[i] = (bf16*)(base + o_rm[i]);
+        cudaMemsetAsync(p->rowp_m[i], 0, rb[i], st);
+        if (!rc) rc = make_map(&p->map_row_a_m[i], p->rowp_m[i], len, p->rk, p->rk, TILE_ROWS);
+        if (!rc) rc = make_map(&p->map_row_b_m[i], p->rowp_m[i], len, p->rk, p->rk, 64);
+      }
       if (rc) { nnfac_nmf_plan_destroy(p); return rc; }
     }
   }
@@ -500,31 +568,44 @@ static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, vo
 
 int nnfac_nmf_plan_create(nnfac_ctx* ctx, int64_t m, int64_t n, int r, nnfac_nmf_plan** out) {
   NNFAC_ARG(out != nullptr, "nnfac_nmf_plan_create: out is NULL");
-  return plan_build(ctx, m, n, r, 3, nullptr, 0, (cudaStream_t)0, out, nullptr);
+  return plan_build(ctx, m, n, r, 3, 2, nullptr, 0, (cudaStream_t)0, out, nullptr);
 }
 
 int nnfac_nmf_plan_bytes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, size_t* bytes) {
   NNFAC_ARG(bytes != nullptr, "nnfac_nmf_plan_bytes: bytes is NULL");
-  return plan_build(ctx, m, n, r, 3, nullptr, 0, (cudaStream_t)0, nullptr, bytes);
+  return plan_build(ctx, m, n, r, 3, 2, nullptr, 0, (cudaStream_t)0, nullptr, bytes);
 }
 
 int nnfac_nmf_plan_create_in(nnfac_ctx* ctx, int64_t m, int64_t n, int r, void* workspace, size_t workspace_bytes,
                              void* stream, nnfac_nmf_plan** out) {
   NNFAC_ARG(out != nullptr && workspace != nullptr, "nnfac_nmf_plan_create_in: NULL argument");
-  return plan_build(ctx, m, n, r, 3, workspace, workspace_bytes, (cudaStream_t)stream, out, nullptr);
+  return plan_build(ctx, m, n, r, 3, 2, workspace, workspace_bytes, (cudaStream_t)stream, out, nullptr);
 }
 
 // One-sided plans: sides = 1 keeps only the planes of X (passes over side 0: V X^T, the MTTKRP of an unfolding),
 // sides = 2 only those of X^T, 3 both.  A pass over an absent side is refused.
 int nnfac_nmf_plan_bytes_sided(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, size_t* bytes) {
   NNFAC_ARG(bytes != nullptr, "nnfac_nmf_plan_bytes_sided: bytes is NULL");
-  return plan_build(ctx, m, n, r, sides, nullptr, 0, (cudaStream_t)0, nullptr, bytes);
+  return plan_build(ctx, m, n, r, sides, 2, nullptr, 0, (cudaStream_t)0, nullptr, bytes);
 }
 
 int nnfac_nmf_plan_create_sided(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, void* workspace, size_t workspace_bytes,
                                 void* stream, nnfac_nmf_plan** out) {
   NNFAC_ARG(out != nullptr && workspace != nullptr, "nnfac_nmf_plan_create_sided: NULL argument");
-  return plan_build(ctx, m, n, r, sides, workspace, workspace_bytes, (cudaStream_t)stream, out, nullptr);
+  return plan_build(ctx, m, n, r, sides, 2, workspace, workspace_bytes, (cudaStream_t)stream, out, nullptr);
+}
+
+// The same with `planes` bf16 planes per value: 2 (as above) or 3 (hi + mid + lo: every fp32 value of X and of the factors
+// exactly; rank <= 64).  The plane count is fixed here because the planes are carved from the one workspace.
+int nnfac_nmf_plan_bytes_planes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, int planes, size_t* bytes) {
+  NNFAC_ARG(bytes != nullptr, "nnfac_nmf_plan_bytes_planes: bytes is NULL");
+  return plan_build(ctx, m, n, r, sides, planes, nullptr, 0, (cudaStream_t)0, nullptr, bytes);
+}
+
+int nnfac_nmf_plan_create_planes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, int planes, void* workspace,
+                                 size_t workspace_bytes, void* stream, nnfac_nmf_plan** out) {
+  NNFAC_ARG(out != nullptr && workspace != nullptr, "nnfac_nmf_plan_create_planes: NULL argument");
+  return plan_build(ctx, m, n, r, sides, planes, workspace, workspace_bytes, (cudaStream_t)stream, out, nullptr);
 }
 
 // View plan: the unfolding of another mode of the C-order tensor whose mode-0 unfolding `base` holds (base: I_0 x rest, planes
@@ -538,6 +619,7 @@ static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, 
                       size_t buffer_bytes, cudaStream_t st, nnfac_nmf_plan** out, size_t* bytes_out) {
   NNFAC_ARG(ctx && base && left >= 1 && I >= 1 && right >= 1 && r > 0 && r <= 128, "nnfac_nmf_plan_view: bad argument");
   NNFAC_ARG(!base->base && (base->sides & 1), "nnfac_nmf_plan_view: the base plan must own the planes of side 0");
+  if (base->planes != 2) { nnfac_set_error("nnfac_nmf_plan_view: views of 3-plane plans are not built"); return NNFAC_ERR_UNSUPPORTED; }
   NNFAC_ARG(left * I * right == base->m * base->n, "nnfac_nmf_plan_view: %lld x %lld x %lld is not the base tensor", (long long)left,
             (long long)I, (long long)right);
   if (left == 1 || base->side[0].ld != base->n || (right == 1 ? (I % 8 != 0) : (right % 64 != 0)) || left * right >= (1ll << 31) - 256) {
@@ -546,13 +628,13 @@ static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, 
   }
   nnfac_nmf_plan* p = (nnfac_nmf_plan*)calloc(1, sizeof(nnfac_nmf_plan));
   if (!p) return NNFAC_ERR_ALLOC;
-  p->ctx = ctx; p->base = base; p->m = I; p->n = left * right; p->r = r; p->sides = 1;
+  p->ctx = ctx; p->base = base; p->m = I; p->n = left * right; p->r = r; p->sides = 1; p->planes = 2;
   p->r_pad = (int)round_up(r, 16);
   p->rk = p->r_pad <= 64 ? 64 : 128;
   p->fused_ok = 0;
   Side* s = &p->side[0];
   s->R = I; s->C = left * right; s->ld = round_up(s->C, 64);
-  choose_partition(ctx->sm_count, s->R, s->C, p->r_pad, s);
+  choose_partition(ctx->sm_count, s->R, s->C, p->r_pad, 2, s);
   s->cp.amode = right == 1 ? 1 : 2;
   s->cp.kb_per_slab = right == 1 ? 1 : (int)(right / 64);
   size_t off = 0;
@@ -585,7 +667,7 @@ static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, 
   }
   if (!rc) rc = make_map(&s->map_fh, s->fh, p->r_pad, s->C, s->ld, p->r_pad);
   if (!rc) rc = make_map(&s->map_fl, s->fl, p->r_pad, s->C, s->ld, p->r_pad);
-  if (!rc && cross_prepare(s, p->r_pad) != cudaSuccess) { nnfac_set_error("cudaFuncSetAttribute failed for a view plan"); rc = NNFAC_ERR_CUDA; }
+  if (!rc && cross_prepare(s, p->r_pad, 2) != cudaSuccess) { nnfac_set_error("cudaFuncSetAttribute failed for a view plan"); rc = NNFAC_ERR_CUDA; }
   if (!rc && cudaGetLastError() != cudaSuccess) { nnfac_set_error("nnfac_nmf_plan_create_view: clearing the workspace failed"); rc = NNFAC_ERR_CUDA; }
   if (rc) { free(p); return rc; }
   *out = p;
@@ -611,9 +693,15 @@ int nnfac_nmf_plan_load_x_rows(nnfac_nmf_plan* p, const float* Xrows, int64_t ld
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t total = rows * p->n;
   int grid = (int)(ceil_div64(total, 256) < (int64_t)p->ctx->sm_count * 32 ? ceil_div64(total, 256) : (int64_t)p->ctx->sm_count * 32);
+  const Side* s0 = &p->side[0];
+  const Side* s1 = &p->side[1];
   if (p->sides & 1) {
-    split_planes_kernel<<<grid, 256, 0, st>>>(Xrows, ldx, rows, p->n, p->side[0].xh + row0 * p->side[0].ld,
-                                              p->side[0].xl + row0 * p->side[0].ld, p->side[0].ld);
+    if (p->planes == 3)
+      split_planes_kernel<3><<<grid, 256, 0, st>>>(Xrows, ldx, rows, p->n, s0->xh + row0 * s0->ld, s0->xl + row0 * s0->ld, s0->ld,
+                                                   s0->xm + row0 * s0->ld);
+    else
+      split_planes_kernel<2><<<grid, 256, 0, st>>>(Xrows, ldx, rows, p->n, s0->xh + row0 * s0->ld, s0->xl + row0 * s0->ld, s0->ld,
+                                                   nullptr);
     NNFAC_LAUNCH_CHECK(p->ctx);
   }
   // grid.y is limited to 65535 blocks of 32 rows: walk the rows in slabs
@@ -621,8 +709,12 @@ int nnfac_nmf_plan_load_x_rows(nnfac_nmf_plan* p, const float* Xrows, int64_t ld
   for (int64_t r0 = 0; (p->sides & 2) && r0 < rows; r0 += slab) {
     const int64_t nr = rows - r0 < slab ? rows - r0 : slab;
     dim3 g((unsigned)ceil_div64(p->n, 32), (unsigned)ceil_div64(nr, 32)), b(32, 8);
-    split_planes_transposed_kernel<<<g, b, 0, st>>>(Xrows + r0 * ldx, ldx, nr, p->n, p->side[1].xh + row0 + r0,
-                                                    p->side[1].xl + row0 + r0, p->side[1].ld);
+    if (p->planes == 3)
+      split_planes_transposed_kernel<3><<<g, b, 0, st>>>(Xrows + r0 * ldx, ldx, nr, p->n, s1->xh + row0 + r0, s1->xl + row0 + r0,
+                                                         s1->ld, s1->xm + row0 + r0);
+    else
+      split_planes_transposed_kernel<2><<<g, b, 0, st>>>(Xrows + r0 * ldx, ldx, nr, p->n, s1->xh + row0 + r0, s1->xl + row0 + r0,
+                                                         s1->ld, nullptr);
     NNFAC_LAUNCH_CHECK(p->ctx);
   }
   return NNFAC_OK;
@@ -633,11 +725,14 @@ int nnfac_nmf_plan_load_x_done(nnfac_nmf_plan* p, void* stream) {
   NNFAC_ARG(p != nullptr, "nnfac_nmf_plan_load_x_done: plan is NULL");
   cudaStream_t st = (cudaStream_t)stream;
   if (p->fused_ok && (p->sides & 1)) {
-    // sum of X as the passes see it (hi + lo planes), fp64, fixed order: the constant term of the KL cost
+    // sum of X as the passes see it (hi + lo (+ mid) planes), fp64, fixed order: the constant term of the KL cost
     const int blocks = p->ctx->sm_count * 4;
     const int grc = nnfac_guard_enter(p->ctx, NNFAC_GUARD_RED, st);
     if (grc) return grc;
-    plane_total_kernel<<<blocks, 256, 0, st>>>(p->side[0].xh, p->side[0].xl, p->side[0].ld, p->m, p->n, p->ctx->red);
+    if (p->planes == 3)
+      plane_total_kernel<3><<<blocks, 256, 0, st>>>(p->side[0].xh, p->side[0].xl, p->side[0].ld, p->m, p->n, p->ctx->red, p->side[0].xm);
+    else
+      plane_total_kernel<2><<<blocks, 256, 0, st>>>(p->side[0].xh, p->side[0].xl, p->side[0].ld, p->m, p->n, p->ctx->red, nullptr);
     NNFAC_LAUNCH_CHECK(p->ctx);
     plane_total_finish_kernel<<<1, 32, 0, st>>>(p->ctx->red, blocks, p->sums);
     NNFAC_LAUNCH_CHECK(p->ctx);
@@ -662,12 +757,13 @@ int nnfac_nmf_plan_cross(nnfac_nmf_plan* p, int which, const float* F, int64_t l
   if (F) {   // F == NULL: the operand planes of the factor installed by nnfac_nmf_plan_set_factor / _mu_finish are current
     const int64_t total = (int64_t)p->r * s->C;
     grid = (int)(ceil_div64(total, 256) < (int64_t)p->ctx->sm_count * 8 ? ceil_div64(total, 256) : (int64_t)p->ctx->sm_count * 8);
-    split_planes_kernel<<<grid, 256, 0, st>>>(F, ldf, p->r, s->C, s->fh, s->fl, s->ld);
+    if (p->planes == 3) split_planes_kernel<3><<<grid, 256, 0, st>>>(F, ldf, p->r, s->C, s->fh, s->fl, s->ld, s->fm);
+    else split_planes_kernel<2><<<grid, 256, 0, st>>>(F, ldf, p->r, s->C, s->fh, s->fl, s->ld, nullptr);
     NNFAC_LAUNCH_CHECK(p->ctx);
   }
   CrossParams cp = s->cp;
   cp.partial = p->partial;
-  cross_launch(s, cp, p->r_pad, st);
+  cross_launch(s, cp, p->r_pad, p->planes, st);
   NNFAC_LAUNCH_CHECK(p->ctx);
   if (!out) return NNFAC_OK;     // the split-K partials stay in the plan (nnfac_nmf_plan_hals_solve / _reduce)
   const int64_t tot2 = (int64_t)p->r * s->R;
@@ -683,6 +779,7 @@ int nnfac_nmf_plan_cross(nnfac_nmf_plan* p, int which, const float* F, int64_t l
 int nnfac_nmf_plan_set_krao(nnfac_nmf_plan* p, const float* At, int64_t lda, int64_t I, const float* Bt, int64_t ldb, int64_t J,
                             void* stream) {
   NNFAC_ARG(p && At && Bt && I > 0 && J > 0 && I * J == p->n && lda >= I && ldb >= J, "nnfac_nmf_plan_set_krao: bad argument");
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_set_krao: writes two planes, the plan has %d", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   Side* s = &p->side[0];
   const int64_t total = I * J;
   const int grid = (int)(ceil_div64(total, 256) < (int64_t)p->ctx->sm_count * 16 ? ceil_div64(total, 256) : (int64_t)p->ctx->sm_count * 16);
@@ -699,6 +796,7 @@ int nnfac_nmf_plan_set_krao_rows(nnfac_nmf_plan* p, const float* At, int64_t lda
                                  void* stream) {
   NNFAC_ARG(p && At && Bt && I > 0 && J > 0 && I * J == p->n && lda >= I && ldb >= J, "nnfac_nmf_plan_set_krao_rows: bad argument");
   NNFAC_ARG(p->fused_ok && !p->base, "nnfac_nmf_plan_set_krao_rows: the plan has no row planes");
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_set_krao_rows: writes two planes, the plan has %d", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   const int64_t total = I * J;
   const int grid = (int)(ceil_div64(total, 256) < (int64_t)p->ctx->sm_count * 16 ? ceil_div64(total, 256) : (int64_t)p->ctx->sm_count * 16);
   krao_row_planes_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(At, lda, I, Bt, ldb, J, p->r, p->rk, p->rowp_h[1], p->rowp_l[1]);

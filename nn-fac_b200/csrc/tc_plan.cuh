@@ -98,7 +98,8 @@ struct Side {           // one orientation of X
   int64_t R, C, ld;     // plane is [R x C], leading dimension ld
   bf16 *xh, *xl;        // X planes
   bf16 *fh, *fl;        // factor planes [r_pad x ld]
-  CUtensorMap map_xh, map_xl, map_fh, map_fl;
+  bf16 *xm, *fm;        // 3-plane plans: the middle planes (x = xh + xm + xl); NULL otherwise
+  CUtensorMap map_xh, map_xl, map_fh, map_fl, map_xm, map_fm;
   CrossParams cp;
   int grid;
   size_t smem;
@@ -117,8 +118,11 @@ struct nnfac_nmf_plan {
   //   rowp[0] = U [m x rk], rowp[1] = V^T [n x rk]; map_row_a: 128-row boxes (A operand of the model GEMM, rk = 64 only),
   //   map_row_b: boxes of 64 rows x 64 ranks (B operand of the model GEMM)
   int rk;
-  __nv_bfloat16 *rowp_h[2], *rowp_l[2];
-  CUtensorMap map_row_a_h[2], map_row_a_l[2], map_row_b_h[2], map_row_b_l[2];
+  __nv_bfloat16 *rowp_h[2], *rowp_l[2], *rowp_m[2];
+  CUtensorMap map_row_a_h[2], map_row_a_l[2], map_row_b_h[2], map_row_b_l[2], map_row_a_m[2], map_row_b_m[2];
+  // bf16 planes per value, fixed at creation: 2 (hi + lo, 16 significant bits) or 3 (hi + mid + lo, the fp32 value
+  // itself; rank <= 64; products of six MMAs).  Writers that only know two planes refuse a 3-plane plan.
+  int planes;
   double* cost_part;    // [1024] per-CTA cost partials of a fused pass ([512 + i]: second partial of CTA i)
   double* sums;         // cost_part + 1024: [0] sum of X (as stored in the planes)
   int fused_ok;

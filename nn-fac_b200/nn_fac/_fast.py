@@ -36,13 +36,27 @@ from nn_fac import _ops as ops
 MODE_RES, MODE_MU = 0, 1
 
 
-def eligible(dtype, rank, update_rule, beta):
-    """fp32 on the tcgen05 path: HALS and Frobenius MU up to rank 128 (residual + cross-product pass), KL MU up to rank 64."""
+def eligible(dtype, rank, update_rule, beta, planes=2):
+    """fp32 on the tcgen05 path: HALS and Frobenius MU up to rank 128 (residual + cross-product pass), KL MU up to rank 64.
+    planes = 3 (precision "fp32x3"): all three up to rank 64."""
     if dtype != torch.float32:
         return False
     if update_rule == "hals" or (update_rule == "mu" and beta == 2):
-        return rank <= 128
+        return rank <= (128 if planes == 2 else 64)
     return update_rule == "mu" and beta == 1 and rank <= 64
+
+
+def planes_of_precision():
+    """bf16 planes per value of the tensor-core NMF path under the current config.precision."""
+    from nn_fac import config
+    return 3 if config.precision == "fp32x3" else 2
+
+
+# HALS solves of a 3-plane factorisation run on a copy (the tensor-core sweep inside nnfac_nmf_plan_hals_solve writes two planes)
+# through nnfac_hals_nnls, with NNFAC_HALS_NO_TC: the fp32 CUDA-core sweep solves instead of the tensor-core one, whose step
+# operand is a bf16 hi/lo split.  At 4096 x 4096, rank 32, near-exact data the tensor-core sweep left the objective 1.6e-4
+# away from float64, the CUDA-core sweep 6.7e-5 (DESIGN.md section 1).
+TC_SWEEP_FP32X3 = False
 
 
 # Peer-mapped resources are expensive to set up (cudaMalloc + CUDA IPC export / open on every rank + a barrier: tens of
@@ -345,8 +359,8 @@ class PeerExchange:
 class CudaEngine:
     """The device operators one outer iteration is made of, all in libnnfac_b200 (no torch arithmetic)."""
 
-    def __init__(self, X, r, device=None):
-        self.plan = ops.NMFPlan(X, device).bind_rank(r)
+    def __init__(self, X, r, device=None, planes=2):
+        self.plan = ops.NMFPlan(X, device).bind_rank(r, planes=planes)
 
     def set_factor(self, which, Ft):
         self.plan.set_factor(which, Ft)
@@ -357,6 +371,10 @@ class CudaEngine:
     def mu_finish(self, which, F, den_vec):
         """mu.py:84-88 on the numerator the last fused(which, MODE_MU, keep_partials=True) left in the plan,
         plus the installation of the new factor: one kernel."""
+        if self.plan.planes == 3:       # nnfac_nmf_plan_mu_finish writes two planes: update on a copy, then install
+            new = self.mu_apply(F, self.plan.reduce(which), den_vec)
+            self.set_factor(which, new)
+            return new
         return self.plan.mu_finish(which, F, den_vec, mu.epsilon)
 
     def cross(self, which, F, keep_partials=False):
@@ -375,7 +393,10 @@ class CudaEngine:
         if UtM is None:
             UtM = self.plan.reduce(which)
         new = F.clone()
-        self.sweep(UtM, UtU, new, r, sparsity, normalize, result)
+        if self.plan.planes == 3 and not TC_SWEEP_FP32X3 and type(self).sweep is CudaEngine.sweep:
+            ops.hals_nnls(UtM, UtU, new, r, 100, 0.01, sp, bool(normalize), False, result, no_tc=True)
+        else:
+            self.sweep(UtM, UtU, new, r, sparsity, normalize, result)
         self.set_factor(which, new)
         return new
 
@@ -427,14 +448,18 @@ class FusedNMF:
 
     def __init__(self, data, U, V, device=None, group=None, engine=None):
         """data: X (m x n), or this rank's column block X_p when `group` spans several ranks;
-        U: m x r (replicated); V: r x n, or this rank's block V_p."""
+        U: m x r (replicated); V: r x n, or this rank's block V_p.  The plan's planes per value follow config.precision
+        (3 under "fp32x3", one GPU only)."""
         self.comm = group if isinstance(group, Comm) else Comm(group)
         self.r = int(U.shape[1])
         if engine is None:
+            planes = planes_of_precision()
+            if planes == 3 and self.comm.world > 1:
+                raise NotImplementedError("precision 'fp32x3' covers one GPU (the sharded exchanges write two planes)")
             # a host-resident X goes straight into the plan (upload pipelined with the ingest)
             if isinstance(data, torch.Tensor) and data.is_cuda:
                 data = data.to(dtype=torch.float32).contiguous()
-            self.eng = CudaEngine(data, self.r, device)
+            self.eng = CudaEngine(data, self.r, device, planes=planes)
             self.m, self.n = self.eng.plan.m, self.eng.plan.n
             self.device = self.eng.plan.device
             U_dev = L.to_device(U, torch.float32, device)

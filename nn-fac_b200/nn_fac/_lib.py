@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("NNFAC_B200_LIB") or os.path.join(os.path.dirname(_HER
 
 F32, F64 = 0, 1
 ERR_UNSUPPORTED = -3
-HALS_NORMALIZE, HALS_NONZERO = 1, 2
+HALS_NORMALIZE, HALS_NONZERO, HALS_NO_TC = 1, 2, 4
 
 _c = ctypes
 _P, _I64, _INT, _DBL, _U32 = _c.c_void_p, _c.c_int64, _c.c_int, _c.c_double, _c.c_uint
@@ -72,6 +72,8 @@ SIGNATURES = {
     "nnfac_nmf_plan_create_in": [_P, _I64, _I64, _INT, _P, _c.c_size_t, _P, _c.POINTER(_P)],
     "nnfac_nmf_plan_bytes_sided": [_P, _I64, _I64, _INT, _INT, _c.POINTER(_c.c_size_t)],
     "nnfac_nmf_plan_create_sided": [_P, _I64, _I64, _INT, _INT, _P, _c.c_size_t, _P, _c.POINTER(_P)],
+    "nnfac_nmf_plan_bytes_planes": [_P, _I64, _I64, _INT, _INT, _INT, _c.POINTER(_c.c_size_t)],
+    "nnfac_nmf_plan_create_planes": [_P, _I64, _I64, _INT, _INT, _INT, _P, _c.c_size_t, _P, _c.POINTER(_P)],
     "nnfac_nmf_plan_view_bytes": [_P, _P, _I64, _I64, _I64, _INT, _c.POINTER(_c.c_size_t)],
     "nnfac_nmf_plan_create_view": [_P, _P, _I64, _I64, _I64, _INT, _P, _c.c_size_t, _P, _c.POINTER(_P)],
     "nnfac_nmf_plan_destroy": [_P],
@@ -195,7 +197,7 @@ def resolve_dtype(*arrays):
     from . import config
     if config.precision == "fp32":
         return torch.float32
-    if config.precision == "fp64":
+    if config.precision in ("fp64", "fp32x3"):
         return torch.float64
     for a in arrays:
         if a is None:
@@ -207,10 +209,25 @@ def resolve_dtype(*arrays):
     return torch.float32
 
 
+def as_output(x):
+    """A result handed back to the caller (torch tensor or numpy array): float32 under precision "fp32x3", which computes every
+    path outside its 3-plane tensor-core NMF in float64; unchanged under the other precisions."""
+    from . import config
+    if config.precision != "fp32x3":
+        return x
+    if isinstance(x, torch.Tensor):
+        return x if x.dtype == torch.float32 else x.to(torch.float32)
+    x = np.asarray(x)
+    return x if x.dtype == np.float32 else x.astype(np.float32)
+
+
 def working_dtype(numel, *arrays):
     """(arithmetic dtype, dtype of the returned arrays): resolve_dtype, except that in "auto" mode a float32 problem of at most
-    config.small_problem_elements data elements computes in float64 (see nn_fac/config.py)."""
+    config.small_problem_elements data elements computes in float64, and that "fp32x3" computes in float64 and returns float32
+    wherever its 3-plane tensor-core path does not apply (see nn_fac/config.py)."""
     from . import config
+    if config.precision == "fp32x3":
+        return torch.float64, torch.float32
     dt = resolve_dtype(*arrays)
     if dt == torch.float32 and config.precision == "auto" and int(numel) <= config.small_problem_elements:
         return torch.float64, torch.float32

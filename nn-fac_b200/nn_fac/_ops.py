@@ -56,12 +56,13 @@ def transpose(A):
     return out
 
 
-def hals_nnls(UtM, UtU, V, r, maxiter, delta, sparsity, normalize, nonzero, result=None):
-    """In-place accelerated HALS on V (r x n).  Returns the device double[4] result vector."""
+def hals_nnls(UtM, UtU, V, r, maxiter, delta, sparsity, normalize, nonzero, result=None, no_tc=False):
+    """In-place accelerated HALS on V (r x n).  Returns the device double[4] result vector.
+    no_tc: never the tensor-core sweep (fp32 CUDA-core sweep instead)."""
     n = UtM.shape[1]
     if result is None:
         result = torch.empty(4, dtype=torch.float64, device=V.device)
-    flags = (L.HALS_NORMALIZE if normalize else 0) | (L.HALS_NONZERO if nonzero else 0)
+    flags = (L.HALS_NORMALIZE if normalize else 0) | (L.HALS_NONZERO if nonzero else 0) | (L.HALS_NO_TC if no_tc else 0)
     L.check(_lib().nnfac_hals_nnls(L.ctx(V.device), L.code_of(V.dtype), L.ptr(UtM), UtM.stride(0), L.ptr(UtU),
                                    UtU.stride(0), L.ptr(V), V.stride(0), r, n, maxiter, float(delta),
                                    float(sparsity), flags, L.ptr(result), L.stream_ptr()))
@@ -278,7 +279,8 @@ def unfold_times(P, B, mode):
 
 
 class NMFPlan:
-    """Owner of an nnfac_nmf_plan (X resident as bf16 hi/lo planes in both orientations; tcgen05 path)."""
+    """Owner of an nnfac_nmf_plan (X resident as bf16 hi/lo planes -- or hi/mid/lo, planes=3 -- in both orientations;
+    tcgen05 path)."""
 
     SLAB_BYTES = 64 << 20     # upload granularity of a host-resident X
 
@@ -298,22 +300,25 @@ class NMFPlan:
         self.m, self.n = X.shape
         self.handle = ctypes.c_void_p()
         self.r = None
+        self.planes = 2
         self._xf32 = None
         self._xf32_refused = False
         self._X = X
 
-    def bind_rank(self, r, sides=3):
-        """sides: 3 = planes of X and of X^T; 1 = only X (passes over side 0, e.g. the MTTKRP of an unfolding); 2 = only X^T."""
+    def bind_rank(self, r, sides=3, planes=2):
+        """sides: 3 = planes of X and of X^T; 1 = only X (passes over side 0, e.g. the MTTKRP of an unfolding); 2 = only X^T.
+        planes: bf16 planes per value, 2 (hi + lo) or 3 (hi + mid + lo, the fp32 values exactly; rank <= 64)."""
         import ctypes
         self.r = r
         self.sides = sides
+        self.planes = planes
         # the plan lives in one block of torch's caching allocator: a second factorisation of same-shaped data
         # reuses it without any cudaMalloc / cudaFree
         nbytes = ctypes.c_size_t()
-        L.check(_lib().nnfac_nmf_plan_bytes_sided(L.ctx(self.device), self.m, self.n, r, sides, ctypes.byref(nbytes)))
+        L.check(_lib().nnfac_nmf_plan_bytes_planes(L.ctx(self.device), self.m, self.n, r, sides, planes, ctypes.byref(nbytes)))
         self._workspace = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
-        L.check(_lib().nnfac_nmf_plan_create_sided(L.ctx(self.device), self.m, self.n, r, sides, L.ptr(self._workspace), nbytes.value,
-                                                   L.stream_ptr(), ctypes.byref(self.handle)))
+        L.check(_lib().nnfac_nmf_plan_create_planes(L.ctx(self.device), self.m, self.n, r, sides, planes, L.ptr(self._workspace),
+                                                    nbytes.value, L.stream_ptr(), ctypes.byref(self.handle)))
         if self._X.is_cuda:
             L.check(_lib().nnfac_nmf_plan_load_x(self.handle, L.ptr(self._X), self._X.stride(0), L.stream_ptr()))
         else:
@@ -331,7 +336,7 @@ class NMFPlan:
             return None
         L.check(rc)
         v = NMFPlan.__new__(NMFPlan)
-        v.device, v.m, v.n, v.r, v.sides = self.device, I, left * right, r, 1
+        v.device, v.m, v.n, v.r, v.sides, v.planes = self.device, I, left * right, r, 1, 2
         v._xf32, v._xf32_refused, v._X, v._base = None, True, None, self          # keeps the base plan (and its planes) alive
         v._workspace = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
         v.handle = ctypes.c_void_p()
@@ -446,10 +451,11 @@ class NMFPlan:
         # instructions per element (no bf16 unpack + add).  With the issuing warps converged the pass is bound by the issue
         # slots of its transform warps, and the copy pays: MU 905 -> 950 it/s at C2.  It costs 2 x 4mn bytes, so it is made on
         # first use only when that leaves at least as much memory free again (NNFAC_MU_F32=0 / 1 force it off / on).
+        # A 3-plane plan's beta = 1 pass always reads the copy (then the caller's fp32 values).
         if mode == 1 and self._xf32 is None and self.fused_ok and self.sides == 3 and not self._xf32_refused:
             want = os.environ.get("NNFAC_MU_F32", "auto")
             need = 2 * 4 * self.m * self.n
-            if want == "1" or (want != "0" and torch.cuda.mem_get_info(self.device)[0] > 2 * need + (1 << 30)):
+            if self.planes == 3 or want == "1" or (want != "0" and torch.cuda.mem_get_info(self.device)[0] > 2 * need + (1 << 30)):
                 self.enable_f32()
             else:
                 self._xf32_refused = True

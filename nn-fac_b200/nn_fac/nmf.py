@@ -177,14 +177,15 @@ def compute_nmf(data, rank, U_in, V_in, n_iter_max=100, tol=1e-8,
     if normalize is None or normalize is False:
         normalize = [False, False]
     dt, dt_out = L.working_dtype(int(np.prod(np.shape(data))), data, U_in, V_in)
-    if n_iter_max > 0 and _fast.eligible(dt, int(np.shape(U_in)[1]), update_rule, beta):
-        # fp32, rank <= 64: two X passes per iteration on tcgen05, cost fused with a lag of one pass
+    planes = _fast.planes_of_precision()
+    if n_iter_max > 0 and _fast.eligible(torch.float32 if planes == 3 else dt, int(np.shape(U_in)[1]), update_rule, beta, planes=planes):
+        # fp32, rank <= 64: two X passes per iteration on tcgen05, cost fused with a lag of one pass ("fp32x3": 3-plane plan)
         _check_step_arguments(update_rule, beta, sparsity_coefficients)
         fast = _fast.FusedNMF(data, U_in, V_in)
         cost_fct_vals, toc = fast.run(n_iter_max, tol, update_rule, sparsity_coefficients, fixed_modes, normalize, verbose,
                                       beta=beta)
         U_dev, V_dev = fast.factors()
-        U_out, V_out = _to_output(U_dev, data), _to_output(V_dev, data)
+        U_out, V_out = _to_output(U_dev, data, dt_out), _to_output(V_dev, data, dt_out)
         if return_costs:
             return U_out, V_out, cost_fct_vals, toc
         return U_out, V_out

@@ -417,9 +417,10 @@ def one_ntd_step(tensor, ranks, in_core, in_factors, norm_tensor, sparsity_coeff
     state = DeviceNTD(tensor, in_core, in_factors, dt)
     terms = state.step_hals_async(float(norm_tensor), sparsity_coefficients, fixed_modes, normalize, mode_core_norm, delta)
     cost = state.finish_cost_hals(terms.cpu().numpy(), float(norm_tensor), sparsity_coefficients)
+    core, factors = L.as_output(state.core), [L.as_output(f) for f in state.factors]
     if isinstance(tensor, torch.Tensor):
-        return state.core, state.factors, cost
-    return state.core.cpu().numpy(), [f.cpu().numpy() for f in state.factors], cost
+        return core, factors, cost
+    return core.cpu().numpy(), [f.cpu().numpy() for f in factors], cost
 
 
 def one_ntd_step_mu(tensor, ranks, in_core, in_factors, beta, norm_tensor,
@@ -430,9 +431,10 @@ def one_ntd_step_mu(tensor, ranks, in_core, in_factors, beta, norm_tensor,
     dt = L.resolve_dtype(tensor, in_core, *in_factors)
     state = DeviceNTD(tensor, in_core, in_factors, dt)
     cost = state.step_mu(beta, fixed_modes, normalize, mode_core_norm)
+    core, factors = L.as_output(state.core), [L.as_output(f) for f in state.factors]
     if isinstance(tensor, torch.Tensor):
-        return state.core, state.factors, cost
-    return state.core.cpu().numpy(), [f.cpu().numpy() for f in state.factors], cost
+        return core, factors, cost
+    return core.cpu().numpy(), [f.cpu().numpy() for f in factors], cost
 
 
 def ntd_mu(*args, **kwargs):

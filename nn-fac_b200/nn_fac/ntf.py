@@ -453,5 +453,6 @@ def one_ntf_step(unfolded_tensors, rank, in_factors, norm_tensor, update_rule, b
     dt = L.resolve_dtype(first, *in_factors)
     state = DeviceNTF(tensor, in_factors, dt)
     cost = state.step(rank, float(norm_tensor), update_rule, beta, sparsity_coefficients, fixed_modes, normalize)
-    factors = state.factors if isinstance(first, torch.Tensor) else [f.cpu().numpy() for f in state.factors]
+    factors = [L.as_output(f) for f in state.factors]
+    factors = factors if isinstance(first, torch.Tensor) else [f.cpu().numpy() for f in factors]
     return factors, cost

@@ -131,9 +131,15 @@ def compute_parafac_2(tensor_slices, rank, W_list_in, H_0, D_list_in, init_with_
             if verbose:
                 print('Converged in {} iterations.'.format(iteration))
             break
+    W_list, H, D_list = _as_output(W_list), L.as_output(np.array(H)), _as_output(D_list)
     if return_costs:
-        return W_list, np.array(H), D_list, cost_fct_vals, toc
-    return W_list, np.array(H), D_list
+        return W_list, H, D_list, cost_fct_vals, toc
+    return W_list, H, D_list
+
+
+def _as_output(arrays):
+    """L.as_output over a list of arrays (or a stacked array, which normalize[2] makes of D_list)."""
+    return L.as_output(arrays) if isinstance(arrays, np.ndarray) else [L.as_output(a) for a in arrays]
 
 
 def one_step_parafac2(slices, rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices,
@@ -142,9 +148,12 @@ def one_step_parafac2(slices, rank, W_list_in, H_in, D_list_in, mu_list_in, norm
                       sparsity_coefficient=None, fixed_modes=[], normalize=[False, False, False, False, False]):
     """One pass over all channels (parafac2.py:402-602).  The slices are uploaded on every call; use compute_parafac_2 to
     keep them resident."""
-    return _one_step(_Slices(slices), rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices, previous_cost_fct_val,
-                     increasing_mu=increasing_mu, tol_mu=tol_mu, step_mu=step_mu, init_with_P=init_with_P, W_star_in=W_star_in,
-                     P_list_in=P_list_in, sparsity_coefficient=sparsity_coefficient, fixed_modes=fixed_modes, normalize=normalize)
+    W_list, H, D_list, W_star, P_list, mu_list, cost, couple_error, increasing_mu = _one_step(
+        _Slices(slices), rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices, previous_cost_fct_val,
+        increasing_mu=increasing_mu, tol_mu=tol_mu, step_mu=step_mu, init_with_P=init_with_P, W_star_in=W_star_in,
+        P_list_in=P_list_in, sparsity_coefficient=sparsity_coefficient, fixed_modes=fixed_modes, normalize=normalize)
+    return (_as_output(W_list), L.as_output(H), _as_output(D_list), L.as_output(W_star), _as_output(P_list), mu_list, cost,
+            couple_error, increasing_mu)
 
 
 def _one_step(slices, rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices, previous_cost_fct_val, increasing_mu=True,
@@ -179,7 +188,7 @@ def _one_step(slices, rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices,
             DkH = D_list[k] @ H
             VVt = DkH @ DkH.T
             VMt = slices.right(k, DkH)                                    # DkH X_k^T on the GPU
-            W_list[k] = np.transpose(nnls.hals_coupling_nnls_acc(VMt, VVt, np.transpose(W_list[k]), np.transpose(P_list[k] @ W_star),
+            W_list[k] = np.transpose(nnls._hals_coupling_nnls_acc(VMt, VVt, np.transpose(W_list[k]), np.transpose(P_list[k] @ W_star),
                                                                  mu_list[k], maxiter=100, delta=0.01, normalize=normalize[0],
                                                                  nonzero=False)[0])
         if 2 not in fixed_modes:
@@ -190,7 +199,7 @@ def _one_step(slices, rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices,
             WtX = slices.left(k, W_list[k])                               # W_k^T X_k on the GPU
             UtM = ops.row_sums(ops.hadamard_(WtX, slices.up(H))).reshape(-1, 1).cpu().numpy()
             diag_D = np.reshape(np.diagonal(D_list[k]), (-1, 1))
-            new_D = nnls.hals_nnls_acc(UtM, UtU, diag_D, maxiter=100, delta=0.01, sparsity_coefficient=None, normalize=False,
+            new_D = nnls._hals_nnls_acc(UtM, UtU, diag_D, maxiter=100, delta=0.01, sparsity_coefficient=None, normalize=False,
                                        nonzero=False)[0]
             D_list[k] = np.diag(np.asarray(new_D).flatten())
     if normalize[2]:                                                      # :559-565 (D_list must be an array here, as in the reference)
@@ -211,7 +220,7 @@ def _one_step(slices, rank, W_list_in, H_in, D_list_in, mu_list_in, norm_slices,
             UtU += WkDk.T @ WkDk
             part = slices.left(k, WkDk)                                   # (W_k D_k)^T X_k on the GPU
             UtM = part if UtM is None else ops.axpby(1.0, UtM, 1.0, part)
-        H = nnls.hals_nnls_acc(UtM, UtU, slices.up(H), maxiter=100, delta=0.01, sparsity_coefficient=sparsity_coefficient,
+        H = nnls._hals_nnls_acc(UtM, UtU, slices.up(H), maxiter=100, delta=0.01, sparsity_coefficient=sparsity_coefficient,
                                normalize=normalize[1], nonzero=False)[0].cpu().numpy()
 
     couple_error = []

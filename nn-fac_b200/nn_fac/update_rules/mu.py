@@ -50,6 +50,7 @@ def mu_update_device(F, other, X, beta, which, K=None):
 
 
 def _out(t, like):
+    t = L.as_output(t)
     return t if isinstance(like, torch.Tensor) else t.cpu().numpy()
 
 

@@ -37,6 +37,12 @@ def hals_nnls_acc(UtM, UtU, in_V, maxiter=500, atime=None, alpha=0.5, delta=0.01
     UtM: r x n, UtU: at least r x r, in_V: at least r x n (only the first r rows are used,
     tests/nnls_tests.py:40-47).  An empty in_V triggers the least-squares start of nnls.py:138-145.
     """
+    V, eps, cnt, rho = _hals_nnls_acc(UtM, UtU, in_V, maxiter, delta, sparsity_coefficient, normalize, nonzero)
+    return L.as_output(V), eps, cnt, rho
+
+
+def _hals_nnls_acc(UtM, UtU, in_V, maxiter=500, delta=0.01, sparsity_coefficient=None, normalize=False, nonzero=False):
+    """hals_nnls_acc with V in the working dtype (callers that keep computing with it: parafac2)."""
     for name, arg in (("UtM", UtM), ("UtU", UtU), ("in_V", in_V)):
         if len(np.shape(arg)) != 2:                                        # nnls.py:130-135
             raise err.ArgumentException(
@@ -77,6 +83,12 @@ def hals_coupling_nnls_acc(UtM, UtU, in_V, Vtarget, mu, maxiter=500, atime=None,
     their diagonal entry is left at zero here, which is what makes the sweep skip them.  As for hals_nnls_acc, the
     deterministic stop rule always applies (`atime` / `alpha` are accepted and ignored); the reference raises ValueError
     (not ZeroColumnWhenUnautorized) for a zero column under `nonzero` (nnls.py:330)."""
+    V, eps, cnt, rho = _hals_coupling_nnls_acc(UtM, UtU, in_V, Vtarget, mu, maxiter, delta, normalize, nonzero)
+    return L.as_output(V), eps, cnt, rho
+
+
+def _hals_coupling_nnls_acc(UtM, UtU, in_V, Vtarget, mu, maxiter=500, delta=0.01, normalize=False, nonzero=False):
+    """hals_coupling_nnls_acc with V in the working dtype (parafac2)."""
     dt = L.resolve_dtype(UtM, UtU, in_V, Vtarget)
     b = L.to_device(UtM, dt)
     r, n = b.shape
