@@ -66,7 +66,8 @@ int64_t nnfac_ctx_launch_count(const nnfac_ctx* ctx);
  *   3. every rank: nnfac_ctx_board_attach(ctx, world, rank, handles ( world x 64 bytes, in rank order ))
  *   4. nnfac_ctx_collective(ctx, 1, slice_lengths ( columns of every rank's slice )) before a solve that is one slice
  *      of a joint solve -- every rank must make the same sequence of such solves -- and (ctx, 0, NULL) after it.
- * world <= 8.  Applies to the tensor-core sweep (fp32, rank <= 128: nnfac_nmf_plan_hals_solve, nnfac_hals_nnls).
+ * 1 <= world <= 8 (a group of one runs the same protocol on its own board; its results equal the plain solve's).
+ * Applies to the tensor-core sweep (fp32, rank <= 128: nnfac_nmf_plan_hals_solve, nnfac_hals_nnls).
  * -------------------------------------------------------------------------------------------*/
 int nnfac_ctx_board_export(nnfac_ctx* ctx, void* handle_out);
 int nnfac_ctx_board_attach(nnfac_ctx* ctx, int world, int rank, const void* handles);

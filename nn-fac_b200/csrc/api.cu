@@ -150,7 +150,8 @@ int nnfac_ctx_board_attach(nnfac_ctx* ctx, int world, int rank, const void* hand
 int nnfac_ctx_collective(nnfac_ctx* ctx, int on, const int64_t* slice_lengths) {
   NNFAC_ARG(ctx != nullptr, "nnfac_ctx_collective: ctx is NULL");
   if (!on) { ctx->collective = 0; return NNFAC_OK; }
-  NNFAC_ARG(ctx->peers.world > 1 && slice_lengths, "nnfac_ctx_collective: no peer group attached");
+  // a group of one is a group: its solves take the board protocol too (which is how that protocol is checked on one GPU)
+  NNFAC_ARG(ctx->peers.world >= 1 && slice_lengths, "nnfac_ctx_collective: no peer group attached");
   for (int q = 0; q < ctx->peers.world; ++q) ctx->collective_n[q] = slice_lengths[q];
   ctx->collective = 1;
   return NNFAC_OK;

@@ -141,7 +141,8 @@ struct TcSweepArgs {
   // Collective solve (several GPUs, one slice of the columns each): the stop test of nnls.py:156 sums the squared steps
   // over ALL columns.  Every CTA posts its partial on the board of every rank (peer-mapped memory, one 8-byte store
   // each over NVLink) and adds up all P x grid partials it finds on its own board, in (rank, CTA) order, so that every
-  // CTA of every GPU obtains the same bits.  xworld <= 1: single-GPU exchange through the private mailboxes above.
+  // CTA of every GPU obtains the same bits (a group of one GPU too).  xworld = 0: not collective, exchange through the private
+  // mailboxes above.
   int xworld, xrank;
   unsigned xgen;                              // collective call counter (host side, the same on every rank)
   unsigned long long* xboard[XMAXW];          // [q]: board of rank q as mapped here; [xrank]: the local one
@@ -338,7 +339,7 @@ __global__ void __launch_bounds__(Cfg<RP, MT, LAG>::NTHREADS, 1) tc_sweep_kernel
     constexpr unsigned MB = C::MBANKS;
     const unsigned nb = gridDim.x;
     const unsigned gen = *a.gen;
-    const bool collective = a.xworld > 1;
+    const bool collective = a.xworld > 0;
     for (unsigned e = 0;; ++e) {
       named_bar_sync(2, UPD_THREADS + 32);
       if (*s_quit) break;
@@ -576,7 +577,7 @@ __global__ void __launch_bounds__(Cfg<RP, MT, LAG>::NTHREADS, 1) tc_sweep_kernel
     unsigned epoch = 0;
     const unsigned nb = gridDim.x;
     const unsigned gen = *a.gen;
-    const bool collective = a.xworld > 1;
+    const bool collective = a.xworld > 0;
     // Stop test of nnls.py:156: it needs the sum of squared steps over ALL columns after every sweep.  Every CTA posts
     // its partial into the mailbox of every CTA (one 64-bit store each, tag | value) and adds the partials it receives
     // in a fixed order, so that all CTAs obtain the same bits and take the same decision.  While the partials travel,

@@ -125,12 +125,15 @@ def test_gram_matches_float64(r, length, dtype):
                                    rtol=1e-12 if dtype == "float64" else 3e-6)
 
 
+@pytest.mark.parametrize("x_source", ["planes", "f32"])
 @pytest.mark.parametrize("m,n,r", [(384, 320, 64), (1000, 500, 10), (777, 1300, 33)])
-def test_mu_finish_equals_reduce_apply_install(m, n, r):
+def test_mu_finish_equals_reduce_apply_install(m, n, r, x_source, monkeypatch):
     """The one-kernel finish of a beta=1 update (split partials -> ratio -> clamp -> planes) against the separate
-    reduce / mu_apply / set_factor kernels, both factors; then the next fused pass must see the new factor."""
+    reduce / mu_apply / set_factor kernels, both factors; then the next fused pass must see the new factor.  x_source: the beta = 1
+    pass rebuilds X from the bf16 planes (NNFAC_MU_F32=0, what runs when X is too large for the copies) or reads the fp32 copies."""
     import torch
     from nn_fac import _ops as ops
+    monkeypatch.setenv("NNFAC_MU_F32", "0" if x_source == "planes" else "1")
     rng = np.random.RandomState(m + n + r)
     U = (rng.rand(m, r) + 0.05).astype(np.float32)
     V = (rng.rand(r, n) + 0.05).astype(np.float32)
@@ -151,6 +154,7 @@ def test_mu_finish_equals_reduce_apply_install(m, n, r):
         a, ca = plans[0].fused(1 - which, 1)
         b, cb = plans[1].fused(1 - which, 1)
         assert torch.equal(a, b) and torch.equal(ca, cb)
+    assert all((p._xf32 is None) == (x_source == "planes") for p in plans)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -273,7 +277,7 @@ def test_plan_from_host_equals_plan_from_device(dtype):
         assert torch.equal(dev_plan.cross(which, F), host_plan.cross(which, F))
 
 
-def test_cross_reuses_installed_planes_and_f32_copies_change_nothing():
+def test_cross_reuses_installed_planes_and_f32_copies_change_nothing(monkeypatch):
     import torch
     from nn_fac import _ops as ops
     rng = np.random.RandomState(12)
@@ -286,7 +290,11 @@ def test_cross_reuses_installed_planes_and_f32_copies_change_nothing():
     plan.set_factor(1, V)
     assert torch.equal(plan.cross(1, None), plan.cross(1, Ut))
     assert torch.equal(plan.cross(0, None), plan.cross(0, V))
+    # the reference reads X from the bf16 planes: without NNFAC_MU_F32=0 the first beta = 1 pass would make the fp32 copies itself
+    # and the comparison below would be the copy path against itself
+    monkeypatch.setenv("NNFAC_MU_F32", "0")
     ref = [(o.clone(), c.clone()) for o, c in (plan.fused(0, 1), plan.fused(1, 1))]
+    assert plan._xf32 is None
     plan.enable_f32()
     for side in (0, 1):
         out, cost = plan.fused(side, 1)
