@@ -80,12 +80,16 @@ int nnfac_ctx_sweep_variant(nnfac_ctx* ctx, int mode);
 
 /* ---------------------------------------------------------------------------------------------
  * Exchange steps of the column-sharded path over peer-mapped memory (new; csrc/peer_xchg.cu).  Every rank owns a region
- * [flags | stage: r x pitch | send: r x pitch'] in device memory, exported with CUDA IPC and mapped by its peers like the boards
- * above (create -> export -> exchange handles -> attach).  A rank writes its partial result into its own stage buffer (the X
- * pass' reduction goes straight there), posts; every rank then pulls and sums ITS columns out of all stages over NVLink
- * (reduce-scatter + reduction in one kernel, fixed order).  After the slice solves into the send buffers and a second post,
- * nnfac_nmf_plan_set_factor_pulled reads all slices from the peers' send buffers while it builds the operand planes
- * (all-gather + install in one kernel).  phase 0 = stage, 1 = send; every rank must make the same sequence of calls.
+ * [flags | stage | send] in device memory, exported with CUDA IPC and mapped by its peers like the boards above
+ * (create -> export -> exchange handles -> attach).  The stage buffer (phase 0) is laid out
+ * [tail block: r x tail_pitch | inbox: (world * splits) slabs of r_pad x chunk]: with nnfac_nmf_plan_set_push (below) the fused
+ * pass of rank p writes the partial of every row tile straight into slab (p * splits + split) of the inbox of the rank that owns
+ * those rows of U, over NVLink, from its own epilogue -- the reduce-scatter is part of the X pass -- and the tail block carries
+ * the rank's own small partial sums (Gram of V, row sums of V).  After its post on phase 0 a rank finds every partial of its
+ * rows in local memory.  The slice results go into the send buffer (phase 1, [r x pitch]: the slice, its Gram behind it); after
+ * a second post nnfac_nmf_plan_set_factor_pulled reads all slices from the peers' send buffers while it builds the operand
+ * planes (all-gather + install in one kernel).  The consumers wait for every rank's post themselves; every rank must make the
+ * same sequence of calls.
  * -------------------------------------------------------------------------------------------*/
 typedef struct nnfac_xchg nnfac_xchg;
 int nnfac_xchg_create(nnfac_ctx* ctx, int64_t stage_floats, int64_t send_floats, nnfac_xchg** out);
@@ -94,29 +98,18 @@ int nnfac_xchg_attach(nnfac_xchg* x, int world, int rank, const void* handles);
 int nnfac_xchg_destroy(nnfac_xchg* x);
 void* nnfac_xchg_ptr(nnfac_xchg* x, int which);                 /* local stage (0) / send (1) buffer */
 int nnfac_xchg_post(nnfac_xchg* x, int phase, void* stream);    /* this rank's buffer `phase` is complete (stream-ordered) */
-int nnfac_xchg_wait(nnfac_xchg* x, int phase, void* stream);    /* every rank has posted as often as this rank (a kernel of its
-                                                                   own; the consumers below wait by themselves) */
 /* nnfac_xchg_post(x, 0) that first writes column `col` of the stage ([rows x pitch]) from tail_src[0 .. rows): the small partial
- * sums that travel behind the big ones (row sums of V, mu.py:85-87) without a copy kernel of their own. */
+ * sums that travel with the post (row sums of V, mu.py:85-87, in column 0 of the tail block) without a copy kernel of their own. */
 int nnfac_xchg_post_tail(nnfac_xchg* x, const float* tail_src, int rows, int64_t pitch, int64_t col, void* stream);
-/* out[k][0:ncols] = sum over ranks of columns [lo, lo+ncols) and out[k][tail_col : tail_col+tail] = sum over ranks of the
- * `tail` columns behind column `len`, of every rank's buffer `which` ([r x pitch]).  Call after this rank's post on `which`;
- * the kernel waits until every rank has posted as often (no nnfac_xchg_wait needed). */
-int nnfac_xchg_pull_reduce(nnfac_xchg* x, int which, float* out, int64_t ld_out, int r, int64_t pitch, int64_t lo, int64_t ncols,
-                           int64_t len, int tail, int64_t tail_col, void* stream);
-/* The U update of the column-sharded beta = 1 rule (nn_fac/update_rules/mu.py:84-88) in ONE kernel after this rank's post on
- * phase 0: waits for every rank's post, sums the partial numerators of this rank's rows [lo, lo+ncols) of U and the partial row
- * sums of V (column `len` of every stage) over NVLink in rank order, and writes max(F[k][lo+c] * num / den[k], floor) into this
+/* out[k][j] = sum over the ranks, in rank order, of element k * pitch + col + j of every rank's buffer `which` ([r x pitch];
+ * k < r, j < tail): the partial Grams in the tail blocks (which = 0, pitch = tail_pitch, col = 0), the slices' Grams behind the
+ * slices in the send buffers (which = 1, col = chunk).  Call after this rank's post on `which`; the kernel waits until every
+ * rank has posted as often. */
+int nnfac_xchg_pull_tail(nnfac_xchg* x, int which, float* out, int64_t ld_out, int r, int64_t pitch, int64_t col, int tail, void* stream);
+/* The beta = 1 update (nn_fac/update_rules/mu.py:84-88) of this rank's rows of U from the inbox: waits for every rank's post on
+ * phase 0, sums the slabs in slab order and the partial row sums of V (column 0 of every rank's tail block, nnfac_xchg_post_tail
+ * with pitch = tail_pitch, col = 0), writes max(F[k][lo+c] * num / den[k], floor) for the rows [lo, lo + ncols) of U^T into this
  * rank's send buffer ([r x ld_send]).  F = the current U^T (r x ld_f). */
-int nnfac_xchg_pull_mu_apply(nnfac_xchg* x, const float* F, int64_t ld_f, int r, int64_t pitch, int64_t lo, int64_t ncols,
-                             int64_t len, double floor_value, int64_t ld_send, void* stream);
-/* PUSH variant of the U-side exchange (nnfac_nmf_plan_set_push below): the stage buffer of every rank is laid out
- * [tail block: r x tail_pitch | inbox: (world * splits) slabs of r_pad x chunk]; the fused pass of rank p writes the partial
- * of every row tile straight into slab (p * splits + split) of the inbox of the rank that owns those rows of U, over NVLink,
- * from its own epilogue -- the reduce-scatter is part of the X pass.  After its post on phase 0 a rank finds every partial of its
- * rows in local memory.  nnfac_xchg_inbox_mu_apply = the beta = 1 update (mu.py:84-88) from the inbox: waits for every rank's
- * post, sums the slabs in slab order and the partial row sums of V (column 0 of every rank's tail block, nnfac_xchg_post_tail
- * with pitch = tail_pitch, col = 0), writes the new rows [lo, lo + ncols) of U^T into this rank's send buffer. */
 int nnfac_xchg_inbox_mu_apply(nnfac_xchg* x, int64_t inbox_off, int nslabs, int64_t slab_stride, int64_t chunk, int64_t tail_pitch,
                               const float* F, int64_t ld_f, int r, int64_t lo, int64_t ncols, double floor_value, int64_t ld_send,
                               void* stream);

@@ -5,17 +5,18 @@
 // every rank needs all slices (an all-gather).  With NCCL each of the two costs 0.1-0.2 ms at C2 on 8 GPUs whatever the
 // size (16.8 MB): launch + protocol latency.  Here every rank owns an exchange region in device memory (cudaMalloc,
 // exported with CUDA IPC, mapped by every peer):
-//     [ flags | stage: r x (len + t) | send: r x (chunk + t) ]
-// * the X pass' reduction kernel writes the rank's partial result straight into its own `stage` (tail columns: the partial
-//   Gram / row sums), then `post` raises a sequence number in every peer's flag block (one st.release.sys each);
-// * `pull_reduce` waits for the flags and sums, in rank order, the columns this rank owns out of all P stages -- loads over
-//   NVLink, the reduce-scatter and the reduction in ONE kernel, deterministic;
-// * the slice solve writes into `send`; after the next `post`, the kernel that installs the new factor in the plan reads the
-//   P slices directly from the peers' `send` regions (nnfac_nmf_plan_set_factor_pulled): the all-gather, the un-permute and
-//   the operand-plane construction in ONE kernel.
-// Nothing is overwritten early: a rank rewrites its stage only after its own install, which waited for every peer's second
-// post (hence for every peer's pull); it rewrites its send only after its own pull of the next iteration, which waited for
-// every peer's first post of that iteration (hence for every peer's install).
+//     [ flags | stage: tail block r x tpad, inbox (P * splits) x r_pad x chunk | send: r x (chunk + tpad) ]
+// * the fused X pass of every rank writes its partial of each row tile straight into the inbox of the rank that owns those
+//   rows of U (nnfac_nmf_plan_set_push, tc_fused.cu); the rank's small partial sums (Gram / row sums of V) go into its own tail
+//   block; then `post` raises a sequence number in every peer's flag block (one st.release.sys each);
+// * the consumers wait for the flags themselves: the slice solve and `inbox_mu_apply` add the slabs of the local inbox in slab
+//   order, `pull_tail` sums the tail blocks of all P ranks in rank order over NVLink -- deterministic;
+// * the slice solve writes into `send` (the slice's Gram behind it); after the next `post`, the kernel that installs the new
+//   factor in the plan reads the P slices directly from the peers' `send` regions (nnfac_nmf_plan_set_factor_pulled): the
+//   all-gather, the un-permute and the operand-plane construction in ONE kernel.
+// Nothing is overwritten early: a rank writes into the inboxes and its tail block again only after its own install, which
+// waited for every peer's second post (hence for every peer's solve and tail pull); it rewrites its send only after its own
+// wait on the first posts of the next iteration (hence after every peer's install and Gram pull).
 #include <stdlib.h>
 #include <string.h>
 
@@ -69,22 +70,7 @@ __device__ __forceinline__ void xchg_block_wait(const unsigned long long* flags,
   }
 }
 
-__global__ void xchg_wait_kernel(const unsigned long long* flags, int world, int phase, unsigned long long seq) {
-  if ((int)threadIdx.x < world) {
-    const unsigned long long* f = flags + phase * NNFAC_MAX_PEERS + threadIdx.x;
-    unsigned long long v;
-    unsigned long long spins = 0;
-    do {
-      asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(f) : "memory");
-      if (++spins > (1ull << 27)) __trap();     // ~1 minute: a protocol bug fails the launch instead of hanging the GPU
-    } while (v < seq);
-  }
-}
-
-// out[k][c] = sum_q src_q[k * pitch + lo + c]  (c < ncols; columns ncols .. out_cols-1-tail are zero padding), and
-// out[k][tail_col + j] = sum_q src_q[k * pitch + len + j]  (j < tail); fixed order q = 0 .. world-1.
-// (the kernels wait for every rank's post themselves; the loads of all ranks are issued together -- 16 bytes each where the
-// layout allows -- and added in rank order)
+// sum_q src_q[off] in the fixed order q = 0 .. world-1 (the loads of all ranks are issued together)
 __device__ __forceinline__ float pull_sum(const PeerPtrs& src, int world, int64_t off) {
   float v[NNFAC_MAX_PEERS];
 #pragma unroll
@@ -94,102 +80,23 @@ __device__ __forceinline__ float pull_sum(const PeerPtrs& src, int world, int64_
   for (int q = 0; q < NNFAC_MAX_PEERS; ++q) if (q < world) s += v[q];
   return s;
 }
-__device__ __forceinline__ float4 pull_sum4(const PeerPtrs& src, int world, int64_t off) {   // off: multiple of 4 floats
-  float4 v[NNFAC_MAX_PEERS];
-#pragma unroll
-  for (int q = 0; q < NNFAC_MAX_PEERS; ++q)
-    v[q] = q < world ? __ldcv(reinterpret_cast<const float4*>(src.p[q] + off)) : make_float4(0.f, 0.f, 0.f, 0.f);
-  float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-  for (int q = 0; q < NNFAC_MAX_PEERS; ++q)
-    if (q < world) { s.x += v[q].x; s.y += v[q].y; s.z += v[q].z; s.w += v[q].w; }
-  return s;
-}
 
-constexpr int PULL_QUADS = 2;      // 4-column groups per thread and step: 2 x world 16-byte loads in flight per thread
-
-// grid = (column blocks, r).  vec: pitch, lo, ld_out and the base pointers allow 16-byte accesses.
-__global__ void __launch_bounds__(256) xchg_pull_reduce_kernel(PeerPtrs src, int world, int r, int64_t pitch, int64_t lo, int64_t ncols,
-                                                               int64_t len, int tail, float* __restrict__ out, int64_t ld_out,
-                                                               int64_t tail_col, const unsigned long long* flags, int phase,
-                                                               unsigned long long seq, int vec) {
+// out[k][j] = sum_q src_q[k * pitch + col + j]  (j < tail), after waiting for every rank's post.  grid = r.
+__global__ void __launch_bounds__(256) xchg_pull_tail_kernel(PeerPtrs src, int world, int64_t pitch, int64_t col, int tail,
+                                                             float* __restrict__ out, int64_t ld_out, const unsigned long long* flags,
+                                                             int phase, unsigned long long seq) {
   xchg_block_wait(flags, world, phase, seq);
-  const int64_t k = blockIdx.y;
-  const int64_t row = k * pitch;
-  // tail columns and the zero padding between the slice and the tail: first block of the row
-  if (blockIdx.x == 0) {
-    for (int64_t c = ncols + threadIdx.x; c < tail_col; c += blockDim.x) out[k * ld_out + c] = 0.f;
-    for (int j = threadIdx.x; j < tail; j += blockDim.x) out[k * ld_out + tail_col + j] = pull_sum(src, world, row + len + j);
-  }
-  const int64_t nquad = (ncols + 3) / 4;
-  for (int64_t q0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * PULL_QUADS; q0 < nquad; q0 += (int64_t)gridDim.x * blockDim.x * PULL_QUADS) {
-    float4 acc[PULL_QUADS];
-    bool full[PULL_QUADS];
-#pragma unroll
-    for (int u = 0; u < PULL_QUADS; ++u) {
-      const int64_t c = (q0 + u) * 4;
-      full[u] = vec && c + 4 <= ncols;
-      if (full[u]) acc[u] = pull_sum4(src, world, row + lo + c);
-    }
-#pragma unroll
-    for (int u = 0; u < PULL_QUADS; ++u) {
-      const int64_t c = (q0 + u) * 4;
-      if (full[u]) {
-        *reinterpret_cast<float4*>(out + k * ld_out + c) = acc[u];
-      } else {
-        for (int64_t cc = c; cc < c + 4 && cc < ncols; ++cc) out[k * ld_out + cc] = pull_sum(src, world, row + lo + cc);
-      }
-    }
-  }
+  const int64_t k = blockIdx.x;
+  for (int j = threadIdx.x; j < tail; j += blockDim.x) out[k * ld_out + j] = pull_sum(src, world, k * pitch + col + j);
 }
 
-// beta = 1 multiplicative update of this rank's rows of U (mu.py:84-88) straight out of the stages: numerator = sum over the
-// ranks of their partial numerators (columns lo .. lo+ncols of the stage), denominator = sum of their partial row sums of V
-// (column `len`); send[k][c] = max(F[k][lo + c] * (num / den[k]), floor), NaN propagating like numpy.  grid = (column blocks, r).
+// beta = 1 multiplicative update (mu.py:84-88): max(f * (num / den), floor), NaN propagating like numpy
 __device__ __forceinline__ float mu_rule(float f, float num, float den, float floor_value) {
   const float v = f * (num / den);
   return v != v ? v : (v > floor_value ? v : floor_value);
 }
-__global__ void __launch_bounds__(256) xchg_pull_mu_apply_kernel(PeerPtrs src, int world, int r, int64_t pitch, int64_t lo, int64_t ncols,
-                                                                 int64_t len, const float* __restrict__ F, int64_t ld_f, float floor_value,
-                                                                 float* __restrict__ send, int64_t ld_send,
-                                                                 const unsigned long long* flags, unsigned long long seq, int vec) {
-  __shared__ float den_s;
-  xchg_block_wait(flags, world, 0, seq);
-  const int64_t k = blockIdx.y;
-  const int64_t row = k * pitch;
-  if (threadIdx.x == 0) den_s = pull_sum(src, world, row + len);
-  __syncthreads();
-  const float den = den_s;
-  const int64_t nquad = (ncols + 3) / 4;
-  for (int64_t q0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * PULL_QUADS; q0 < nquad; q0 += (int64_t)gridDim.x * blockDim.x * PULL_QUADS) {
-    float4 num[PULL_QUADS], f[PULL_QUADS];
-    bool full[PULL_QUADS];
-#pragma unroll
-    for (int u = 0; u < PULL_QUADS; ++u) {
-      const int64_t c = (q0 + u) * 4;
-      full[u] = vec && c + 4 <= ncols;
-      if (full[u]) {
-        num[u] = pull_sum4(src, world, row + lo + c);
-        f[u] = *reinterpret_cast<const float4*>(F + k * ld_f + lo + c);
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < PULL_QUADS; ++u) {
-      const int64_t c = (q0 + u) * 4;
-      if (full[u]) {
-        *reinterpret_cast<float4*>(send + k * ld_send + c) =
-            make_float4(mu_rule(f[u].x, num[u].x, den, floor_value), mu_rule(f[u].y, num[u].y, den, floor_value),
-                        mu_rule(f[u].z, num[u].z, den, floor_value), mu_rule(f[u].w, num[u].w, den, floor_value));
-      } else {
-        for (int64_t cc = c; cc < c + 4 && cc < ncols; ++cc)
-          send[k * ld_send + cc] = mu_rule(F[k * ld_f + lo + cc], pull_sum(src, world, row + lo + cc), den, floor_value);
-      }
-    }
-  }
-}
 
-// The same update when the partial numerators were PUSHED into this rank's inbox by the peers' fused passes
+// The update of this rank's rows of U when the partial numerators were PUSHED into this rank's inbox by the peers' fused passes
 // (nnfac_nmf_plan_set_push): numerator = sum of the nslabs local slabs [r_pad x chunk] in slab order (rank-major, then split),
 // denominator = sum over the ranks of column 0 of their tail blocks ([r x tail_pitch] at the start of every stage, read over
 // NVLink: r floats per rank).  grid = (column blocks, r).
@@ -323,51 +230,20 @@ void nnfac_xchg_wait_args(const nnfac_xchg* x, int phase, const unsigned long lo
   *seq = x->seq[phase];
 }
 
-// every rank has made as many posts on `phase` as this rank (call after the own post)
-int nnfac_xchg_wait(nnfac_xchg* x, int phase, void* stream) {
-  NNFAC_ARG(x && (phase == 0 || phase == 1), "nnfac_xchg_wait: bad argument");
-  xchg_wait_kernel<<<1, 32, 0, (cudaStream_t)stream>>>((const unsigned long long*)x->region, x->world, phase, x->seq[phase]);
-  NNFAC_LAUNCH_CHECK(x->ctx);
-  return NNFAC_OK;
-}
-
-// Sum over the ranks of the columns [lo, lo + ncols) and of the `tail` columns behind column `len` of every rank's buffer
-// `which` ([r x pitch] each): out (r x ld_out) receives the columns at 0 and the tail at tail_col.  Call after this rank's
-// nnfac_xchg_post(x, which): the kernel itself waits until every rank has posted as often.
-int nnfac_xchg_pull_reduce(nnfac_xchg* x, int which, float* out, int64_t ld_out, int r, int64_t pitch, int64_t lo, int64_t ncols,
-                           int64_t len, int tail, int64_t tail_col, void* stream) {
-  NNFAC_ARG(x && out && (which == 0 || which == 1) && r > 0 && ncols >= 0 && tail >= 0 && tail_col >= ncols && ld_out >= tail_col + tail &&
-                lo >= 0 && lo + ncols <= len && len + tail <= pitch, "nnfac_xchg_pull_reduce: bad argument");
-  PeerPtrs src;
+// out[k][j] = sum over the ranks, in rank order, of element k * pitch + col + j of their buffer `which` ([r x pitch] each;
+// k < r, j < tail).  Call after this rank's nnfac_xchg_post(x, which): the kernel itself waits until every rank has posted as
+// often.
+int nnfac_xchg_pull_tail(nnfac_xchg* x, int which, float* out, int64_t ld_out, int r, int64_t pitch, int64_t col, int tail,
+                         void* stream) {
+  NNFAC_ARG(x && out && (which == 0 || which == 1) && r > 0 && tail > 0 && ld_out >= tail && col >= 0 && col + tail <= pitch,
+            "nnfac_xchg_pull_tail: bad argument");
   const size_t off = which == 0 ? x->stage_off : x->send_off;
-  for (int q = 0; q < NNFAC_MAX_PEERS; ++q) src.p[q] = q < x->world ? (const float*)((const char*)x->peer[q] + off) : nullptr;
-  int64_t gx = ceil_div64(ceil_div64(ncols, 4 * PULL_QUADS), 256);
-  if (gx < 1) gx = 1;
-  const int vec = pitch % 4 == 0 && lo % 4 == 0 && ld_out % 4 == 0 && ((uintptr_t)out & 15) == 0 && (off & 15) == 0;
-  xchg_pull_reduce_kernel<<<dim3((unsigned)gx, (unsigned)r), 256, 0, (cudaStream_t)stream>>>(
-      src, x->world, r, pitch, lo, ncols, len, tail, out, ld_out, tail_col, (const unsigned long long*)x->region, which, x->seq[which], vec);
-  NNFAC_LAUNCH_CHECK(x->ctx);
-  return NNFAC_OK;
-}
-
-// The U update of the column-sharded beta = 1 rule over peer memory (mu.py:84-88), after this rank's post on phase 0: waits for
-// every rank's post, sums the partial numerators of this rank's rows [lo, lo + ncols) of U and the partial row sums of V
-// (column `len` of every stage, [r x pitch] each) over NVLink in rank order, applies the update to F[:, lo : lo + ncols]
-// (F: r x ld_f, the current U^T) and writes the new slice into this rank's send buffer ([r x ld_send], ld_send = chunk + tail).
-int nnfac_xchg_pull_mu_apply(nnfac_xchg* x, const float* F, int64_t ld_f, int r, int64_t pitch, int64_t lo, int64_t ncols, int64_t len,
-                             double floor_value, int64_t ld_send, void* stream) {
-  NNFAC_ARG(x && F && r > 0 && ncols >= 0 && lo >= 0 && lo + ncols <= len && len < pitch && ld_f >= len && ld_send >= ncols,
-            "nnfac_xchg_pull_mu_apply: bad argument");
-  NNFAC_ARG((size_t)r * (size_t)ld_send * sizeof(float) <= x->bytes - x->send_off, "nnfac_xchg_pull_mu_apply: beyond the send buffer");
-  if (ncols == 0) return NNFAC_OK;
+  const size_t end = which == 0 ? x->send_off : x->bytes;
+  NNFAC_ARG((size_t)r * (size_t)pitch * sizeof(float) <= end - off, "nnfac_xchg_pull_tail: beyond the buffer");
   PeerPtrs src;
-  for (int q = 0; q < NNFAC_MAX_PEERS; ++q) src.p[q] = q < x->world ? (const float*)((const char*)x->peer[q] + x->stage_off) : nullptr;
-  const int64_t gx = ceil_div64(ceil_div64(ncols, 4 * PULL_QUADS), 256);
-  const int vec = pitch % 4 == 0 && lo % 4 == 0 && ld_f % 4 == 0 && ld_send % 4 == 0 && ((uintptr_t)F & 15) == 0 &&
-                  (x->stage_off & 15) == 0 && (x->send_off & 15) == 0;
-  xchg_pull_mu_apply_kernel<<<dim3((unsigned)gx, (unsigned)r), 256, 0, (cudaStream_t)stream>>>(
-      src, x->world, r, pitch, lo, ncols, len, F, ld_f, (float)floor_value, (float*)((char*)x->region + x->send_off), ld_send,
-      (const unsigned long long*)x->region, x->seq[0], vec);
+  for (int q = 0; q < NNFAC_MAX_PEERS; ++q) src.p[q] = q < x->world ? (const float*)((const char*)x->peer[q] + off) : nullptr;
+  xchg_pull_tail_kernel<<<(unsigned)r, 256, 0, (cudaStream_t)stream>>>(src, x->world, pitch, col, tail, out, ld_out,
+                                                                       (const unsigned long long*)x->region, which, x->seq[which]);
   NNFAC_LAUNCH_CHECK(x->ctx);
   return NNFAC_OK;
 }

@@ -12,10 +12,12 @@ cost-only pass closes the last iteration.
 
 Several GPUs (one process each): X is sharded by COLUMNS.  Rank p holds X_p (m x n_p) and V_p (r x n_p);
 U is replicated.  Per outer iteration there is one exchange step on each side of the U update:
-  * the partial cross products of the first pass (V_p X_p^T, r x m) and the partial Gram V_p V_p^T are
-    summed with one all-reduce (HALS), or the partial MU numerator and the partial row sums of V (MU);
-  * for HALS the U solve is split by rows of U (columns of U^T): every rank sweeps its own m/P slice and
-    the slices are all-gathered, so the solve shrinks with P instead of being repeated on every rank.
+  * the partial cross products of the first pass (V_p X_p^T, r x m) and the partial Gram V_p V_p^T (HALS), or the partial
+    MU numerator and the partial row sums of V (MU), are summed, every rank receiving only the rows of U it updates: the
+    fused pass of every rank writes its partials straight into the owners' inboxes in peer-mapped memory (PeerExchange);
+  * the U update is split by rows of U (columns of U^T): every rank solves / updates its own m/P slice and the install
+    kernel reads all slices from their owners' send buffers, so the solve shrinks with P instead of being repeated on every
+    rank.  Without peer access the same steps run as NCCL collectives (reduce-scatter / all-reduce, all-gather).
 The V side needs no exchange of factor data.  The HALS stop test (nnls.py:156) sums the squared steps over ALL columns
 of a solve, also when they are spread over several GPUs: the sweep kernels of all ranks exchange their partial sums once per
 sweep through peer-mapped "boards" (8-byte stores over NVLink, csrc/tc_sweep.cu), so a sharded solve stops after exactly
@@ -228,28 +230,23 @@ class _RawView:
 
 
 class PeerExchange:
-    """The U-side exchange of the sharded path over peer-mapped memory instead of NCCL (csrc/peer_xchg.cu): every rank's stage
-    buffer [r x (m + t)] receives its partial cross product / numerator (+ t tail columns: partial Gram or row sums), a pull
-    kernel sums this rank's columns out of all stages over NVLink, the slice results go to the send buffers [r x (chunk + t)],
+    """The U-side exchange of the sharded path over peer-mapped memory instead of NCCL (csrc/peer_xchg.cu).  Every rank's stage
+    buffer is [tail block r x tpad | inbox (world * splits) x r_pad x chunk]: the peers' fused passes write their partials of this
+    rank's rows of U straight into the inbox (nnfac_nmf_plan_set_push), the first t columns of the tail block carry this rank's
+    partial Gram or row sums.  The slice results go to the send buffers [r x (chunk + tpad)] (the slice's Gram behind the slice),
     and the install kernel reads all slices from the peers' send buffers.  One region per FusedNMF state."""
 
-    def __init__(self, comm, device, r, m, chunk, tail, push=None):
-        """push = (splits, r_pad): PUSH layout of the stage buffer, [tail block r x tpad | inbox (world * splits) x r_pad x chunk]:
-        the peers' fused passes write their partials of this rank's rows straight into the inbox (nnfac_nmf_plan_set_push); else
-        the stage holds this rank's own r x (m + tpad) partial result and the owners pull their columns out of it."""
+    def __init__(self, comm, device, r, chunk, tail, splits):
+        """splits: split-K partials per row tile of the fused pass over side 0 (the inbox holds world * splits slabs)."""
         lib = L.load_library()
-        self.comm, self.device, self.r, self.m, self.chunk, self.tail = comm, device, r, m, chunk, tail
+        self.comm, self.device, self.r, self.chunk, self.tail = comm, device, r, chunk, tail
         self.tpad = -(-tail // 4) * 4                 # row pitches stay multiples of 4 floats: 16-byte loads over NVLink
-        self.push = push
+        self.r_pad = -(-r // 16) * 16
+        self.nslabs, self.slab_stride = comm.world * splits, self.r_pad * chunk
+        self.inbox_off = r * self.tpad
         self.handle = ctypes.c_void_p()
-        if push is not None:
-            splits, r_pad = push
-            self.nslabs, self.r_pad, self.slab_stride = comm.world * splits, r_pad, r_pad * chunk
-            self.inbox_off = r * self.tpad
-            stage_floats = self.inbox_off + self.nslabs * self.slab_stride
-        else:
-            stage_floats = r * (m + self.tpad)
-        L.check(lib.nnfac_xchg_create(L.ctx(device), stage_floats, r * (chunk + self.tpad), ctypes.byref(self.handle)))
+        L.check(lib.nnfac_xchg_create(L.ctx(device), self.inbox_off + self.nslabs * self.slab_stride, r * (chunk + self.tpad),
+                                      ctypes.byref(self.handle)))
         mine = (ctypes.c_ubyte * 64)()
         L.check(lib.nnfac_xchg_export(self.handle, mine))
         send = torch.tensor(list(mine), dtype=torch.uint8, device=device)
@@ -257,50 +254,35 @@ class PeerExchange:
         comm.dist.all_gather_into_tensor(recv, send, group=comm.group)
         handles = (ctypes.c_ubyte * (64 * comm.world))(*recv.cpu().tolist())
         L.check(lib.nnfac_xchg_attach(self.handle, comm.world, comm.rank, handles))
-        if push is not None:
-            base = lib.nnfac_xchg_ptr(self.handle, 0)
-            self.stage = None
-            self.tailblk = torch.as_tensor(_RawView(base, (r, self.tpad)), device=device)
-            self.inbox = torch.as_tensor(_RawView(base + 4 * self.inbox_off, (self.nslabs, self.r_pad, chunk)), device=device)
-            self._scratch = None
-        else:
-            self.stage = torch.as_tensor(_RawView(lib.nnfac_xchg_ptr(self.handle, 0), (r, m + self.tpad)), device=device)
+        base = lib.nnfac_xchg_ptr(self.handle, 0)
+        self.tailblk = torch.as_tensor(_RawView(base, (r, self.tpad)), device=device)
+        self.inbox = torch.as_tensor(_RawView(base + 4 * self.inbox_off, (self.nslabs, self.r_pad, chunk)), device=device)
+        self._scratch = None
         self.send = torch.as_tensor(_RawView(lib.nnfac_xchg_ptr(self.handle, 1), (r, chunk + self.tpad)), device=device)
         comm.dist.barrier(group=comm.group)              # every region is mapped everywhere before anybody posts
 
     def post(self, phase):
         L.check(L.load_library().nnfac_xchg_post(self.handle, phase, L.stream_ptr()))
 
-    def post_tail(self, vec, length):
-        """post(0) that first writes `vec` (r values) into column `length` of the stage -- PUSH layout: into column 0 of the tail
-        block (one kernel)."""
-        if self.push is not None:
-            L.check(L.load_library().nnfac_xchg_post_tail(self.handle, L.ptr(vec), self.r, self.tpad, 0, L.stream_ptr()))
-        else:
-            L.check(L.load_library().nnfac_xchg_post_tail(self.handle, L.ptr(vec), self.r, length + self.tpad, length, L.stream_ptr()))
+    def post_tail(self, vec):
+        """post(0) that first writes `vec` (r values) into column 0 of the tail block (one kernel)."""
+        L.check(L.load_library().nnfac_xchg_post_tail(self.handle, L.ptr(vec), self.r, self.tpad, 0, L.stream_ptr()))
 
     def attach_plan(self, plan):
-        """PUSH layout: the fused passes of `plan` over side 0 that keep their partials write them into the owners' inboxes."""
+        """The fused passes of `plan` over side 0 that keep their partials write them into the owners' inboxes."""
         slabs, stride = ctypes.c_int(), ctypes.c_int64()
         L.check(L.load_library().nnfac_nmf_plan_set_push(plan.handle, self.handle, self.inbox_off, self.chunk, ctypes.byref(slabs),
                                                          ctypes.byref(stride)))
         assert slabs.value == self.nslabs and stride.value == self.slab_stride, (slabs.value, stride.value, self.nslabs, self.slab_stride)
 
-    def pull_tail0(self):
-        """PUSH layout: sum over the ranks of the first `tail` columns of their tail blocks -> (r x tail) (after post(0); waits)."""
-        out = torch.empty((self.r, self.tail), dtype=torch.float32, device=self.device)
-        L.check(L.load_library().nnfac_xchg_pull_reduce(self.handle, 0, L.ptr(out), out.stride(0), self.r, self.tpad, 0, 0, 0, self.tail, 0,
-                                                        L.stream_ptr()))
-        return out
-
     def inbox_mu_apply(self, Ft, lo, ncols, floor):
-        """PUSH layout: mu.py:84-88 for this rank's rows of U from the inbox (local) and the peers' tail blocks -> send buffer."""
+        """mu.py:84-88 for this rank's rows of U from the inbox (local) and the peers' tail blocks -> send buffer."""
         L.check(L.load_library().nnfac_xchg_inbox_mu_apply(self.handle, self.inbox_off, self.nslabs, self.slab_stride, self.chunk, self.tpad,
                                                            L.ptr(Ft), Ft.stride(0), self.r, lo, ncols, float(floor), self.chunk + self.tpad,
                                                            L.stream_ptr()))
 
     def inbox_sum(self, ncols):
-        """PUSH layout: the plain sum of the slabs of the inbox -> (r x ncols) (after a kernel that waited for the posts)."""
+        """The plain sum of the slabs of the inbox -> (r x ncols) (after a kernel that waited for the posts)."""
         out = torch.empty((self.r, ncols), dtype=torch.float32, device=self.device)
         L.check(L.load_library().nnfac_reduce_slabs_f32(L.ctx(self.device), L.ptr(self.inbox), self.chunk, self.nslabs, self.r, self.r_pad,
                                                         ncols, L.ptr(out), out.stride(0), L.stream_ptr()))
@@ -311,30 +293,12 @@ class PeerExchange:
             self._scratch = torch.empty(r * n, dtype=torch.float32, device=self.device)
         return self._scratch
 
-    def wait(self, phase):
-        """A wait kernel of its own -- not needed before pull_reduce / pull_mu_apply / install, which wait by themselves."""
-        L.check(L.load_library().nnfac_xchg_wait(self.handle, phase, L.stream_ptr()))
-
-    def pull_mu_apply(self, Ft, lo, ncols, length, floor):
-        """mu.py:84-88 for this rank's rows of U straight out of all stages into the send buffer (after post(0); one kernel:
-        wait + reduce-scatter + reduction + update)."""
-        L.check(L.load_library().nnfac_xchg_pull_mu_apply(self.handle, L.ptr(Ft), Ft.stride(0), self.r, length + self.tpad, lo, ncols,
-                                                          length, float(floor), self.chunk + self.tpad, L.stream_ptr()))
-
-    def pull_reduce(self, phase, lo, ncols, length):
-        """Sum over the ranks of columns [lo, lo + ncols) and of the tail of every rank's buffer `phase` -> (r x (chunk + tail))
-        with the tail at column chunk (after post; the kernel waits for the other ranks' posts itself)."""
-        out = torch.empty((self.r, self.chunk + self.tail), dtype=torch.float32, device=self.device)
-        pitch = length + self.tpad
-        L.check(L.load_library().nnfac_xchg_pull_reduce(self.handle, phase, L.ptr(out), out.stride(0), self.r, pitch, lo, ncols, length,
-                                                        self.tail, self.chunk, L.stream_ptr()))
-        return out
-
     def pull_tail(self, phase, length):
-        """Only the sum of the tails of every rank's buffer `phase` -> (r x tail)."""
+        """Sum over the ranks of the `tail` columns behind column `length` of every rank's buffer `phase` ([r x (length + tpad)])
+        -> (r x tail) (after post(phase); waits).  (0, 0): the partial Grams in the tail blocks; (1, chunk): the slices' Grams."""
         out = torch.empty((self.r, self.tail), dtype=torch.float32, device=self.device)
-        L.check(L.load_library().nnfac_xchg_pull_reduce(self.handle, phase, L.ptr(out), out.stride(0), self.r, length + self.tpad, 0, 0,
-                                                        length, self.tail, 0, L.stream_ptr()))
+        L.check(L.load_library().nnfac_xchg_pull_tail(self.handle, phase, L.ptr(out), out.stride(0), self.r, length + self.tpad, length,
+                                                      self.tail, L.stream_ptr()))
         return out
 
     def install(self, plan, which, length):
@@ -377,8 +341,8 @@ class CudaEngine:
             return new
         return self.plan.mu_finish(which, F, den_vec, mu.epsilon)
 
-    def cross(self, which, F, keep_partials=False):
-        return self.plan.cross(which, F, keep_partials=keep_partials)
+    def cross(self, which, F):
+        return self.plan.cross(which, F)
 
     gram = staticmethod(ops.gram)                      # F (r x len) -> F F^T (nmf.py:407 / :432)
 
@@ -435,12 +399,6 @@ class CudaEngine:
         return ops.norm1(F)
 
     transpose = staticmethod(ops.transpose)
-
-
-# HALS solve reads the split-K partials of the X pass itself instead of a reduced right-hand side: "u" = the U solve only
-# (measured at C2: -0.025 ms, the reduction kernel disappears), "1" = both (the V solve has 64 columns per CTA and 16+ slabs:
-# +0.05 ms), "0" = neither
-_SPLIT_RHS = os.environ.get("NNFAC_HALS_SPLIT_RHS", "u")
 
 
 class FusedNMF:
@@ -501,23 +459,22 @@ class FusedNMF:
 
     def _exchange(self, tail):
         """The peer-memory exchange region of this state (tail = r: HALS, partial Gram; tail = 1: MU, partial row sums), or None:
-        one rank, CPU stand-in engine, no peer access, or NNFAC_PEER_EXCHANGE=0 (then the NCCL collectives are used)."""
+        one rank, CPU stand-in engine, no peer access, NNFAC_PEER_EXCHANGE=0, or slices of U that are not whole 128-row tiles of
+        the fused pass (then the NCCL collectives are used)."""
         if (self.comm.world == 1 or not self._on_gpu or not hasattr(self.eng, "plan") or self.comm._boards_device is None
                 or os.environ.get("NNFAC_PEER_EXCHANGE", "1") == "0"):
             return None
         if tail not in self._px:
             chunk = self.comm.slice_of(self.m)[0]
-            # PUSH: the fused pass writes its partials straight into the owners' inboxes (needs the fused pass, i.e. rank <= 128;
-            # NNFAC_PEER_PUSH=0: every rank stages its own partial result and the owners pull)
-            push = None
-            if os.environ.get("NNFAC_PEER_PUSH", "1") != "0" and chunk % 128 == 0:
-                push = (self.eng.plan.info(0)["splits"], -(-self.r // 16) * 16)
-            key = (self.comm.group, L.device_index(self.device), self.r, self.m, chunk, tail, push)
+            if chunk % 128 != 0:
+                return None
+            splits = self.eng.plan.info(0)["splits"]
+            key = (self.comm.group, L.device_index(self.device), self.r, self.m, chunk, tail, splits)
             if key not in _EXCHANGES:
-                _EXCHANGES[key] = PeerExchange(self.comm, self.device, self.r, self.m, chunk, tail, push)
+                _EXCHANGES[key] = PeerExchange(self.comm, self.device, self.r, chunk, tail, splits)
             self._px[tail] = _EXCHANGES[key]
         px = self._px[tail]
-        if px.push is not None and self._pushing is not px:
+        if self._pushing is not px:
             px.attach_plan(self.eng.plan)          # the plan pushes into ONE region at a time (HALS: tail r, MU: tail 1)
             self._pushing = px
         return px
@@ -575,31 +532,18 @@ class FusedNMF:
                     # summed Gram) -> reduce-scatter
                     chunk, lo, hi = comm.slice_of(m)
                     px = self._exchange(r) if VMt is None else None
-                    if px is not None and px.push is not None:
-                        # PUSH: the fused pass of every rank has already written its partials of MY rows into my inbox; only the
-                        # partial Grams (r x r) are pulled.  pull_tail0 waits for every rank's post.
+                    if px is not None:
+                        # peer-memory exchange: the fused pass of every rank has already written its partials of MY rows into my
+                        # inbox; only the partial Grams (r x r) are pulled.  pull_tail waits for every rank's post.
                         if VVt_join is not None:
-                            g = VVt_join()
+                            g = VVt_join()                                         # run() aimed it at the tail block already
                             if g.data_ptr() != px.tailblk.data_ptr():
                                 px.tailblk[:, :r].copy_(g)
                         else:
                             eng.gram(V, out=px.tailblk[:, :r])
                         px.post(0)
-                        VVt = px.pull_tail0()
+                        VVt = px.pull_tail(0, 0)
                         VMt_slice = None
-                    elif px is not None:
-                        # peer-memory exchange: the split-K partials are summed straight into this rank's stage buffer, the
-                        # partial Gram lands behind them; after the post every rank pulls and sums ITS columns of all stages
-                        eng.plan.reduce(0, out=px.stage[:, :m])
-                        if VVt_join is not None:
-                            g = VVt_join()                                         # run() aimed it at the stage tail already
-                            if g.data_ptr() != px.stage[:, m:m + r].data_ptr():
-                                px.stage[:, m:m + r].copy_(g)
-                        else:
-                            eng.gram(V, out=px.stage[:, m:m + r])
-                        px.post(0)
-                        recv = px.pull_reduce(0, lo, hi - lo, m)
-                        VMt_slice, VVt = recv[:, :chunk], recv[:, chunk:]
                     elif VMt is None:
                         # the pass left its split-K partials in the plan: ONE kernel sums them straight into the send layout of the
                         # reduce-scatter and appends the partial Gram (computed under the pass, on the side stream)
@@ -620,15 +564,11 @@ class FusedNMF:
                     # slice solve straight into this rank's send buffer (the partial Gram of the new slice behind it); after the
                     # post the install kernel reads every slice from its owner's send buffer while it builds the operand planes
                     px = self._exchange(r)
-                    if px.push is not None:
-                        with comm.collective(comm.slice_lengths(m)):
-                            if hi > lo:
-                                ops.hals_solve_slabs(px.inbox, chunk, px.nslabs, px.slab_stride, px.r_pad, px.scratch(r, hi - lo), VVt,
-                                                     Ut[:, lo:hi], px.send[:, :hi - lo], r, hi - lo, 100, 0.01,
-                                                     0.0 if sparsity[0] is None else float(sparsity[0]), self.hals_stats[0])
-                    else:
-                        eng.solve_slice(VMt_slice[:, :hi - lo], VVt, Ut[:, lo:hi], px.send[:, :hi - lo], r, sparsity[0],
-                                        self.hals_stats[0], comm, comm.slice_lengths(m))
+                    with comm.collective(comm.slice_lengths(m)):
+                        if hi > lo:
+                            ops.hals_solve_slabs(px.inbox, chunk, px.nslabs, px.slab_stride, px.r_pad, px.scratch(r, hi - lo), VVt,
+                                                 Ut[:, lo:hi], px.send[:, :hi - lo], r, hi - lo, 100, 0.01,
+                                                 0.0 if sparsity[0] is None else float(sparsity[0]), self.hals_stats[0])
                     if hi > lo:
                         eng.gram(px.send[:, :hi - lo], out=px.send[:, chunk:chunk + r])
                     else:
@@ -656,8 +596,7 @@ class FusedNMF:
                 pulled = getattr(self, "_utu_pulled", None)                           # sharded: sum of the slices' Grams
                 self._utu_pulled = None
                 join = self._gram_async(1, Ut) if (self._side is not None and pulled is None) else None    # nmf.py:432, under the X pass
-                keepV = _SPLIT_RHS == "1" and hasattr(eng, "plan") and not normalize[1]   # the V solve adds the split-K partials itself
-                UtM = eng.cross(1, None, keep_partials=True) if keepV else eng.cross(1, None)   # nmf.py:433
+                UtM = eng.cross(1, None)                                              # nmf.py:433
                 UtU = pulled if pulled is not None else (join() if join is not None else eng.gram(Ut))
             with self._phase("sweep_V"):
                 if hasattr(eng, "solve_install"):
@@ -692,7 +631,7 @@ class FusedNMF:
                     if g.data_ptr() != px.tailblk.data_ptr():
                         px.tailblk[:, :r].copy_(g)
                     px.post(0)
-                    VVt = px.pull_tail0()                                          # waits for every rank's post
+                    VVt = px.pull_tail(0, 0)                                       # waits for every rank's post
                     if hi > lo:
                         num = px.inbox_sum(hi - lo)
                         den = eng.matmul(VVt, Ut[:, lo:hi])
@@ -724,19 +663,13 @@ class FusedNMF:
                 den = den_join() if den_join is not None else eng.row_sums(V)      # mu.py:85-87
                 px = self._exchange(1) if (comm.world > 1 and numU is None) else None
                 if px is not None:
-                    # peer-memory exchange: partial numerator -> stage, partial row sums of V behind it; every rank pulls and
-                    # sums its own rows of U, applies mu.py:84-88 to them, and the install kernel collects the slices
-                    # (five kernels: reduction of the split partials into the stage, post with the row sums, pull + update of
-                    # this rank's rows, post, pulled install)
+                    # peer-memory exchange: the partial numerators of my rows are already in my inbox (written by every rank's
+                    # fused pass), the partial row sums of V travel with the post; every rank applies mu.py:84-88 to its own rows
+                    # of U and the install kernel collects the slices (four kernels: post with the row sums, update of this
+                    # rank's rows, post, pulled install)
                     chunk, lo, hi = comm.slice_of(m)
-                    if px.push is not None:
-                        # PUSH: the partial numerators of my rows are already in my inbox (written by every rank's fused pass)
-                        px.post_tail(den, m)
-                        px.inbox_mu_apply(Ut, lo, hi - lo, mu.epsilon)
-                    else:
-                        eng.plan.reduce(0, out=px.stage[:, :m])
-                        px.post_tail(den, m)
-                        px.pull_mu_apply(Ut, lo, hi - lo, m, mu.epsilon)
+                    px.post_tail(den)
+                    px.inbox_mu_apply(Ut, lo, hi - lo, mu.epsilon)
                     px.post(1)
                     Ut = px.install(eng.plan, 0, m)
                 elif comm.world > 1:
@@ -764,8 +697,8 @@ class FusedNMF:
         mu2 = update_rule == "mu" and beta == 2       # Frobenius MU: cross products + squared residual, like HALS
         if mu2 and self.comm.world > 1:
             px = self._exchange(self.r) if hasattr(self.eng, "plan") else None
-            if px is None or px.push is None or 0 in fixed_modes:
-                raise NotImplementedError("column-sharded beta = 2 needs the peer-memory exchange in its push form (and a free U)")
+            if px is None or 0 in fixed_modes:
+                raise NotImplementedError("column-sharded beta = 2 needs the peer-memory exchange (and a free U)")
         mode = MODE_RES if (update_rule == "hals" or mu2) else MODE_MU
         sp = [0.0 if s is None else float(s) for s in sparsity]
         with_sparsity = update_rule == "hals" and (sp[0] != 0.0 or sp[1] != 0.0)
@@ -782,27 +715,25 @@ class FusedNMF:
             VVt_join = den_join = None
             if mode == MODE_RES and (self.comm.world == 1 or self._side is not None) and it < n_iter_max and 0 not in fixed_modes \
                     and not (self.comm.world > 1 and normalize[0]):
-                # V V^T under the first pass; sharded over peer memory: straight into the tail of this rank's stage buffer (the
-                # stage is free by now: this stream is behind the install of the previous iteration, which waited for every
-                # peer's second post, hence for every peer's pull)
+                # V V^T under the first pass; sharded over peer memory: straight into this rank's tail block (it is free by
+                # now: this stream is behind the install of the previous iteration, which waited for every peer's second post,
+                # hence for every peer's pull of the partial Grams)
                 px = self._exchange(self.r) if (self.comm.world > 1 and mode == MODE_RES and hasattr(self.eng, "plan")) else None
-                gout = None
-                if px is not None:
-                    gout = px.tailblk[:, :self.r] if px.push is not None else px.stage[:, self.m:self.m + self.r]
-                VVt_join = self._gram_async(0, self.V, out=gout)
+                VVt_join = self._gram_async(0, self.V, out=px.tailblk[:, :self.r] if px is not None else None)
             if mode == MODE_MU and self.comm.world == 1 and it < n_iter_max and 0 not in fixed_modes:
                 den_join = self._row_sums_async(0, self.V)                         # row sums of V under the first pass
             with self._phase("pass_U"):
-                # single GPU, MU: the numerator stays in the plan as split partials and is consumed by mu_finish.  (The
-                # HALS solve can add the partials itself too -- nnfac_nmf_plan_hals_solve(UtM = NULL), NNFAC_HALS_SPLIT_RHS=1.)
+                # single GPU: the numerator (MU) / cross product (HALS) stays in the plan as split partials, consumed by
+                # mu_finish / by the U solve, which adds them itself (nnfac_nmf_plan_hals_solve(UtM = NULL): 0.025 ms less at C2,
+                # no reduction kernel).  The V solve (64 columns per CTA, 16+ slabs) was 0.05 ms slower that way: cross_V reduces.
                 keep = self.comm.world == 1 and it < n_iter_max and 0 not in fixed_modes and (
-                    mode == MODE_MU or (_SPLIT_RHS in ("u", "1") and not mu2 and not normalize[0] and hasattr(self.eng, "plan")))
+                    mode == MODE_MU or (not mu2 and not normalize[0] and hasattr(self.eng, "plan")))
                 # sharded HALS: the partials stay in the plan too; the reduce-scatter's send buffer is built from them
                 keep = keep or (self.comm.world > 1 and mode == MODE_RES and it < n_iter_max and 0 not in fixed_modes
                                 and (mu2 or not normalize[0]) and hasattr(self.eng, "plan"))
                 # the cost lands directly in the scalar block that travels to the host
                 if self.comm.world > 1 and mode == MODE_MU and it < n_iter_max and 0 not in fixed_modes and self._exchange(1) is not None:
-                    # sharded MU over peer memory: the numerator partials stay in the plan and are reduced into the stage buffer
+                    # sharded MU over peer memory: the fused pass writes the numerator partials into the owners' inboxes
                     outA, _ = self.eng.fused(0, mode, True, keep_partials=True, cost_out=self._dev_scal[0:1])
                 elif self.comm.world > 1 and mode == MODE_MU and hasattr(self.eng, "plan"):
                     # sharded MU: the partial numerator lands directly in the exchange buffer (no 16.8 MB copy before the sum)

@@ -37,10 +37,8 @@ SIGNATURES = {
     "nnfac_xchg_destroy": [_P],
     "nnfac_xchg_ptr": [_P, _INT],
     "nnfac_xchg_post": [_P, _INT, _P],
-    "nnfac_xchg_wait": [_P, _INT, _P],
-    "nnfac_xchg_pull_reduce": [_P, _INT, _P, _I64, _INT, _I64, _I64, _I64, _I64, _INT, _I64, _P],
     "nnfac_xchg_post_tail": [_P, _P, _INT, _I64, _I64, _P],
-    "nnfac_xchg_pull_mu_apply": [_P, _P, _I64, _INT, _I64, _I64, _I64, _I64, _c.c_double, _I64, _P],
+    "nnfac_xchg_pull_tail": [_P, _INT, _P, _I64, _INT, _I64, _I64, _INT, _P],
     "nnfac_nmf_plan_set_factor_pulled": [_P, _INT, _P, _I64, _I64, _P, _I64, _P],
     "nnfac_hals_nnls": [_P, _INT, _P, _I64, _P, _I64, _P, _I64, _INT, _I64, _INT, _DBL, _DBL, _U32, _P, _P],
     "nnfac_hals_solve_f32": [_P, _P, _I64, _P, _I64, _P, _I64, _P, _I64, _INT, _I64, _INT, _DBL, _DBL, _P, _P],

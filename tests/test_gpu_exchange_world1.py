@@ -2,10 +2,10 @@
 
 At world size 1 an exchange region (nnfac_xchg_*) and the sweep boards (nnfac_ctx_board_*) map this process' own memory and open
 no IPC handle, so every kernel of the sharded U side -- chunked reduction, gathered / pulled install, the push layout of the fused
-pass, the pull kernels, the multi-slab HALS solve and the collective stop rule -- runs here and is compared bit for bit with its
+pass, the tail pull, the multi-slab HALS solve and the collective stop rule -- runs here and is compared bit for bit with its
 single-GPU twin (or with float64).
 
-Every call that waits (pull_*, inbox_mu_apply, set_factor_pulled) is issued after this rank's own post of that phase: a wait with
+Every call that waits (pull_tail, inbox_mu_apply, set_factor_pulled) is issued after this rank's own post of that phase: a wait with
 no matching post would spin until the kernel traps."""
 import contextlib
 import ctypes
@@ -171,11 +171,13 @@ def test_hals_solve_slabs_equals_solve_of_the_slab_sum(r, n, nslabs):
 # ---------------------------------------------------------------------------------------------
 def test_set_push_inbox_equals_plan_partials():
     """After fused(0, mode, keep_partials=True) into the inbox: inbox_mu_apply gives the bits of mu_finish, hals_solve_slabs the
-    bits of plan.hals_solve(0, None, ...), reduce_slabs_f32 the bits of plan.reduce(0); set_push(None) restores the plain pass."""
+    bits of plan.hals_solve(0, None, ...), reduce_slabs_f32 the bits of plan.reduce(0); set_push(None) restores the plain pass.
+    A zero row of X gives a zero numerator: inbox_mu_apply writes the floor there."""
     from nn_fac import _ops as ops
     L, lib = _lib()
     m, n, r = 1000, 4096, 40
     X, Ut, V = _problem(m, n, r, 11)
+    X[7] = 0.0
     push, ref = _plan_pair(X, Ut, V, r)
     splits = push.info(0)["splits"]
     assert splits > 1
@@ -202,6 +204,7 @@ def test_set_push_inbox_equals_plan_partials():
         want = ref.mu_finish(0, Ut, den, 1e-12)
         ref.set_factor(0, Ut)
         assert torch.equal(send[:, :m], want)
+        assert (send[:, 7] == np.float32(1e-12)).all()
         total = torch.empty((r, m), dtype=torch.float32, device="cuda")
         L.check(lib.nnfac_reduce_slabs_f32(L.ctx(), L.ptr(inbox), chunk, nslabs, r, r_pad, m, L.ptr(total), m, L.stream_ptr()))
         ref.fused(0, 1, want_cost=False, keep_partials=True)
@@ -234,39 +237,36 @@ def test_set_push_inbox_equals_plan_partials():
 
 
 # ---------------------------------------------------------------------------------------------
-# stage / send buffers: post_tail + pull_reduce + pull_mu_apply, set_factor_pulled
+# tail pull (post_tail / post + pull_tail), set_factor_pulled
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("lo,ncols", [(256, 333), (130, 517)])
-def test_pull_reduce_and_pull_mu_apply_of_a_column_slice(lo, ncols):
-    """The stage holds a numerator (r x m) and, posted with it, the row sums of V in column m.  pull_reduce returns exactly columns
-    [lo, lo + ncols), zeros up to the chunk and the tail; pull_mu_apply the bits of ops.mu_apply on that slice.  lo = 130: the
-    scalar path of the pull kernels (16-byte loads need lo % 4 == 0)."""
-    from nn_fac import _ops as ops
+@pytest.mark.parametrize("phase", [0, 1])
+def test_pull_tail_returns_the_posted_tail(phase):
+    """Phase 0: the row sums of V, posted by post_tail into column 0 of the tail block [r x tpad] (tail = 1).  Phase 1: an r x r
+    Gram behind the chunk of the send buffer [r x (chunk + tpad)] (col = chunk, tail = r).  Everything around the tail holds large
+    values that must not be read; pull_tail returns the posted values bit for bit and writes nothing beyond `tail` columns."""
     L, lib = _lib()
-    m, r = 1000, 24
-    chunk = 640
-    tpad = 4
-    pitch = m + tpad
-    rng = np.random.RandomState(lo)
-    num = _dev((rng.rand(r, m) + 0.01).astype(np.float32))
-    den = _dev((rng.rand(r) + 0.5).astype(np.float32))
-    F = _dev((rng.rand(r, m) + 0.05).astype(np.float32))
-    num[:, lo + 3] = 0.0                                              # a zero numerator: the floor
-    with _region(r * pitch, r * (chunk + tpad)) as h:
-        stage = _view(h, 0, (r, pitch))
-        send = _view(h, 1, (r, chunk + tpad))
-        stage[:, :m].copy_(num)
-        L.check(lib.nnfac_xchg_post_tail(h, L.ptr(den), r, pitch, m, L.stream_ptr()))
-        out = torch.full((r, chunk + 4), 5.0, dtype=torch.float32, device="cuda")
-        L.check(lib.nnfac_xchg_pull_reduce(h, 0, L.ptr(out), out.stride(0), r, pitch, lo, ncols, m, 1, chunk, L.stream_ptr()))
-        assert torch.equal(out[:, :ncols], num[:, lo:lo + ncols])
-        assert torch.equal(out[:, ncols:chunk], torch.zeros((r, chunk - ncols), device="cuda"))
-        assert torch.equal(out[:, chunk], den)
-        L.check(lib.nnfac_xchg_pull_mu_apply(h, L.ptr(F), F.stride(0), r, pitch, lo, ncols, m, 1e-12, chunk + tpad, L.stream_ptr()))
-        want = ops.mu_apply(F[:, lo:lo + ncols].contiguous(), num[:, lo:lo + ncols].contiguous(), den_vec=den, vec_per_row=True,
-                            gamma=1.0, floor=1e-12)
-        assert torch.equal(send[:, :ncols], want)
-        assert (send[:, 3] == np.float32(1e-12)).all()
+    r, chunk = 22, 640
+    tpad = -(-r // 4) * 4
+    assert tpad > r                                                   # a padding column in the phase-1 tail
+    rng = np.random.RandomState(phase)
+    with _region(r * tpad, r * (chunk + tpad)) as h:
+        if phase == 0:
+            pitch, col, tail = tpad, 0, 1
+            want = _dev((rng.rand(r, 1) + 0.5).astype(np.float32))
+            stage = _view(h, 0, (r, tpad))
+            stage.fill_(1e30)
+            L.check(lib.nnfac_xchg_post_tail(h, L.ptr(want), r, tpad, 0, L.stream_ptr()))
+        else:
+            pitch, col, tail = chunk + tpad, chunk, r
+            want = _dev(rng.rand(r, r).astype(np.float32))
+            send = _view(h, 1, (r, pitch))
+            send.fill_(1e30)
+            send[:, chunk:chunk + r].copy_(want)
+            L.check(lib.nnfac_xchg_post(h, 1, L.stream_ptr()))
+        out = torch.full((r, tail + 3), 5.0, dtype=torch.float32, device="cuda")
+        L.check(lib.nnfac_xchg_pull_tail(h, phase, L.ptr(out), out.stride(0), r, pitch, col, tail, L.stream_ptr()))
+        assert torch.equal(out[:, :tail], want)
+        assert (out[:, tail:] == 5.0).all()
 
 
 def test_set_factor_pulled_equals_set_factor():
