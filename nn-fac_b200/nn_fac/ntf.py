@@ -94,11 +94,19 @@ class DeviceNTF:
         iteration starts from, formed on chip by the fused pass that also yields the first MTTKRP of that iteration (the model
         tile never reaches HBM) -- instead of the reference's ||T||^2 - 2 <F, rhs> + ||F krao^T||^2 (ntf.py:470), which
         subtracts numbers of the size of ||T||^2 and in fp32 keeps an error of ~7e-7 ||T||^2 (the truncation of the tensor
-        core's fp32 accumulator biases rhs by -3.5e-7): 1.4e-4 of the objective at C4, more when the fit is better."""
+        core's fp32 accumulator biases rhs by -3.5e-7): 1.4e-4 of the objective at C4, more when the fit is better.
+        The pass runs on the plan of the first free mode when that is a full plan; when it is a view (mode 0 fixed), on the
+        plan of mode 0, which always is one: one extra pass over the tensor per iteration, its MTTKRP unused
+        (_residual_mode)."""
         free = [m for m in range(len(self.shape)) if m not in fixed_modes]
         return (update_rule == "hals" and self.plans is not None and self.T.dim() == 3 and self.T.dtype == torch.float32
-                and len(free) > 0 and getattr(self.plans[free[0]], "_base", None) is None      # the fused pass needs a full plan
-                and os.environ.get("NNFAC_NTF_DIRECT", "1") != "0")
+                and len(free) > 0 and os.environ.get("NNFAC_NTF_DIRECT", "1") != "0")
+
+    def _residual_mode(self, fixed_modes):
+        """The mode whose fused pass forms the direct residual (the fused pass needs a full plan, a view has no row planes):
+        the first free mode, whose MTTKRP the pass also yields, or mode 0 when that one is a view."""
+        free = [m for m in range(len(self.shape)) if m not in fixed_modes]
+        return free[0] if free and getattr(self.plans[free[0]], "_base", None) is None else 0
 
     def _residual_pass(self, mode):
         """Fused pass over unfold(T, mode): returns ((unfold(T, mode) @ krao)^T, || T - F_mode krao^T ||^2) for the CURRENT factors."""
@@ -110,8 +118,7 @@ class DeviceNTF:
 
     def cost_terms_now(self, sparsity, fixed_modes=()):
         """Device vector [direct residual of the current state, l1 norms for the sparsity terms...] (closing pass of a run)."""
-        mode = [m for m in range(3) if m not in fixed_modes][0] if len(fixed_modes) < 3 else 0
-        _, res = self._residual_pass(mode)
+        _, res = self._residual_pass(self._residual_mode(fixed_modes))
         terms = [res]
         for idx, sp in enumerate(sparsity):
             if sp:
@@ -181,9 +188,13 @@ class DeviceNTF:
         rhs = krao = cross = None
         mode = None
         direct = self.direct_cost(update_rule, fixed_modes)
-        lag_terms = None
+        lag_terms = res_mode = None
         if direct:
             lag_terms = []
+            res_mode = self._residual_mode(fixed_modes)
+            if res_mode not in modes:
+                # mode 0 is fixed and the first free mode a view: a pass over unfold(T, 0) just for the residual
+                lag_terms.append(self._residual_pass(res_mode)[1])
             for idx, sp in enumerate(sparsity):
                 if sp:
                     lag_terms.append(ops.norm1(self.factors[idx]))          # of the incoming state, like the residual
@@ -196,8 +207,8 @@ class DeviceNTF:
                 for i in others:
                     gram = self._gram(i)                                     # F_i^T F_i, ntf.py:445
                     cross = gram.clone() if cross is None else ops.hadamard_(cross, gram)
-                if direct and mode == modes[0]:
-                    # first mode: the fused pass yields the MTTKRP AND the residual of the incoming state
+                if mode == res_mode:
+                    # first free mode: the fused pass yields the MTTKRP AND the residual of the incoming state
                     rhs_t, res_in = self._residual_pass(mode)
                     lag_terms.insert(0, res_in)
                     rhs = None
