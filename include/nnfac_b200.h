@@ -349,6 +349,20 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* plan, int side, int mode, int want_cost
  * F_out is installed in the plan as nnfac_nmf_plan_set_factor would do.  One kernel. */
 int nnfac_nmf_plan_mu_finish(nnfac_nmf_plan* plan, int which, const float* F_in, int64_t ld_in, const float* den,
                              double floor_value, float* F_out, int64_t ld_out, void* stream);
+/* General-beta MU pass (beta >= 0 other than 1 and 2; mu.py:84-97) over side 0 or 1 with the installed factors, K = U V formed
+ * and consumed on chip.  The split partials of the numerator (K^(beta-2) * X) V^T (side 0; its twin for V on side 1) stay in the
+ * plan; those of the denominator K^(beta-1) V^T go to den_partial, a caller-owned device buffer of at least
+ * nnfac_nmf_plan_fused_beta_bytes bytes.  cost_out (device double, may be NULL): the beta-divergence of X from U V when
+ * want_cost != 0.  NNFAC_ERR_UNSUPPORTED for rank > 64, 3-plane plans, view plans, plans with the push exchange set, and
+ * beta = 1 or 2 (nnfac_nmf_plan_fused). */
+int nnfac_nmf_plan_fused_beta_bytes(const nnfac_nmf_plan* plan, size_t* bytes);
+int nnfac_nmf_plan_fused_beta(nnfac_nmf_plan* plan, int side, double beta, int want_cost, float* den_partial, double* cost_out,
+                              void* stream);
+/* General-beta update of factor `which` from the two partial sets of the last nnfac_nmf_plan_fused_beta pass over side `which`
+ * (both summed in the order of nnfac_nmf_plan_reduce): F_out = max(F_in * (num / den)^gamma, floor_value), gamma = the
+ * exponent of beta_divergence.py:75-80; F_out is installed in the plan as nnfac_nmf_plan_set_factor would do.  One kernel. */
+int nnfac_nmf_plan_mu_finish_beta(nnfac_nmf_plan* plan, int which, const float* F_in, int64_t ld_in, const float* den_partial,
+                                  double gamma, double floor_value, float* F_out, int64_t ld_out, void* stream);
 /* Work decomposition chosen for one side (for benchmarks / DESIGN.md); any pointer may be NULL. */
 int nnfac_nmf_plan_info(const nnfac_nmf_plan* plan, int which, int* splits, int* stages_per_unit,
                         int* num_units, int* num_stages, int* grid);

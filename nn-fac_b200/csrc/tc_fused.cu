@@ -13,6 +13,14 @@
 // from (the reference re-forms U V in a third pass for that).  All products are bf16 hi/lo splits
 // (3 MMAs each) with fp32 accumulation in TMEM; D2 chains are cut every `drain` stages and summed in
 // registers because the tensor core accumulates with truncation.
+//
+// General beta (MODE_BETA0 / _BETAI / _BETAG: beta = 0, integer beta >= 3, any other beta; 2 planes, rank <= 64), mu.py:84-97:
+//   transform   Q_num = x k^(beta-2), Q_den = k^(beta-1) (both 0 where k = 0: padding), cost += k^beta h_beta(x / k)
+//   GEMM-2      two chains per stage against the same factor slab: D2_num += Q_num Fn^T, D2_den += Q_den Fn^T
+// Tensor memory: D1 2 x 64 | D2_num 2 x 64 | D2_den 2 x 64 | Q_num 64 | Q_den 64 = 512 columns.  A1 is not copied to tensor
+// memory: the model GEMM reads it from its shared-memory staging buffer (SS form), so the next unit's A1 is only loaded once
+// the unit's last model GEMM has retired.  The ratio tiles are single-buffered: the transform of stage i + 1 writes them
+// after the contraction of stage i has retired.
 #include "tc_plan.cuh"
 
 #include <string.h>
@@ -27,7 +35,7 @@ constexpr int NWT = 4 * NSP;         // transform warps: 4 TMEM lane quadrants x
 constexpr int FUSED_THREADS = 128 + 32 * NWT;   // warp0 TMA, warps 1/3 MMA issuers, warp2 TMEM, then transform warps
 static_assert(CW == 16, "the transform below moves 16 columns per tcgen05.ld / 8 words per tcgen05.st");
 constexpr uint32_t X_BYTES = TILE_ROWS * BK * sizeof(bf16);   // 16 KiB per plane tile
-constexpr int MODE_RES = 0, MODE_MU = 1;
+constexpr int MODE_RES = 0, MODE_MU = 1, MODE_BETA0 = 2, MODE_BETAI = 3, MODE_BETAG = 4;
 #ifndef FUSED_PREFETCH
 #define FUSED_PREFETCH 0             // 1: fetch the model tile of stage i + 1 from tensor memory while stage i is transformed (measured: 9-13 % slower)
 #endif
@@ -75,6 +83,17 @@ struct FusedParams {
   int push_src;
 };
 
+// Constants of a general-beta pass (MODE_BETA*), a kernel argument of its own behind the others.  hc[i] = c_(i+2), the
+// coefficients of h_beta(1 + d) = sum_n c_n d^n (n >= 2): c_2 = 1/2, c_(n+1) = c_n (beta - n) / (n + 1).
+constexpr int NHC = 11;            // d^2 .. d^12: truncation < 4e-8 relative for |d| < 1/4 and 0 <= beta <= 5
+struct BetaParams {
+  float* den;                      // [splits][r_pad][ld_partial]: split partials of the denominator contraction
+  float beta, bm2;                 // beta, beta - 2
+  int ibm2, ibeta;                 // MODE_BETAI: beta - 2 and beta as integers
+  float inv_bb1, inv_beta;         // 1 / (beta (beta - 1)), 1 / beta
+  float hc[NHC];
+};
+
 __device__ __forceinline__ float rcp_approx(float x) {   // MUFU.RCP, <= 1 ulp: no IEEE fix-up branch
   float y;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -99,6 +118,40 @@ __device__ __forceinline__ float kl_g(float q) {
   }
   return fmaf(q, lg2_approx(q + 1e-30f) * 0.6931471805599453f, -d);
 }
+__device__ __forceinline__ float ex2_approx(float x) {    // MUFU.EX2
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+__device__ __forceinline__ float ipow(float b, int n) {   // b^n, n >= 0: products only
+  float r = 1.f;
+  for (; n; n >>= 1, b *= b)
+    if (n & 1) r *= b;
+  return r;
+}
+// k^beta h_beta(x / k), h_beta(q) = (q^beta - beta q + beta - 1) / (beta (beta - 1)) >= 0 (beta = 0: q - 1 - ln q), so that the
+// beta-divergence is a sum of non-negative terms (no cancellation against the sums of x^beta and k^beta); near q = 1 the series
+// of h_beta in d = q - 1.  kb = k^beta, ik = 1 / k.  Padding (k = 0) contributes 0; x = 0 contributes what
+// beta_divergence.py:49-52 gives there: k^beta / beta, and -1 at beta = 0 (its masked logarithm).
+template <int MODE>
+__device__ __forceinline__ float beta_cost(float x, float k, float kb, float ik, const BetaParams& bp) {
+  if (!(k > 0.f)) return 0.f;
+  if (x == 0.f) return MODE == MODE_BETA0 ? -1.f : kb * bp.inv_beta;
+  const float q = x * ik, d = q - 1.f;
+  float h;
+  if (fabsf(d) < 0.25f) {
+    float c = bp.hc[NHC - 1];
+#pragma unroll
+    for (int i = NHC - 2; i >= 0; --i) c = fmaf(d, c, bp.hc[i]);
+    h = d * d * c;
+  } else if (MODE == MODE_BETA0) {
+    h = fmaf(lg2_approx(q), -0.6931471805599453f, d);
+  } else {
+    const float qb = MODE == MODE_BETAI ? ipow(q, bp.ibeta) : ex2_approx(bp.beta * lg2_approx(q));
+    h = (fmaf(-bp.beta, q, qb) + (bp.beta - 1.f)) * bp.inv_bb1;
+  }
+  return kb * h;
+}
 __device__ __forceinline__ float bf_lo(uint32_t w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
 
@@ -109,11 +162,14 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
                 const __grid_constant__ CUtensorMap map_fkh, const __grid_constant__ CUtensorMap map_fkl,
                 const __grid_constant__ CUtensorMap map_a1h, const __grid_constant__ CUtensorMap map_a1l,
                 const FusedParams p, const __grid_constant__ CUtensorMap map_xm, const __grid_constant__ CUtensorMap map_fkm,
-                const __grid_constant__ CUtensorMap map_a1m) {
+                const __grid_constant__ CUtensorMap map_a1m, const BetaParams bp) {
   using C = Cfg<RK, PLANES, PLANES == 3 && XF32>;
+  constexpr bool BETA = MODE >= MODE_BETA0;
+  static_assert(!BETA || (RK == 64 && PLANES == 2), "general beta: 2 planes, rank <= 64");
   static_assert(RK == 64 || (MODE == MODE_RES && !XF32), "rank 65..128: residual + cross-product pass only");
   static_assert(PLANES == 2 || (RK == 64 && (MODE == MODE_RES) != XF32), "3 planes: rank <= 64; beta = 1 reads X from its fp32 copy");
-  constexpr int FSTAGES = C::FSTAGES, ND1 = C::ND1, CWD = C::CWD;
+  constexpr int FSTAGES = C::FSTAGES, ND1 = BETA ? 2 : C::ND1, CWD = C::CWD;
+  constexpr int NQ = BETA ? 1 : 2;     // ratio-tile buffers in tensor memory
   // 3 planes: one stage per contraction chain (24 MMAs, as many as two stages of the 2-plane products), drained two stages late
   constexpr int DRAIN_P = PLANES == 3 ? 1 : DRAIN;
   constexpr uint32_t FK_BYTES = C::FK_BYTES, STAGE_BYTES = C::STAGE_BYTES, A1_BYTES = C::A1_BYTES, XB = C::XB;
@@ -146,7 +202,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < FSTAGES; ++s) { tc::mbar_init(&full[s], 1); tc::mbar_init(&empty[s], NWT + 1); }
-    tc::mbar_init(a1_full, 1); tc::mbar_init(a1_empty, NWT);
+    tc::mbar_init(a1_full, 1); tc::mbar_init(a1_empty, BETA ? 1 : NWT);   // BETA: released by the unit's last model GEMM
     tc::mbar_init(a1t_ready, NWT); tc::mbar_init(a1t_free, 1);
     for (int b = 0; b < 2; ++b) { tc::mbar_init(&q_ready[b], NWT); tc::mbar_init(&q_free[b], 1); }
     for (int b = 0; b < ND1; ++b) { tc::mbar_init(&d1_full[b], 1); tc::mbar_init(&d1_empty[b], NWT); }
@@ -159,7 +215,9 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
   tc::tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   // tensor-memory map (columns): D1 ND1 x 64 | D2 2 x RK | A1 hi RK/2 + lo RK/2 (+ mid RK/2) | Q 2 x (hi 32 + lo 32) (MU)  (512 in all)
-  const uint32_t D1 = tmem_base, D2 = tmem_base + 64 * ND1, A1T = D2 + 2 * RK, QT = A1T + PLANES * (RK / 2);
+  // BETA: D1 2 x 64 | D2 (numerator) 2 x 64 | D2D (denominator) 2 x 64 | Q_num (hi 32 + lo 32) | Q_den (hi 32 + lo 32)
+  const uint32_t D1 = tmem_base, D2 = tmem_base + 64 * ND1, A1T = D2 + 2 * RK, QT = BETA ? A1T + 2 * RK : A1T + PLANES * (RK / 2);
+  const uint32_t D2D = A1T;
   const int S = p.stages_per_unit;
 
   if (warp == 0 && lane == 0) {
@@ -203,7 +261,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
     int b1 = 0; uint32_t b1_phase = 0;
     uint32_t a1_phase = 0;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
-      tc::mbar_wait(a1t_ready, a1_phase);
+      tc::mbar_wait(BETA ? a1_full : a1t_ready, a1_phase);
       a1_phase ^= 1;
       for (int i = 0; i < S; ++i) {
         tc::mbar_wait(&full[st1], ph1);
@@ -231,6 +289,18 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #pragma unroll
             for (int k = 0; k < RK / UMMA_K; ++k)
               if (k < ksteps) tc::umma_bf16_ts(d, ah + 8 * k, fkh + (uint64_t)((k & 3) * 2), idesc1, true);
+          } else if constexpr (BETA) {
+            // A1 from its shared-memory staging buffer (K-major, like an X tile)
+            const uint64_t ah = tc::umma_desc_k_sw128(tc::smem_u32(a1)), al = tc::umma_desc_k_sw128(tc::smem_u32(a1 + X_BYTES));
+#pragma unroll
+            for (int k = 0; k < RK / UMMA_K; ++k) {
+              if (k < ksteps) {
+                const uint64_t ko = (uint64_t)(k * 2), bo = (uint64_t)((k & 3) * 2);
+                tc::umma_bf16(d, ah + ko, fkh + bo, idesc1, k != 0);
+                tc::umma_bf16(d, al + ko, fkh + bo, idesc1, true);
+                tc::umma_bf16(d, ah + ko, fkl + bo, idesc1, true);
+              }
+            }
           } else {
 #pragma unroll
           for (int k = 0; k < RK / UMMA_K; ++k) {
@@ -243,7 +313,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           }
           }
           tc::umma_commit(&d1_full[b1]);
-          if (i == S - 1) tc::umma_commit(a1t_free);
+          if (i == S - 1) tc::umma_commit(BETA ? a1_empty : a1t_free);
         }
         __syncwarp();
         if (++b1 == ND1) { b1 = 0; b1_phase ^= 1; }
@@ -261,7 +331,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         const bool chain_start = (j % DRAIN_P) == 0;
         const bool chain_end = ((j + 1) % DRAIN_P) == 0 || j == S - 1;
         tc::mbar_wait(&full[st2], ph2);
-        if (MODE == MODE_MU) tc::mbar_wait(&q_ready[qb], qb_phase);
+        if (MODE == MODE_MU || BETA) tc::mbar_wait(&q_ready[qb], qb_phase);
         if (chain_start) tc::mbar_wait(&d2_empty[b2], b2_phase ^ 1);
         tc::tcgen05_fence_after();
         if (tc::elect_one()) {
@@ -299,6 +369,21 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
               if (MODE == MODE_MU) tc::umma_bf16_ts(d, QT + (uint32_t)qb * 64 + 8 * k, fnh + (uint64_t)(k * 128), idesc2, true);
               else tc::umma_bf16(d, xh + (uint64_t)(k * 2), fnh + (uint64_t)(k * 128), idesc2, true);
             }
+          } else if constexpr (BETA) {
+            // two chains against the same slab: numerator into D2, denominator into D2D
+            const uint32_t dd = D2D + (uint32_t)b2 * RK;
+#pragma unroll
+            for (int k = 0; k < BK / UMMA_K; ++k) {
+              const uint64_t kb = (uint64_t)(k * 128);
+              const uint32_t qa = QT + 8 * k, qd = qa + 64;
+              const bool acc0 = !(chain_start && k == 0);
+              tc::umma_bf16_ts(d, qa, fnh + kb, idesc2, acc0);
+              tc::umma_bf16_ts(d, qa + 32, fnh + kb, idesc2, true);
+              tc::umma_bf16_ts(d, qa, fnl + kb, idesc2, true);
+              tc::umma_bf16_ts(dd, qd, fnh + kb, idesc2, acc0);
+              tc::umma_bf16_ts(dd, qd + 32, fnh + kb, idesc2, true);
+              tc::umma_bf16_ts(dd, qd, fnl + kb, idesc2, true);
+            }
           } else {
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
@@ -317,11 +402,11 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           }
           }
           tc::umma_commit(&empty[st2]);
-          if (MODE == MODE_MU) tc::umma_commit(&q_free[qb]);
+          if (MODE == MODE_MU || BETA) tc::umma_commit(&q_free[qb]);
           if (chain_end) tc::umma_commit(&d2_full[b2]);
         }
         __syncwarp();
-        if (MODE == MODE_MU) { if (++qb == 2) { qb = 0; qb_phase ^= 1; } }
+        if (MODE == MODE_MU || BETA) { if (++qb == NQ) { qb = 0; qb_phase ^= 1; } }
         if (chain_end) { if (++b2 == 2) { b2 = 0; b2_phase ^= 1; } }
         if (++st2 == FSTAGES) { st2 = 0; ph2 ^= 1; }
       }
@@ -339,10 +424,13 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
     double cost = 0.0, costk = 0.0;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
       const int tile = p.split_major ? u % p.tiles : u / p.splits, split = p.split_major ? u / p.tiles : u % p.splits;
-      float sum[CWD];
+      float sum[CWD], sumd[BETA ? CWD : 1];     // sumd: denominator (BETA)
 #pragma unroll
       for (int j = 0; j < CWD; ++j) sum[j] = 0.f;
-      if (RK == 64) {
+      if (BETA) {
+#pragma unroll
+        for (int j = 0; j < CWD; ++j) sumd[BETA ? j : 0] = 0.f;
+      } else if (RK == 64) {
         // A1 (this unit's rows of the aligned factor): shared memory -> tensor memory, this thread's row and K part
         tc::mbar_wait(a1_full, a1_phase);
         tc::mbar_wait(a1t_free, a1_phase ^ 1);
@@ -398,6 +486,12 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
             tc::tmem_ld_wait();
 #pragma unroll
             for (int j = 0; j < 16; ++j) sum[c0 + j] += __uint_as_float(v[j]);
+            if (BETA) {
+              tc::tmem_ld16(D2D + (uint32_t)b2 * RK + lane_base + CWD * part + c0, v);
+              tc::tmem_ld_wait();
+#pragma unroll
+              for (int j = 0; j < 16; ++j) sumd[BETA ? c0 + j : 0] += __uint_as_float(v[j]);
+            }
           }
         }
         tc::tcgen05_fence_before();
@@ -449,6 +543,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         // is on its way to the contraction GEMM; only then are the MUFU.LG2 terms computed (nothing waits for them)
         constexpr bool DEFER = FUSED_DEFER_COST && FUSED_PACKED && MODE == MODE_MU && COST;
         float2 xs[DEFER ? 4 * NCHK : 1], qs[DEFER ? 4 * NCHK : 1];
+        uint32_t dhw[BETA ? 4 * NCHK : 1], dlw[BETA ? 4 * NCHK : 1];   // BETA: denominator operand (qhw / qlw: numerator)
 #pragma unroll
         for (int cc = 0; cc < NCHK; ++cc) {
           float2 xv[4];
@@ -487,6 +582,38 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #endif
             }
           }
+          if constexpr (BETA) {
+#pragma unroll
+            for (int w = 0; w < 4; ++w) {
+              float an[2], ad[2];
+#pragma unroll
+              for (int h = 0; h < 2; ++h) {
+                const float x = h ? xv[w].y : xv[w].x, k = __uint_as_float(kk[cc * 8 + 2 * w + h]);
+                float ik = 0.f, pk, kb = 1.f;                                  // pk = k^(beta - 2), kb = k^beta
+                if (MODE == MODE_BETA0) {
+                  ik = rcp_approx(k);
+                  pk = ik * ik;
+                  ad[h] = ik;
+                } else {
+                  pk = MODE == MODE_BETAI ? ipow(k, bp.ibm2) : ex2_approx(bp.bm2 * lg2_approx(k));
+                  ad[h] = pk * k;
+                  if (COST) { ik = rcp_approx(k); kb = ad[h] * k; }
+                }
+                an[h] = x * pk;
+                if (!(k > 0.f)) { an[h] = 0.f; ad[h] = 0.f; }                   // padding: never 0 * inf
+                if (COST) acc2.x += beta_cost<MODE>(x, k, kb, ik, bp);
+              }
+              // hi / lo bf16 pairs: lo = bf16(v - hi), exact remainder
+              const __nv_bfloat162 hn = __floats2bfloat162_rn(an[0], an[1]), hd = __floats2bfloat162_rn(ad[0], ad[1]);
+              const uint32_t hnw = *reinterpret_cast<const uint32_t*>(&hn), hdw = *reinterpret_cast<const uint32_t*>(&hd);
+              const __nv_bfloat162 ln = __floats2bfloat162_rn(an[0] - bf_lo(hnw), an[1] - bf_hi(hnw));
+              const __nv_bfloat162 ld = __floats2bfloat162_rn(ad[0] - bf_lo(hdw), ad[1] - bf_hi(hdw));
+              qhw[4 * cc + w] = hnw;
+              qlw[4 * cc + w] = *reinterpret_cast<const uint32_t*>(&ln);
+              dhw[BETA ? 4 * cc + w : 0] = hdw;
+              dlw[BETA ? 4 * cc + w : 0] = *reinterpret_cast<const uint32_t*>(&ld);
+            }
+          } else {
 #if FUSED_PACKED
 #pragma unroll
           for (int w = 0; w < 4; ++w) {
@@ -544,6 +671,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
             }
           }
 #endif
+          }
         }
         auto flush_cost = [&]() {
           if (COST && ((i & 7) == 7 || i == S - 1)) {
@@ -567,7 +695,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           tc::tcgen05_fence_before();
           __syncwarp();
           if (lane == 0) tc::mbar_arrive(&q_ready[qb]);
-          if (++qb == 2) { qb = 0; qb_phase ^= 1; }
+          if (++qb == NQ) { qb = 0; qb_phase ^= 1; }
           if (DEFER) {
 #pragma unroll
             for (int e = 0; e < 4 * NCHK; ++e) {
@@ -581,6 +709,21 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
             }
             flush_cost();
           }
+        }
+        if constexpr (BETA) {
+          // numerator and denominator operands -> tensor memory (single buffer: the contraction of the previous stage has retired)
+          tc::mbar_wait(&q_free[0], qb_phase ^ 1);
+          tc::tcgen05_fence_after();
+          const uint32_t qa = QT + lane_base + (CW / 2) * part;
+          tc::tmem_st8(qa, qhw);
+          tc::tmem_st8(qa + 32, qlw);
+          tc::tmem_st8(qa + 64, dhw);
+          tc::tmem_st8(qa + 96, dlw);
+          tc::tmem_st_wait();
+          tc::tcgen05_fence_before();
+          __syncwarp();
+          if (lane == 0) tc::mbar_arrive(&q_ready[0]);
+          qb_phase ^= 1;
         }
         // drain with a lag of one more stage: chain (i-3)/2 ended with stage i-2, its GEMMs have retired by now, and
         // its TMEM buffer is only needed again by the chain that starts with stage i+1
@@ -599,6 +742,12 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #pragma unroll
         for (int j = 0; j < CWD; ++j)
           if (CWD * part + j < p.r_pad) out[(int64_t)j * p.ld_partial] = sum[j];
+        if (BETA) {     // the denominator partials, same layout
+          float* outd = bp.den + ((int64_t)split * p.r_pad + CWD * part) * p.ld_partial + (int64_t)tile * TILE_ROWS + row;
+#pragma unroll
+          for (int j = 0; j < CWD; ++j)
+            if (CWD * part + j < p.r_pad) outd[(int64_t)j * p.ld_partial] = sumd[BETA ? j : 0];
+        }
       }
     }
     // per-CTA cost partials (fixed order): [blockIdx] = sum of squares or sum of x log2(x/k); [512 + blockIdx] = sum of k
@@ -622,6 +771,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 
 // One pass that finishes a factor update and installs the factor in the plan:
 //   APPLY: F = max(F_in * (sum of the split partials of the last fused pass) / den[k], floor)      (mu.py:84-88)
+//          DENP (general beta): F = max(F_in * (num / den)^gamma, floor), den = the sum of the denominator partials
+//          `den` of the same pass ([splits][r_pad][ldp], summed in the order of the numerator)          (mu.py:84-97)
 //   else : F = F_in                                                                                 (after a HALS solve)
 // and writes F (fp32, rank-major), its K-major bf16 hi/lo planes [r_pad x ld_plane] (operand of the cross product)
 // and its rank-contiguous planes [R x 64] (operands of the fused pass).  Block = 32 columns x all ranks.
@@ -633,14 +784,15 @@ struct PeerG {                      // PULL: slice s of the factor lives in p[s]
 };
 
 // PLANES = 3: the middle planes go to fm / rowm.
-template <bool APPLY, int RK, bool PULL, int PLANES = 2>
+template <bool APPLY, int RK, bool PULL, int PLANES = 2, bool DENP = false>
 __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restrict__ partial, int splits, int r, int r_pad, int64_t R,
                                                             int64_t ldp, const float* __restrict__ F_in, int64_t ld_in,
                                                             int64_t in_chunk, int64_t in_slab, const PeerG G,
                                                             const float* __restrict__ den, float floor_value, float* __restrict__ F_out,
                                                             int64_t ld_out, bf16* __restrict__ fh, bf16* __restrict__ fl, int64_t ld_plane,
                                                             bf16* __restrict__ rowh, bf16* __restrict__ rowl,
-                                                            bf16* __restrict__ fm = nullptr, bf16* __restrict__ rowm = nullptr) {
+                                                            bf16* __restrict__ fm = nullptr, bf16* __restrict__ rowm = nullptr,
+                                                            float gamma = 1.f) {
   __shared__ float tile[RK][33];
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   if (PULL && G.flags != nullptr) {
@@ -673,17 +825,29 @@ __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restr
     if (k < r && c < R) {
       f = PULL ? pulled[PULL ? (k - ty) / 8 : 0] : F_in[(int64_t)k * ld_in + cin];
       if (APPLY) {
-        float num = 0.f;                            // fixed order; loads issued eight at a time (few blocks, many splits
-        int sp = 0;                                 // when the other dimension is short: NTD has 64 splits for 256 rows)
-        for (; sp + 8 <= splits; sp += 8) {
-          float t[8];
+        auto sum_splits = [&](const float* __restrict__ part) {
+          float s = 0.f;                            // fixed order; loads issued eight at a time (few blocks, many splits
+          int sp = 0;                               // when the other dimension is short: NTD has 64 splits for 256 rows)
+          for (; sp + 8 <= splits; sp += 8) {
+            float t[8];
 #pragma unroll
-          for (int u = 0; u < 8; ++u) t[u] = partial[((int64_t)(sp + u) * r_pad + k) * ldp + c];
+            for (int u = 0; u < 8; ++u) t[u] = part[((int64_t)(sp + u) * r_pad + k) * ldp + c];
 #pragma unroll
-          for (int u = 0; u < 8; ++u) num += t[u];
+            for (int u = 0; u < 8; ++u) s += t[u];
+          }
+          for (; sp < splits; ++sp) s += part[((int64_t)sp * r_pad + k) * ldp + c];
+          return s;
+        };
+        const float num = sum_splits(partial);
+        float v;
+        if constexpr (DENP) {
+          float ratio = num / sum_splits(den);
+          if (gamma == 0.5f) ratio = sqrtf(ratio);  // beta = 0 (gamma_beta, beta_divergence.py:75-80)
+          else if (gamma != 1.f) ratio = powf(ratio, gamma);
+          v = f * ratio;
+        } else {
+          v = f * (num / den[k]);
         }
-        for (; sp < splits; ++sp) num += partial[((int64_t)sp * r_pad + k) * ldp + c];
-        const float v = f * (num / den[k]);
         f = v > floor_value ? v : floor_value;      // np.maximum(., epsilon); NaN propagates like numpy
         if (v != v) f = v;
       }
@@ -801,6 +965,19 @@ static int finish_factor(nnfac_nmf_plan* p, int which, bool apply, const float* 
 #undef NNFAC_FINISH
   NNFAC_LAUNCH_CHECK(p->ctx);
   return NNFAC_OK;
+}
+
+static FusedParams fused_params(const nnfac_nmf_plan* p, int side, bool want_cost) {
+  const Side* s = &p->side[side];
+  FusedParams fp;
+  fp.r_pad = p->r_pad; fp.splits = s->cp.splits; fp.stages_per_unit = s->cp.stages_per_unit; fp.num_units = s->cp.num_units;
+  fp.drain = DRAIN; fp.want_cost = want_cost ? 1 : 0;
+  fp.tiles = s->cp.tiles; fp.split_major = s->cp.split_major;
+  fp.ld_partial = s->cp.ld_partial; fp.partial = p->partial; fp.cost_part = p->cost_part;
+  fp.a1h = p->rowp_h[side]; fp.a1l = p->rowp_l[side]; fp.R = s->R;
+  fp.push_chunk = 0; fp.push_src = 0;
+  for (int q = 0; q < NNFAC_MAX_PEERS; ++q) fp.push[q] = nullptr;
+  return fp;
 }
 
 extern "C" {
@@ -1004,14 +1181,9 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
   Side* s = &p->side[side];
   NNFAC_ARG(!out || ld_out >= s->R, "nnfac_nmf_plan_fused: leading dimension too small");
   cudaStream_t st = (cudaStream_t)stream;
-  FusedParams fp;
-  fp.r_pad = p->r_pad; fp.splits = s->cp.splits; fp.stages_per_unit = s->cp.stages_per_unit; fp.num_units = s->cp.num_units;
-  fp.drain = DRAIN; fp.want_cost = (mode == 0 || want_cost) ? 1 : 0;
-  fp.tiles = s->cp.tiles; fp.split_major = s->cp.split_major;
-  fp.ld_partial = s->cp.ld_partial; fp.partial = p->partial; fp.cost_part = p->cost_part;
-  fp.a1h = p->rowp_h[side]; fp.a1l = p->rowp_l[side]; fp.R = s->R;
-  fp.push_chunk = 0; fp.push_src = 0;
-  for (int q = 0; q < NNFAC_MAX_PEERS; ++q) fp.push[q] = nullptr;
+  FusedParams fp = fused_params(p, side, mode == 0 || want_cost);
+  BetaParams bp;
+  memset(&bp, 0, sizeof(bp));
   if (side == 0 && !out && p->push_chunk > 0) {       // sharded U side: partials go straight to their owners' inboxes
     fp.push_chunk = p->push_chunk; fp.push_src = p->push_src;
     for (int q = 0; q < p->push_world; ++q) fp.push[q] = p->push[q];
@@ -1023,7 +1195,7 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
     NNFAC_CUDA(cudaFuncSetAttribute(tc_fused_kernel<M, C, XF, RKV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     tc_fused_kernel<M, C, XF, RKV><<<s->grid, FUSED_THREADS, smem, st>>>(MAPH, MAPL, p->map_row_b_h[other],                  \
         p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp, MAPH, p->map_row_b_h[other],                  \
-        p->map_row_a_h[side]);                                                                                                \
+        p->map_row_a_h[side], bp);                                                                                            \
   } while (0)
 #define NNFAC_LAUNCH_FUSED3(M, C, XF, MAPH, MAPL)                                                                                \
   do {                                                                                                                        \
@@ -1031,7 +1203,7 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
     NNFAC_CUDA(cudaFuncSetAttribute(tc_fused_kernel<M, C, XF, 64, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     tc_fused_kernel<M, C, XF, 64, 3><<<s->grid, FUSED_THREADS, smem, st>>>(MAPH, MAPL, p->map_row_b_h[other],                \
         p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp, s->map_xm, p->map_row_b_m[other],             \
-        p->map_row_a_m[side]);                                                                                                \
+        p->map_row_a_m[side], bp);                                                                                            \
   } while (0)
   if (p->planes == 3) {
     if (mode == 0) NNFAC_LAUNCH_FUSED3(MODE_RES, true, false, s->map_xh, s->map_xl);
@@ -1060,6 +1232,86 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
       kl_cost_finish_kernel<<<1, 32, 0, st>>>(p->cost_part, s->grid, p->sums, cost_out);
     NNFAC_LAUNCH_CHECK(p->ctx);
   }
+  return NNFAC_OK;
+}
+
+// Bytes of the caller-owned buffer that receives the denominator partials of nnfac_nmf_plan_fused_beta (either side).
+int nnfac_nmf_plan_fused_beta_bytes(const nnfac_nmf_plan* p, size_t* bytes) {
+  NNFAC_ARG(p && bytes, "nnfac_nmf_plan_fused_beta_bytes: NULL argument");
+  *bytes = p->partial_bytes;
+  return NNFAC_OK;
+}
+
+// General-beta pass (beta >= 0 other than 1 and 2) over side `side`: numerator partials of (K^(beta-2) * X) Fn^T into the
+// plan's partial buffer, denominator partials of K^(beta-1) Fn^T into den_partial, cost_out = beta-divergence(X | U V).
+int nnfac_nmf_plan_fused_beta(nnfac_nmf_plan* p, int side, double beta, int want_cost, float* den_partial, double* cost_out,
+                              void* stream) {
+  NNFAC_ARG(p && den_partial && (side == 0 || side == 1), "nnfac_nmf_plan_fused_beta: bad argument");
+  NNFAC_ARG(beta >= 0.0, "nnfac_nmf_plan_fused_beta: beta must be >= 0 (got %g)", beta);
+  NNFAC_ARG((p->sides >> side) & 1, "nnfac_nmf_plan_fused_beta: this plan keeps no planes of side %d", side);
+  if (beta == 1.0 || beta == 2.0) { nnfac_set_error("nnfac_nmf_plan_fused_beta: beta = %g is the mode-1 / cross-product pass", beta); return NNFAC_ERR_UNSUPPORTED; }
+  if (p->base) { nnfac_set_error("nnfac_nmf_plan_fused_beta: not available on a view plan"); return NNFAC_ERR_UNSUPPORTED; }
+  if (!p->fused_ok || p->rk != 64) { nnfac_set_error("nnfac_nmf_plan_fused_beta: covers rank <= 64 (rank %d)", p->r); return NNFAC_ERR_UNSUPPORTED; }
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_fused_beta: covers 2-plane plans (the plan has %d)", p->planes); return NNFAC_ERR_UNSUPPORTED; }
+  if (p->push_chunk > 0) { nnfac_set_error("nnfac_nmf_plan_fused_beta: not available with the push exchange (nnfac_nmf_plan_set_push)"); return NNFAC_ERR_UNSUPPORTED; }
+  Side* s = &p->side[side];
+  cudaStream_t st = (cudaStream_t)stream;
+  const FusedParams fp = fused_params(p, side, want_cost != 0);
+  BetaParams bp;
+  memset(&bp, 0, sizeof(bp));
+  bp.den = den_partial;
+  bp.beta = (float)beta; bp.bm2 = (float)(beta - 2.0);
+  bp.ibm2 = (int)beta - 2; bp.ibeta = (int)beta;
+  bp.inv_bb1 = (float)(1.0 / (beta * (beta - 1.0))); bp.inv_beta = beta > 0.0 ? (float)(1.0 / beta) : 0.f;
+  double c = 0.5;
+  for (int i = 0; i < NHC; ++i) { bp.hc[i] = (float)c; c *= (beta - (i + 2)) / (i + 3); }
+  const bool integral = beta >= 3.0 && beta == (double)(int)beta;
+  const int other = 1 - side;
+#define NNFAC_LAUNCH_BETA(M, C, XF, MAPH, MAPL)                                                                                \
+  do {                                                                                                                        \
+    const size_t smem = Cfg<64>::SMEM;                                                                                        \
+    NNFAC_CUDA(cudaFuncSetAttribute(tc_fused_kernel<M, C, XF, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  \
+    tc_fused_kernel<M, C, XF, 64><<<s->grid, FUSED_THREADS, smem, st>>>(MAPH, MAPL, p->map_row_b_h[other],                    \
+        p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp, MAPH, p->map_row_b_h[other],                  \
+        p->map_row_a_h[side], bp);                                                                                            \
+  } while (0)
+#define NNFAC_LAUNCH_BETA_X(M, C)                                                                                              \
+  do {                                                                                                                        \
+    if (p->xf_ready) NNFAC_LAUNCH_BETA(M, C, true, p->map_xf[side], p->map_xf[side]);                                         \
+    else NNFAC_LAUNCH_BETA(M, C, false, s->map_xh, s->map_xl);                                                                \
+  } while (0)
+  if (beta == 0.0) { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETA0, true); else NNFAC_LAUNCH_BETA_X(MODE_BETA0, false); }
+  else if (integral) { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETAI, true); else NNFAC_LAUNCH_BETA_X(MODE_BETAI, false); }
+  else { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETAG, true); else NNFAC_LAUNCH_BETA_X(MODE_BETAG, false); }
+#undef NNFAC_LAUNCH_BETA_X
+#undef NNFAC_LAUNCH_BETA
+  NNFAC_LAUNCH_CHECK(p->ctx);
+  if (cost_out && fp.want_cost) {
+    sum_cost_parts_kernel<<<1, 32, 0, st>>>(p->cost_part, s->grid, cost_out);
+    NNFAC_LAUNCH_CHECK(p->ctx);
+  }
+  return NNFAC_OK;
+}
+
+// General-beta multiplicative update of factor `which` from the partials of the last nnfac_nmf_plan_fused_beta pass over side
+// `which`: F_out = max(F_in * (num / den)^gamma, floor_value) (mu.py:84-97), installed in the plan.  One kernel.
+int nnfac_nmf_plan_mu_finish_beta(nnfac_nmf_plan* p, int which, const float* F_in, int64_t ld_in, const float* den_partial, double gamma,
+                                  double floor_value, float* F_out, int64_t ld_out, void* stream) {
+  NNFAC_ARG(p && F_in && den_partial && F_out && (which == 0 || which == 1), "nnfac_nmf_plan_mu_finish_beta: bad argument");
+  const int64_t len = which == 0 ? p->m : p->n;
+  NNFAC_ARG(ld_in >= len && ld_out >= len, "nnfac_nmf_plan_mu_finish_beta: leading dimension too small");
+  if (p->base || !p->fused_ok || p->rk != 64 || p->planes != 2) {
+    nnfac_set_error("nnfac_nmf_plan_mu_finish_beta: covers the plans of nnfac_nmf_plan_fused_beta (rank <= 64, 2 planes, no view)");
+    return NNFAC_ERR_UNSUPPORTED;
+  }
+  const Side* cs = &p->side[which == 0 ? 1 : 0];
+  const Side* ps = &p->side[which];
+  PeerG none;
+  memset(&none, 0, sizeof(none));
+  factor_finish_kernel<true, 64, false, 2, true><<<(unsigned)ceil_div64(len, 32), 256, 0, (cudaStream_t)stream>>>(
+      p->partial, ps->cp.splits, p->r, p->r_pad, len, ps->cp.ld_partial, F_in, ld_in, 0, 0, none, den_partial, (float)floor_value,
+      F_out, ld_out, cs->fh, cs->fl, cs->ld, p->rowp_h[which], p->rowp_l[which], nullptr, nullptr, (float)gamma);
+  NNFAC_LAUNCH_CHECK(p->ctx);
   return NNFAC_OK;
 }
 

@@ -34,18 +34,27 @@ import torch
 import nn_fac.update_rules.mu as mu
 from nn_fac import _lib as L
 from nn_fac import _ops as ops
+from nn_fac.utils.beta_divergence import gamma_beta
 
 MODE_RES, MODE_MU = 0, 1
 
 
 def eligible(dtype, rank, update_rule, beta, planes=2):
-    """fp32 on the tcgen05 path: HALS and Frobenius MU up to rank 128 (residual + cross-product pass), KL MU up to rank 64.
-    planes = 3 (precision "fp32x3"): all three up to rank 64."""
+    """fp32 on the tcgen05 path: HALS and Frobenius MU up to rank 128 (residual + cross-product pass), MU with any other
+    beta >= 0 up to rank 64 (beta = 1: one contraction; every other beta: numerator and denominator contractions).
+    planes = 3 (precision "fp32x3"): HALS and MU with beta = 1 or 2, up to rank 64."""
     if dtype != torch.float32:
         return False
     if update_rule == "hals" or (update_rule == "mu" and beta == 2):
         return rank <= (128 if planes == 2 else 64)
-    return update_rule == "mu" and beta == 1 and rank <= 64
+    if update_rule != "mu" or rank > 64:
+        return False
+    return beta == 1 or (planes == 2 and beta >= 0)
+
+
+def general_beta(update_rule, beta):
+    """MU with a beta that needs both contractions (the general-beta pass).  FusedNMF.run takes beta = None as 1."""
+    return update_rule == "mu" and beta is not None and beta != 1 and beta != 2
 
 
 def planes_of_precision():
@@ -340,6 +349,13 @@ class CudaEngine:
             self.set_factor(which, new)
             return new
         return self.plan.mu_finish(which, F, den_vec, mu.epsilon)
+
+    def fused_beta(self, side, beta, want_cost, cost_out=None):
+        return self.plan.fused_beta(side, beta, want_cost=want_cost, cost_out=cost_out)
+
+    def mu_finish_beta(self, which, F, beta):
+        """mu.py:84-97 from the two partial sets of the last fused_beta(which), plus the installation of the new factor."""
+        return self.plan.mu_finish_beta(which, F, gamma_beta(beta), mu.epsilon)
 
     def cross(self, which, F):
         return self.plan.cross(which, F)
@@ -691,9 +707,26 @@ class FusedNMF:
                 V = eng.mu_finish(1, V, join() if join is not None else eng.row_sums(Ut))   # mu.py:27
         return Ut, V
 
+    def _apply_mu_beta(self, beta, fixed_modes):
+        """General-beta multiplicative update (mu.py:84-97) from the partials of the first pass: both contractions of each
+        factor come out of one pass over X, and the finish kernel divides, raises to gamma and installs."""
+        Ut, V, eng = self.Ut, self.V, self.eng
+        if 0 not in fixed_modes:
+            with self._phase("apply_U"):
+                Ut = eng.mu_finish_beta(0, Ut, beta)
+        if 1 not in fixed_modes:
+            with self._phase("pass_V"):
+                eng.fused_beta(1, beta, False)
+            with self._phase("apply_V"):
+                V = eng.mu_finish_beta(1, V, beta)
+        return Ut, V
+
     def run(self, n_iter_max, tol, update_rule, sparsity=(None, None), fixed_modes=(), normalize=(False, False),
             verbose=False, beta=None):
         """The reference's outer loop (nmf.py:298-324).  Returns (costs, toc)."""
+        gen = general_beta(update_rule, beta)
+        if gen and self.comm.world > 1:
+            raise NotImplementedError("the column-sharded path covers MU with beta = 1 or 2 only")
         mu2 = update_rule == "mu" and beta == 2       # Frobenius MU: cross products + squared residual, like HALS
         if mu2 and self.comm.world > 1:
             px = self._exchange(self.r) if hasattr(self.eng, "plan") else None
@@ -720,7 +753,7 @@ class FusedNMF:
                 # hence for every peer's pull of the partial Grams)
                 px = self._exchange(self.r) if (self.comm.world > 1 and mode == MODE_RES and hasattr(self.eng, "plan")) else None
                 VVt_join = self._gram_async(0, self.V, out=px.tailblk[:, :self.r] if px is not None else None)
-            if mode == MODE_MU and self.comm.world == 1 and it < n_iter_max and 0 not in fixed_modes:
+            if mode == MODE_MU and not gen and self.comm.world == 1 and it < n_iter_max and 0 not in fixed_modes:
                 den_join = self._row_sums_async(0, self.V)                         # row sums of V under the first pass
             with self._phase("pass_U"):
                 # single GPU: the numerator (MU) / cross product (HALS) stays in the plan as split partials, consumed by
@@ -732,7 +765,11 @@ class FusedNMF:
                 keep = keep or (self.comm.world > 1 and mode == MODE_RES and it < n_iter_max and 0 not in fixed_modes
                                 and (mu2 or not normalize[0]) and hasattr(self.eng, "plan"))
                 # the cost lands directly in the scalar block that travels to the host
-                if self.comm.world > 1 and mode == MODE_MU and it < n_iter_max and 0 not in fixed_modes and self._exchange(1) is not None:
+                if gen:
+                    # numerator and denominator partials of U's update stay in the plan and the plan object
+                    outA = None
+                    self.eng.fused_beta(0, beta, True, cost_out=self._dev_scal[0:1])
+                elif self.comm.world > 1 and mode == MODE_MU and it < n_iter_max and 0 not in fixed_modes and self._exchange(1) is not None:
                     # sharded MU over peer memory: the fused pass writes the numerator partials into the owners' inboxes
                     outA, _ = self.eng.fused(0, mode, True, keep_partials=True, cost_out=self._dev_scal[0:1])
                 elif self.comm.world > 1 and mode == MODE_MU and hasattr(self.eng, "plan"):
@@ -752,7 +789,9 @@ class FusedNMF:
                     done.record()
             # launch iteration `it` before looking at the cost of iteration it-1
             if it < n_iter_max:
-                if mu2:
+                if gen:
+                    new_Ut, new_V = self._apply_mu_beta(beta, fixed_modes)
+                elif mu2:
                     new_Ut, new_V = self._apply_mu2(outA, fixed_modes, VVt_join)
                 elif mode == MODE_RES:
                     new_Ut, new_V = self._apply_hals(outA, sparsity, fixed_modes, normalize, VVt_join)

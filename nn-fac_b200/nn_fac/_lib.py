@@ -90,6 +90,9 @@ SIGNATURES = {
     "nnfac_nmf_plan_hals_solve": [_P, _INT, _P, _I64, _P, _I64, _P, _I64, _P, _I64, _INT, _DBL, _DBL, _P, _P],
     "nnfac_nmf_plan_fused": [_P, _INT, _INT, _INT, _P, _I64, _P, _P],
     "nnfac_nmf_plan_mu_finish": [_P, _INT, _P, _I64, _P, _DBL, _P, _I64, _P],
+    "nnfac_nmf_plan_fused_beta_bytes": [_P, _c.POINTER(_c.c_size_t)],
+    "nnfac_nmf_plan_fused_beta": [_P, _INT, _DBL, _INT, _P, _P, _P],
+    "nnfac_nmf_plan_mu_finish_beta": [_P, _INT, _P, _I64, _P, _DBL, _DBL, _P, _I64, _P],
     "nnfac_nmf_plan_info": [_P, _INT, _c.POINTER(_INT), _c.POINTER(_INT), _c.POINTER(_INT), _c.POINTER(_INT),
                             _c.POINTER(_INT)],
 }

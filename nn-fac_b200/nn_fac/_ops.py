@@ -303,6 +303,7 @@ class NMFPlan:
         self.planes = 2
         self._xf32 = None
         self._xf32_refused = False
+        self._den = None
         self._X = X
 
     def bind_rank(self, r, sides=3, planes=2):
@@ -338,6 +339,7 @@ class NMFPlan:
         v = NMFPlan.__new__(NMFPlan)
         v.device, v.m, v.n, v.r, v.sides, v.planes = self.device, I, left * right, r, 1, 2
         v._xf32, v._xf32_refused, v._X, v._base = None, True, None, self          # keeps the base plan (and its planes) alive
+        v._den = None
         v._workspace = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
         v.handle = ctypes.c_void_p()
         L.check(_lib().nnfac_nmf_plan_create_view(L.ctx(self.device), self.handle, left, I, right, r, L.ptr(v._workspace), nbytes.value,
@@ -447,18 +449,8 @@ class NMFPlan:
         mode 1: beta=1 MU numerator + KL(X|UV).  Returns (out r x rows, cost device scalar or None).
         keep_partials: leave the split partials in the plan for mu_finish instead of reducing them into `out`."""
         R = self.m if side == 0 else self.n
-        # The beta = 1 pass only needs x in registers (never as a tensor-core operand): from an fp32 copy of X it saves three
-        # instructions per element (no bf16 unpack + add).  With the issuing warps converged the pass is bound by the issue
-        # slots of its transform warps, and the copy pays: MU 905 -> 950 it/s at C2.  It costs 2 x 4mn bytes, so it is made on
-        # first use only when that leaves at least as much memory free again (NNFAC_MU_F32=0 / 1 force it off / on).
-        # A 3-plane plan's beta = 1 pass always reads the copy (then the caller's fp32 values).
-        if mode == 1 and self._xf32 is None and self.fused_ok and self.sides == 3 and not self._xf32_refused:
-            want = os.environ.get("NNFAC_MU_F32", "auto")
-            need = 2 * 4 * self.m * self.n
-            if self.planes == 3 or want == "1" or (want != "0" and torch.cuda.mem_get_info(self.device)[0] > 2 * need + (1 << 30)):
-                self.enable_f32()
-            else:
-                self._xf32_refused = True
+        if mode == 1:
+            self._want_f32()
         if out is None and not keep_partials:
             out = torch.empty((self.r, R), dtype=torch.float32, device=self.device)
         if cost_out is None and (want_cost or mode == 0):
@@ -466,6 +458,44 @@ class NMFPlan:
         L.check(_lib().nnfac_nmf_plan_fused(self.handle, side, mode, 1 if want_cost else 0, L.ptr(out),
                                             out.stride(0) if out is not None else 0, L.ptr(cost_out), L.stream_ptr()))
         return out, cost_out
+
+    def _want_f32(self):
+        """The beta = 1 and general-beta passes only need x in registers (never as a tensor-core operand): from an fp32 copy of X
+        they save three instructions per element (no bf16 unpack + add).  With the issuing warps converged the beta = 1 pass is
+        bound by the issue slots of its transform warps, and the copy pays: MU 905 -> 950 it/s at C2.  It costs 2 x 4mn bytes, so
+        it is made on first use only when that leaves at least as much memory free again (NNFAC_MU_F32=0 / 1 force it off / on).
+        A 3-plane plan's beta = 1 pass always reads the copy (then the caller's fp32 values)."""
+        if self._xf32 is None and self.fused_ok and self.sides == 3 and not self._xf32_refused:
+            want = os.environ.get("NNFAC_MU_F32", "auto")
+            need = 2 * 4 * self.m * self.n
+            if self.planes == 3 or want == "1" or (want != "0" and torch.cuda.mem_get_info(self.device)[0] > 2 * need + (1 << 30)):
+                self.enable_f32()
+            else:
+                self._xf32_refused = True
+
+    def fused_beta(self, side, beta, want_cost=True, cost_out=None):
+        """One general-beta pass (beta >= 0 other than 1 and 2, rank <= 64, two planes): the split partials of the numerator
+        (K^(beta-2) * X) V^T (side 0; its twin for V on side 1) stay in the plan, those of the denominator K^(beta-1) V^T in a
+        buffer the plan object owns; both are consumed by mu_finish_beta.  Returns the cost (device scalar) or None."""
+        import ctypes
+        self._want_f32()
+        if self._den is None:
+            nbytes = ctypes.c_size_t()
+            L.check(_lib().nnfac_nmf_plan_fused_beta_bytes(self.handle, ctypes.byref(nbytes)))
+            self._den = torch.empty(nbytes.value // 4, dtype=torch.float32, device=self.device)
+        if cost_out is None and want_cost:
+            cost_out = torch.empty(1, dtype=torch.float64, device=self.device)
+        L.check(_lib().nnfac_nmf_plan_fused_beta(self.handle, side, float(beta), 1 if want_cost else 0, L.ptr(self._den),
+                                                 L.ptr(cost_out), L.stream_ptr()))
+        return cost_out
+
+    def mu_finish_beta(self, which, F, gamma, floor):
+        """max(F * (num / den)^gamma, floor) from the two partial sets of the last fused_beta(which); the result is installed as
+        factor `which` (mu.py:84-97 + set_factor in one kernel)."""
+        out = torch.empty_like(F)
+        L.check(_lib().nnfac_nmf_plan_mu_finish_beta(self.handle, which, L.ptr(F), F.stride(0), L.ptr(self._den), float(gamma),
+                                                     float(floor), L.ptr(out), out.stride(0), L.stream_ptr()))
+        return out
 
     def enable_f32(self):
         """fp32 copies of X / X^T for the beta = 1 fused pass (made from the planes on first use)."""

@@ -26,6 +26,8 @@ def compute_nmf_sharded(data_block, rank, U_in, V_block, n_iter_max=100, tol=1e-
     """compute_nmf on this rank's column block.  Returns (U, V_block) or (U, V_block, cost_fct_vals, toc):
     U and the costs are identical on every rank, V_block is this rank's columns of V."""
     _check_step_arguments(update_rule, beta, sparsity_coefficients)
+    if _fast.general_beta(update_rule, beta):
+        raise NotImplementedError(f"the sharded path covers update_rule 'mu' with beta = 1 or 2 only (got beta = {beta})")
     if _fast.planes_of_precision() == 3:
         raise NotImplementedError("precision 'fp32x3' is not covered by the sharded path (its exchanges write two planes)")
     if not _fast.eligible(torch.float32, int(np.shape(U_in)[1]), update_rule, beta):
