@@ -263,7 +263,8 @@ int nnfac_nmf_plan_create_planes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, in
  * addressed in place through TMA maps over the SAME planes -- the reference copies the tensor once per mode (ntf.py:309-311).
  * The tensor is read as (left, I, right); the view is the I x (left*right) unfolding of the middle axis: the last mode
  * (right == 1, I % 8 == 0) as an MN-major tensor-core operand, middle modes (right % 64 == 0) through a 3-D map.  A view supports
- * nnfac_nmf_plan_set_krao, nnfac_nmf_plan_cross(which = 0), _reduce and _info; NNFAC_ERR_UNSUPPORTED when the extents do not
+ * nnfac_nmf_plan_set_krao, nnfac_nmf_plan_cross(which = 0), _reduce and _info, and at rank <= 64 the NTF multiplicative update
+ * (set_factor_rows, fused(mode 1), fused_beta, mu_finish_rows); NNFAC_ERR_UNSUPPORTED when the extents do not
  * allow it (the caller then builds a one-sided plan on a copy of that unfolding).  `base` must outlive the view. */
 int nnfac_nmf_plan_view_bytes(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, int64_t I, int64_t right, int r, size_t* bytes);
 int nnfac_nmf_plan_create_view(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, int64_t I, int64_t right, int r,
@@ -304,7 +305,7 @@ int nnfac_nmf_plan_reduce(nnfac_nmf_plan* plan, int side, float* out, int64_t ld
 int nnfac_nmf_plan_reduce_chunked(nnfac_nmf_plan* plan, int side, float* out, int64_t chunk, int slabs, const float* tail,
                                   int64_t ld_tail, int tail_cols, void* stream);
 /* Install a factor into the plan (builds all of its bf16 operand planes):
- * which = 0: U, passed as U^T (r x m, row-major); which = 1: V (r x n). */
+ * which = 0: U, passed as U^T (r x m, row-major); which = 1: V (r x n).  Refused on views (nnfac_nmf_plan_set_factor_rows). */
 int nnfac_nmf_plan_set_factor(nnfac_nmf_plan* plan, int which, const float* Ft, int64_t ld, void* stream);
 /* The same from the output of an all-gather of column slices, G = [slices][r][chunk] (slice s = columns
  * [s*chunk, (s+1)*chunk) of the factor); also writes the factor itself, rank-major, into Ft_out (r x len). */
@@ -340,7 +341,10 @@ int nnfac_nmf_plan_hals_solve(nnfac_nmf_plan* plan, int which, const float* UtM,
  *   mode 0: out (r x rows) = the HALS cross product of nmf.py:408 / :433, cost_out = ||X - U V||_F^2 (nmf.py:452)
  *   mode 1: out (r x rows) = the beta=1 MU numerator ((X / UV) V^T)^T of mu.py:84-88 (side 0) or its
  *           transposed twin for V (mu.py:27, side 1); cost_out = KL(X | U V) when want_cost != 0.
- * cost_out is a device double and may be NULL.  out may be NULL in mode 1 (see nnfac_nmf_plan_mu_finish). */
+ * cost_out is a device double and may be NULL.  out may be NULL in mode 1 (see nnfac_nmf_plan_mu_finish).
+ * One-sided plans (sides = 1) and views, mode 1: the NTF update of the mode whose unfolding side 0 is -- "V" is the Khatri-Rao
+ * operand installed by nnfac_nmf_plan_set_krao (or set_factor(which = 1)), "U" factor 0; X is read where the plan addresses it
+ * (views: in place) and only in registers.  Mode 0 is refused on views. */
 int nnfac_nmf_plan_fused(nnfac_nmf_plan* plan, int side, int mode, int want_cost, float* out, int64_t ld_out,
                          double* cost_out, void* stream);
 /* beta = 1 multiplicative update of factor `which` (0: U as U^T, 1: V), mu.py:84-88, straight from the numerator
@@ -353,7 +357,8 @@ int nnfac_nmf_plan_mu_finish(nnfac_nmf_plan* plan, int which, const float* F_in,
  * and consumed on chip.  The split partials of the numerator (K^(beta-2) * X) V^T (side 0; its twin for V on side 1) stay in the
  * plan; those of the denominator K^(beta-1) V^T go to den_partial, a caller-owned device buffer of at least
  * nnfac_nmf_plan_fused_beta_bytes bytes.  cost_out (device double, may be NULL): the beta-divergence of X from U V when
- * want_cost != 0.  NNFAC_ERR_UNSUPPORTED for rank > 64, 3-plane plans, view plans, plans with the push exchange set, and
+ * want_cost != 0.  One-sided plans and views: side 0, "V" = the Khatri-Rao operand of nnfac_nmf_plan_set_krao, as in
+ * nnfac_nmf_plan_fused.  NNFAC_ERR_UNSUPPORTED for rank > 64, 3-plane plans, plans with the push exchange set, and
  * beta = 1 or 2 (nnfac_nmf_plan_fused). */
 int nnfac_nmf_plan_fused_beta_bytes(const nnfac_nmf_plan* plan, size_t* bytes);
 int nnfac_nmf_plan_fused_beta(nnfac_nmf_plan* plan, int side, double beta, int want_cost, float* den_partial, double* cost_out,
@@ -362,6 +367,16 @@ int nnfac_nmf_plan_fused_beta(nnfac_nmf_plan* plan, int side, double beta, int w
  * (both summed in the order of nnfac_nmf_plan_reduce): F_out = max(F_in * (num / den)^gamma, floor_value), gamma = the
  * exponent of beta_divergence.py:75-80; F_out is installed in the plan as nnfac_nmf_plan_set_factor would do.  One kernel. */
 int nnfac_nmf_plan_mu_finish_beta(nnfac_nmf_plan* plan, int which, const float* F_in, int64_t ld_in, const float* den_partial,
+                                  double gamma, double floor_value, float* F_out, int64_t ld_out, void* stream);
+/* Factor 0 of a one-sided plan or view of rank <= 64 (F^T, r x m) installed as its row planes only: the operand of the NTF MU
+ * pass (nnfac_nmf_plan_fused mode 1 / _fused_beta on such a plan). */
+int nnfac_nmf_plan_set_factor_rows(nnfac_nmf_plan* plan, const float* Ft, int64_t ld, void* stream);
+/* The update of factor 0 of a one-sided plan or view (rank <= 64; the NTF factor of the plan's mode, rank-major r x m) from the
+ * partials of its last MU pass over side 0: after nnfac_nmf_plan_fused(mode 1), den = r floats (the column sums of the
+ * Khatri-Rao operand) and F_out = max(F_in * num / den[k], floor_value); after nnfac_nmf_plan_fused_beta, den_partial = its
+ * denominator partials and F_out = max(F_in * (num / den)^gamma, floor_value).  Exactly one of den / den_partial.  F_out is
+ * installed as the row planes of factor 0 (no other planes). */
+int nnfac_nmf_plan_mu_finish_rows(nnfac_nmf_plan* plan, const float* F_in, int64_t ld_in, const float* den, const float* den_partial,
                                   double gamma, double floor_value, float* F_out, int64_t ld_out, void* stream);
 /* Work decomposition chosen for one side (for benchmarks / DESIGN.md); any pointer may be NULL. */
 int nnfac_nmf_plan_info(const nnfac_nmf_plan* plan, int which, int* splits, int* stages_per_unit,

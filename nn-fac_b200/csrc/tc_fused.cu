@@ -92,6 +92,8 @@ struct BetaParams {
   int ibm2, ibeta;                 // MODE_BETAI: beta - 2 and beta as integers
   float inv_bb1, inv_beta;         // 1 / (beta (beta - 1)), 1 / beta
   float hc[NHC];
+  int kb_per_slab;                 // NTF middle-mode views (AMODE 2): 64-wide k-blocks per slab of the 3-D map.  Kept here, behind
+                                   // every field the other passes read, so that their kernels compile as before
 };
 
 __device__ __forceinline__ float rcp_approx(float x) {   // MUFU.RCP, <= 1 ulp: no IEEE fix-up branch
@@ -156,7 +158,14 @@ __device__ __forceinline__ float bf_lo(uint32_t w) { return __uint_as_float(w <<
 __device__ __forceinline__ float bf_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
 
 // map_xm / map_fkm / map_a1m: the middle planes (PLANES = 3 only).
-template <int MODE, bool COST, bool XF32, int RK, int PLANES = 2>
+//
+// KRAO (NTF: one-sided plans and views, MODE_MU / MODE_BETA*, rank <= 64, 2 planes): the factor slab of a stage is 64 columns of
+// the Khatri-Rao operand as set_krao writes it, the K-major planes [r_pad x ld] of side 0 (a 64 x 64 box; ranks beyond r_pad read
+// as zeros): the contraction GEMM reads it K-major, the model GEMM MN-major.  AMODE addresses X as tc_cross_kernel does:
+// 0 rows of a 2-D map; 2 a middle mode through the 3-D map {right, I, left} (the same 128 x 64 K-major tile); 1 the last mode,
+// two 64 x 64 boxes of the planes read as [left x I] (an MN-major tile: the transform reads its row's columns transposed).
+// X only passes through registers there, so its addressing changes nothing else.
+template <int MODE, bool COST, bool XF32, int RK, int PLANES = 2, int AMODE = 0, bool KRAO = false>
 __global__ void __launch_bounds__(FUSED_THREADS, 1)
 tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constant__ CUtensorMap map_xl,
                 const __grid_constant__ CUtensorMap map_fkh, const __grid_constant__ CUtensorMap map_fkl,
@@ -168,6 +177,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
   static_assert(!BETA || (RK == 64 && PLANES == 2), "general beta: 2 planes, rank <= 64");
   static_assert(RK == 64 || (MODE == MODE_RES && !XF32), "rank 65..128: residual + cross-product pass only");
   static_assert(PLANES == 2 || (RK == 64 && (MODE == MODE_RES) != XF32), "3 planes: rank <= 64; beta = 1 reads X from its fp32 copy");
+  static_assert(!KRAO || (RK == 64 && PLANES == 2 && !XF32 && MODE != MODE_RES), "Khatri-Rao operand: MU / general beta, 2 planes, rank <= 64");
+  static_assert(AMODE == 0 || KRAO, "X addressing modes 1 and 2: NTF views only");
   constexpr int FSTAGES = C::FSTAGES, ND1 = BETA ? 2 : C::ND1, CWD = C::CWD;
   constexpr int NQ = BETA ? 1 : 2;     // ratio-tile buffers in tensor memory
   // 3 planes: one stage per contraction chain (24 MMAs, as many as two stages of the 2-plane products), drained two stages late
@@ -239,15 +250,32 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         uint8_t* st = ring + (size_t)stage * STAGE_BYTES;
         tc::mbar_arrive_expect_tx(&full[stage], STAGE_BYTES);
         const int c = k0 + ks * BK;
+        if constexpr (AMODE == 1) {
+#pragma unroll
+          for (int mb = 0; mb < 2; ++mb) {             // rows row0 + 64 mb .. + 63 of the tile, columns c .. c + 63
+            tc::tma_load_2d_hint(st + mb * 8192, &map_xh, &full[stage], row0 + 64 * mb, c, tc::kEvictFirst);
+            tc::tma_load_2d_hint(st + X_BYTES + mb * 8192, &map_xl, &full[stage], row0 + 64 * mb, c, tc::kEvictFirst);
+          }
+        } else if constexpr (AMODE == 2) {
+          const int b = c / BK, slab = b / bp.kb_per_slab, off = (b - slab * bp.kb_per_slab) * BK;
+          tc::tma_load_3d_hint(st, &map_xh, &full[stage], off, row0, slab, tc::kEvictFirst);
+          tc::tma_load_3d_hint(st + X_BYTES, &map_xl, &full[stage], off, row0, slab, tc::kEvictFirst);
+        } else {
         // XF32: map_xh is the fp32 copy of X; the two 16 KiB halves of the tile are its columns [c, c+32) and [c+32, c+64)
         tc::tma_load_2d_hint(st, &map_xh, &full[stage], c, row0, tc::kEvictFirst);
         tc::tma_load_2d_hint(st + X_BYTES, XF32 ? &map_xh : &map_xl, &full[stage], XF32 ? c + 32 : c, row0, tc::kEvictFirst);
         if (PLANES == 3 && !XF32) tc::tma_load_2d_hint(st + 2 * X_BYTES, &map_xm, &full[stage], c, row0, tc::kEvictFirst);
+        }
+        if constexpr (KRAO) {                          // ranks 0 .. 63 x columns c .. c + 63 of the Khatri-Rao planes
+          tc::tma_load_2d_hint(st + XB, &map_fkh, &full[stage], c, 0, tc::kEvictLast);
+          tc::tma_load_2d_hint(st + XB + FK_BYTES, &map_fkl, &full[stage], c, 0, tc::kEvictLast);
+        } else {
 #pragma unroll
         for (int kr = 0; kr < C::KR; ++kr) {   // 64 columns of X x 64 ranks per box
           tc::tma_load_2d_hint(st + XB + kr * 8192, &map_fkh, &full[stage], kr * 64, c, tc::kEvictLast);
           tc::tma_load_2d_hint(st + XB + FK_BYTES + kr * 8192, &map_fkl, &full[stage], kr * 64, c, tc::kEvictLast);
           if (PLANES == 3) tc::tma_load_2d_hint(st + XB + 2 * FK_BYTES + kr * 8192, &map_fkm, &full[stage], kr * 64, c, tc::kEvictLast);
+        }
         }
         if (++stage == FSTAGES) { stage = 0; phase ^= 1; }
       }
@@ -255,7 +283,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
   } else if (warp == 1) {
     // ===================== MMA issuer 1: model GEMM  D1 = A1 * Fk^T =====================
     // (two issuing warps, each running its loop converged with one elected lane issuing: see tc::elect_one)
-    const uint32_t idesc1 = tc::umma_idesc_bf16(TILE_ROWS, 64);
+    // KRAO: the slab is [ranks x columns], columns contiguous -> B operand MN-major, a K step (16 ranks) is 16 rows of 128 B
+    const uint32_t idesc1 = tc::umma_idesc_bf16(TILE_ROWS, 64) | (KRAO ? (1u << 16) : 0u);
     const int ksteps = p.r_pad / UMMA_K;             // the planes are zero beyond r_pad: shorter contraction for small ranks
     int st1 = 0; uint32_t ph1 = 0;
     int b1 = 0; uint32_t b1_phase = 0;
@@ -269,7 +298,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
         tc::tcgen05_fence_after();
         if (tc::elect_one()) {
           const uint32_t sb = tc::smem_u32(ring + (size_t)st1 * STAGE_BYTES);
-          const uint64_t fkh = tc::umma_desc_k_sw128(sb + XB), fkl = tc::umma_desc_k_sw128(sb + XB + FK_BYTES);
+          const uint64_t fkh = KRAO ? tc::umma_desc_mn_sw128(sb + XB) : tc::umma_desc_k_sw128(sb + XB);
+          const uint64_t fkl = KRAO ? tc::umma_desc_mn_sw128(sb + XB + FK_BYTES) : tc::umma_desc_k_sw128(sb + XB + FK_BYTES);
           const uint32_t d = D1 + (uint32_t)b1 * 64;
           if constexpr (PLANES == 3) {
             // the five small products over the whole contraction first, the hi * hi ones last (truncating accumulation)
@@ -295,7 +325,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #pragma unroll
             for (int k = 0; k < RK / UMMA_K; ++k) {
               if (k < ksteps) {
-                const uint64_t ko = (uint64_t)(k * 2), bo = (uint64_t)((k & 3) * 2);
+                const uint64_t ko = (uint64_t)(k * 2), bo = KRAO ? (uint64_t)(k * 128) : (uint64_t)((k & 3) * 2);
                 tc::umma_bf16(d, ah + ko, fkh + bo, idesc1, k != 0);
                 tc::umma_bf16(d, al + ko, fkh + bo, idesc1, true);
                 tc::umma_bf16(d, ah + ko, fkl + bo, idesc1, true);
@@ -305,7 +335,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #pragma unroll
           for (int k = 0; k < RK / UMMA_K; ++k) {
             if (k < ksteps) {
-              const uint64_t bo = (uint64_t)((k >> 2) * (8192 >> 4) + (k & 3) * 2);   // 64-rank atom, 32 B inside its 128 B row
+              const uint64_t bo = KRAO ? (uint64_t)(k * 128)                             // 16 rank rows of 128 B
+                                       : (uint64_t)((k >> 2) * (8192 >> 4) + (k & 3) * 2);   // 64-rank atom, 32 B inside its 128 B row
               tc::umma_bf16_ts(d, A1T + 8 * k, fkh + bo, idesc1, k != 0);
               tc::umma_bf16_ts(d, A1T + RK / 2 + 8 * k, fkh + bo, idesc1, true);
               tc::umma_bf16_ts(d, A1T + 8 * k, fkl + bo, idesc1, true);
@@ -322,7 +353,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
     }
   } else if (warp == 3) {
     // ===================== MMA issuer 2: contraction GEMM  D2 += A2 * Fn^T =====================
-    const uint32_t idesc2 = tc::umma_idesc_bf16(TILE_ROWS, p.r_pad) | (1u << 16);   // B operand MN-major
+    // B operand MN-major (the rank-contiguous slab); KRAO: K-major (the Khatri-Rao planes, columns contiguous)
+    const uint32_t idesc2 = tc::umma_idesc_bf16(TILE_ROWS, p.r_pad) | (KRAO ? 0u : (1u << 16));
     int qb = 0; uint32_t qb_phase = 0;      // Q buffer (MU)
     int st2 = 0; uint32_t ph2 = 0;
     int b2 = 0; uint32_t b2_phase = 0;      // D2 buffer
@@ -339,8 +371,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
           const uint64_t xh = tc::umma_desc_k_sw128(sb), xl = tc::umma_desc_k_sw128(sb + X_BYTES);
           // B operand = the SAME 64-column slab of the other factor that the model GEMM reads K-major, addressed
           // MN-major here (rank contiguous = N, columns = K): no second copy of the factor travels through L2
-          const uint64_t fnh = tc::umma_desc_mn_sw128(sb + XB);
-          const uint64_t fnl = tc::umma_desc_mn_sw128(sb + XB + FK_BYTES);
+          const uint64_t fnh = KRAO ? tc::umma_desc_k_sw128(sb + XB) : tc::umma_desc_mn_sw128(sb + XB);
+          const uint64_t fnl = KRAO ? tc::umma_desc_k_sw128(sb + XB + FK_BYTES) : tc::umma_desc_mn_sw128(sb + XB + FK_BYTES);
           const uint32_t d = D2 + (uint32_t)b2 * RK;
           if constexpr (PLANES == 3) {
             // small products of the stage first, hi * hi last (see the model GEMM)
@@ -374,7 +406,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
             const uint32_t dd = D2D + (uint32_t)b2 * RK;
 #pragma unroll
             for (int k = 0; k < BK / UMMA_K; ++k) {
-              const uint64_t kb = (uint64_t)(k * 128);
+              const uint64_t kb = KRAO ? (uint64_t)(k * 2) : (uint64_t)(k * 128);   // KRAO: 16 columns = 32 B inside the 128 B row
               const uint32_t qa = QT + 8 * k, qd = qa + 64;
               const bool acc0 = !(chain_start && k == 0);
               tc::umma_bf16_ts(d, qa, fnh + kb, idesc2, acc0);
@@ -388,7 +420,8 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
             const uint64_t ko = (uint64_t)(k * 2);            // A (K-major): 16 bf16 = 32 B inside the 128 B row
-            const uint64_t kb = (uint64_t)(k * 128);          // B (MN-major): 16 rows of 128 B = 2048 B
+            const uint64_t kb = KRAO ? (uint64_t)(k * 2)      // B (KRAO, K-major): 32 B inside the 128 B row
+                                     : (uint64_t)(k * 128);   // B (MN-major): 16 rows of 128 B = 2048 B
             if (MODE == MODE_MU) {
               const uint32_t qa = QT + (uint32_t)qb * 64 + 8 * k;
               tc::umma_bf16_ts(d, qa, fnh + kb, idesc2, !(chain_start && k == 0));
@@ -556,6 +589,23 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap map_xh, const __grid_constan
               const int chunk = 4 * (part & 1) + 2 * cc + h;
               const float4 v4 = *reinterpret_cast<const float4*>(xb + ((chunk ^ (row & 7)) << 4));
               xv[2 * h] = make_float2(v4.x, v4.y); xv[2 * h + 1] = make_float2(v4.z, v4.w);
+            }
+          } else if constexpr (AMODE == 1) {
+            // MN-major tile: this thread's row is element (row & 63) of the 128 B rows of box (row >> 6), one row per column.  The
+            // 32 lanes of a warp read 64 neighbouring bytes of the same row: no bank conflict.
+            const uint8_t* xb = xh + (row >> 6) * 8192 + (row & 7) * 2;
+            const int rc = (row & 63) >> 3;
+#pragma unroll
+            for (int w = 0; w < 4; ++w) {
+              float v[2];
+#pragma unroll
+              for (int h = 0; h < 2; ++h) {
+                const int col = CW * part + 8 * cc + 2 * w + h;
+                const uint32_t off = (uint32_t)col * 128u + (uint32_t)((rc ^ (col & 7)) << 4);
+                const uint32_t hb = *reinterpret_cast<const uint16_t*>(xb + off), lb = *reinterpret_cast<const uint16_t*>(xb + X_BYTES + off);
+                v[h] = __uint_as_float(hb << 16) + __uint_as_float(lb << 16);
+              }
+              xv[w] = make_float2(v[0], v[1]);
             }
           } else {
             const int chunk = NCHK * part + cc;
@@ -783,8 +833,9 @@ struct PeerG {                      // PULL: slice s of the factor lives in p[s]
   unsigned long long seq;
 };
 
-// PLANES = 3: the middle planes go to fm / rowm.
-template <bool APPLY, int RK, bool PULL, int PLANES = 2, bool DENP = false>
+// PLANES = 3: the middle planes go to fm / rowm.  KPLANES = false (one-sided plans and views, nnfac_nmf_plan_mu_finish_rows):
+// no K-major planes; the factor is the one aligned with the rows of side 0, installed as its row planes only.
+template <bool APPLY, int RK, bool PULL, int PLANES = 2, bool DENP = false, bool KPLANES = true>
 __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restrict__ partial, int splits, int r, int r_pad, int64_t R,
                                                             int64_t ldp, const float* __restrict__ F_in, int64_t ld_in,
                                                             int64_t in_chunk, int64_t in_slab, const PeerG G,
@@ -852,6 +903,7 @@ __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restr
         if (v != v) f = v;
       }
       if (F_out) F_out[(int64_t)k * ld_out + c] = f;
+      if constexpr (KPLANES) {
       bf16 h, l;
       if constexpr (PLANES == 3) {
         bf16 md;
@@ -862,6 +914,7 @@ __global__ void __launch_bounds__(256) factor_finish_kernel(const float* __restr
       }
       fh[(int64_t)k * ld_plane + c] = h;
       fl[(int64_t)k * ld_plane + c] = l;
+      }
     }
     tile[k][tx] = f;
   }
@@ -978,6 +1031,26 @@ static FusedParams fused_params(const nnfac_nmf_plan* p, int side, bool want_cos
   fp.push_chunk = 0; fp.push_src = 0;
   for (int q = 0; q < NNFAC_MAX_PEERS; ++q) fp.push[q] = nullptr;
   return fp;
+}
+
+// The MU / general-beta pass of a one-sided plan or a view (NTF): X of side 0 as the plan addresses it, the Khatri-Rao operand
+// from the K-major planes of side 0 (nnfac_nmf_plan_set_krao), A1 from the row planes of factor 0.
+template <int M, bool C, int AM>
+static cudaError_t launch_krao_am(const nnfac_nmf_plan* p, const FusedParams& fp, const BetaParams& bp, cudaStream_t st) {
+  const Side* s = &p->side[0];
+  const size_t smem = Cfg<64>::SMEM;
+  const cudaError_t e = cudaFuncSetAttribute(tc_fused_kernel<M, C, false, 64, 2, AM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  tc_fused_kernel<M, C, false, 64, 2, AM, true><<<s->grid, FUSED_THREADS, smem, st>>>(s->map_xh, s->map_xl, s->map_kh, s->map_kl,
+      p->map_row_a_h[0], p->map_row_a_l[0], fp, s->map_xh, s->map_kh, p->map_row_a_h[0], bp);
+  return cudaSuccess;
+}
+template <int M, bool C>
+static cudaError_t launch_krao(const nnfac_nmf_plan* p, const FusedParams& fp, BetaParams bp, cudaStream_t st) {
+  const CrossParams& cp = p->side[0].cp;
+  bp.kb_per_slab = cp.kb_per_slab;
+  return cp.amode == 1 ? launch_krao_am<M, C, 1>(p, fp, bp, st) : cp.amode == 2 ? launch_krao_am<M, C, 2>(p, fp, bp, st)
+                                                                                 : launch_krao_am<M, C, 0>(p, fp, bp, st);
 }
 
 extern "C" {
@@ -1163,6 +1236,7 @@ int nnfac_nmf_plan_mu_finish(nnfac_nmf_plan* p, int which, const float* F_in, in
   const int64_t len = which == 0 ? p->m : p->n;
   NNFAC_ARG(ld_in >= len && ld_out >= len, "nnfac_nmf_plan_mu_finish: leading dimension too small");
   if (!p->fused_ok) { nnfac_set_error("nnfac_nmf_plan_mu_finish: rank %d > 128 is not covered by the fused pass", p->r); return NNFAC_ERR_UNSUPPORTED; }
+  if (p->base) { nnfac_set_error("nnfac_nmf_plan_mu_finish: a view has no side-1 planes (nnfac_nmf_plan_mu_finish_rows)"); return NNFAC_ERR_UNSUPPORTED; }
   if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_mu_finish: writes two planes, the plan has %d (apply + set_factor)", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   return finish_factor(p, which, true, F_in, ld_in, 0, 0, den, (float)floor_value, F_out, ld_out, (cudaStream_t)stream);
 }
@@ -1175,8 +1249,9 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
                          void* stream) {
   NNFAC_ARG(p && (side == 0 || side == 1) && (mode == 0 || mode == 1), "nnfac_nmf_plan_fused: bad argument");
   NNFAC_ARG((p->sides >> side) & 1, "nnfac_nmf_plan_fused: this plan keeps no planes of side %d", side);
-  if (!p->fused_ok) { nnfac_set_error("nnfac_nmf_plan_fused: not covered by the fused pass (rank %d > 128, or a view plan)", p->r); return NNFAC_ERR_UNSUPPORTED; }
+  if (!p->fused_ok) { nnfac_set_error("nnfac_nmf_plan_fused: not covered by the fused pass (rank %d > 128, or a view plan of rank > 64)", p->r); return NNFAC_ERR_UNSUPPORTED; }
   if (mode == 1 && p->rk != 64) { nnfac_set_error("nnfac_nmf_plan_fused: the beta = 1 pass covers rank <= 64 (rank %d)", p->r); return NNFAC_ERR_UNSUPPORTED; }
+  if (mode == 0 && p->base) { nnfac_set_error("nnfac_nmf_plan_fused: the residual pass reads row planes a view does not have (set_krao_rows)"); return NNFAC_ERR_UNSUPPORTED; }
   if (mode == 1 && p->planes == 3 && !p->xf_ready) { nnfac_set_error("nnfac_nmf_plan_fused: the beta = 1 pass of a 3-plane plan reads X from its fp32 copies (nnfac_nmf_plan_enable_f32)"); return NNFAC_ERR_UNSUPPORTED; }
   Side* s = &p->side[side];
   NNFAC_ARG(!out || ld_out >= s->R, "nnfac_nmf_plan_fused: leading dimension too small");
@@ -1189,6 +1264,8 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
     for (int q = 0; q < p->push_world; ++q) fp.push[q] = p->push[q];
   }
   const int other = 1 - side;
+  const bool krao = mode == 1 && p->sides == 1;       // one-sided plan or view: the Khatri-Rao operand of set_krao
+  if (krao && p->push_chunk > 0) { nnfac_set_error("nnfac_nmf_plan_fused: no push exchange on a one-sided plan"); return NNFAC_ERR_UNSUPPORTED; }
 #define NNFAC_LAUNCH_FUSED(M, C, XF, RKV, MAPH, MAPL)                                                                             \
   do {                                                                                                                        \
     const size_t smem = Cfg<RKV>::SMEM;                                                                                       \
@@ -1205,7 +1282,9 @@ int nnfac_nmf_plan_fused(nnfac_nmf_plan* p, int side, int mode, int want_cost, f
         p->map_row_b_l[other], p->map_row_a_h[side], p->map_row_a_l[side], fp, s->map_xm, p->map_row_b_m[other],             \
         p->map_row_a_m[side], bp);                                                                                            \
   } while (0)
-  if (p->planes == 3) {
+  if (krao) {
+    NNFAC_CUDA((fp.want_cost ? launch_krao<MODE_MU, true>(p, fp, bp, st) : launch_krao<MODE_MU, false>(p, fp, bp, st)));
+  } else if (p->planes == 3) {
     if (mode == 0) NNFAC_LAUNCH_FUSED3(MODE_RES, true, false, s->map_xh, s->map_xl);
     else if (fp.want_cost) NNFAC_LAUNCH_FUSED3(MODE_MU, true, true, p->map_xf[side], p->map_xf[side]);
     else NNFAC_LAUNCH_FUSED3(MODE_MU, false, true, p->map_xf[side], p->map_xf[side]);
@@ -1250,7 +1329,6 @@ int nnfac_nmf_plan_fused_beta(nnfac_nmf_plan* p, int side, double beta, int want
   NNFAC_ARG(beta >= 0.0, "nnfac_nmf_plan_fused_beta: beta must be >= 0 (got %g)", beta);
   NNFAC_ARG((p->sides >> side) & 1, "nnfac_nmf_plan_fused_beta: this plan keeps no planes of side %d", side);
   if (beta == 1.0 || beta == 2.0) { nnfac_set_error("nnfac_nmf_plan_fused_beta: beta = %g is the mode-1 / cross-product pass", beta); return NNFAC_ERR_UNSUPPORTED; }
-  if (p->base) { nnfac_set_error("nnfac_nmf_plan_fused_beta: not available on a view plan"); return NNFAC_ERR_UNSUPPORTED; }
   if (!p->fused_ok || p->rk != 64) { nnfac_set_error("nnfac_nmf_plan_fused_beta: covers rank <= 64 (rank %d)", p->r); return NNFAC_ERR_UNSUPPORTED; }
   if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_fused_beta: covers 2-plane plans (the plan has %d)", p->planes); return NNFAC_ERR_UNSUPPORTED; }
   if (p->push_chunk > 0) { nnfac_set_error("nnfac_nmf_plan_fused_beta: not available with the push exchange (nnfac_nmf_plan_set_push)"); return NNFAC_ERR_UNSUPPORTED; }
@@ -1280,7 +1358,13 @@ int nnfac_nmf_plan_fused_beta(nnfac_nmf_plan* p, int side, double beta, int want
     if (p->xf_ready) NNFAC_LAUNCH_BETA(M, C, true, p->map_xf[side], p->map_xf[side]);                                         \
     else NNFAC_LAUNCH_BETA(M, C, false, s->map_xh, s->map_xl);                                                                \
   } while (0)
-  if (beta == 0.0) { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETA0, true); else NNFAC_LAUNCH_BETA_X(MODE_BETA0, false); }
+  if (p->sides == 1) {      // one-sided plan or view: the Khatri-Rao operand of set_krao
+    if (side != 0) { nnfac_set_error("nnfac_nmf_plan_fused_beta: a one-sided plan passes over side 0"); return NNFAC_ERR_UNSUPPORTED; }
+    const bool wc = fp.want_cost != 0;
+    if (beta == 0.0) NNFAC_CUDA((wc ? launch_krao<MODE_BETA0, true>(p, fp, bp, st) : launch_krao<MODE_BETA0, false>(p, fp, bp, st)));
+    else if (integral) NNFAC_CUDA((wc ? launch_krao<MODE_BETAI, true>(p, fp, bp, st) : launch_krao<MODE_BETAI, false>(p, fp, bp, st)));
+    else NNFAC_CUDA((wc ? launch_krao<MODE_BETAG, true>(p, fp, bp, st) : launch_krao<MODE_BETAG, false>(p, fp, bp, st)));
+  } else if (beta == 0.0) { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETA0, true); else NNFAC_LAUNCH_BETA_X(MODE_BETA0, false); }
   else if (integral) { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETAI, true); else NNFAC_LAUNCH_BETA_X(MODE_BETAI, false); }
   else { if (fp.want_cost) NNFAC_LAUNCH_BETA_X(MODE_BETAG, true); else NNFAC_LAUNCH_BETA_X(MODE_BETAG, false); }
 #undef NNFAC_LAUNCH_BETA_X
@@ -1311,6 +1395,50 @@ int nnfac_nmf_plan_mu_finish_beta(nnfac_nmf_plan* p, int which, const float* F_i
   factor_finish_kernel<true, 64, false, 2, true><<<(unsigned)ceil_div64(len, 32), 256, 0, (cudaStream_t)stream>>>(
       p->partial, ps->cp.splits, p->r, p->r_pad, len, ps->cp.ld_partial, F_in, ld_in, 0, 0, none, den_partial, (float)floor_value,
       F_out, ld_out, cs->fh, cs->fl, cs->ld, p->rowp_h[which], p->rowp_l[which], nullptr, nullptr, (float)gamma);
+  NNFAC_LAUNCH_CHECK(p->ctx);
+  return NNFAC_OK;
+}
+
+// Factor 0 of a one-sided plan or view (rank <= 64; F^T, r x m) installed as its row planes only: the A1 operand of the MU pass
+// (a view has no side-1 planes, and that pass reads no others).
+int nnfac_nmf_plan_set_factor_rows(nnfac_nmf_plan* p, const float* Ft, int64_t ld, void* stream) {
+  NNFAC_ARG(p && Ft && ld >= p->m, "nnfac_nmf_plan_set_factor_rows: bad argument");
+  if (p->sides != 1 || !p->fused_ok || p->rk != 64 || p->planes != 2) {
+    nnfac_set_error("nnfac_nmf_plan_set_factor_rows: covers one-sided plans and views of rank <= 64 with 2 planes");
+    return NNFAC_ERR_UNSUPPORTED;
+  }
+  PeerG none;
+  memset(&none, 0, sizeof(none));
+  factor_finish_kernel<false, 64, false, 2, false, false><<<(unsigned)ceil_div64(p->m, 32), 256, 0, (cudaStream_t)stream>>>(
+      nullptr, 0, p->r, p->r_pad, p->m, 0, Ft, ld, 0, 0, none, nullptr, 0.f, nullptr, 0, nullptr, nullptr, 0, p->rowp_h[0], p->rowp_l[0]);
+  NNFAC_LAUNCH_CHECK(p->ctx);
+  return NNFAC_OK;
+}
+
+// Multiplicative update of factor 0 of a one-sided plan or view (the NTF factor of the plan's mode) from the partials of the last
+// MU pass over side 0: F_out = max(F_in * num / den[k], floor) after nnfac_nmf_plan_fused(mode 1) with `den` = r floats (the
+// column sums of the Khatri-Rao operand), or F_out = max(F_in * (num / den)^gamma, floor) after nnfac_nmf_plan_fused_beta with
+// `den_partial` its denominator partials; exactly one of the two.  F_out is installed as the row planes of factor 0 only.
+int nnfac_nmf_plan_mu_finish_rows(nnfac_nmf_plan* p, const float* F_in, int64_t ld_in, const float* den, const float* den_partial,
+                                  double gamma, double floor_value, float* F_out, int64_t ld_out, void* stream) {
+  NNFAC_ARG(p && F_in && F_out && (den == nullptr) != (den_partial == nullptr), "nnfac_nmf_plan_mu_finish_rows: bad argument");
+  NNFAC_ARG(ld_in >= p->m && ld_out >= p->m, "nnfac_nmf_plan_mu_finish_rows: leading dimension too small");
+  if (p->sides != 1 || !p->fused_ok || p->rk != 64 || p->planes != 2) {
+    nnfac_set_error("nnfac_nmf_plan_mu_finish_rows: covers one-sided plans and views of rank <= 64 with 2 planes");
+    return NNFAC_ERR_UNSUPPORTED;
+  }
+  const Side* s = &p->side[0];
+  const unsigned grid = (unsigned)ceil_div64(p->m, 32);
+  cudaStream_t st = (cudaStream_t)stream;
+  PeerG none;
+  memset(&none, 0, sizeof(none));
+  if (den)
+    factor_finish_kernel<true, 64, false, 2, false, false><<<grid, 256, 0, st>>>(p->partial, s->cp.splits, p->r, p->r_pad, p->m,
+        s->cp.ld_partial, F_in, ld_in, 0, 0, none, den, (float)floor_value, F_out, ld_out, nullptr, nullptr, 0, p->rowp_h[0], p->rowp_l[0]);
+  else
+    factor_finish_kernel<true, 64, false, 2, true, false><<<grid, 256, 0, st>>>(p->partial, s->cp.splits, p->r, p->r_pad, p->m,
+        s->cp.ld_partial, F_in, ld_in, 0, 0, none, den_partial, (float)floor_value, F_out, ld_out, nullptr, nullptr, 0, p->rowp_h[0],
+        p->rowp_l[0], nullptr, nullptr, (float)gamma);
   NNFAC_LAUNCH_CHECK(p->ctx);
   return NNFAC_OK;
 }

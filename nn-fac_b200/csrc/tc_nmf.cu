@@ -532,6 +532,10 @@ static int plan_build(nnfac_ctx* ctx, int64_t m, int64_t n, int r, int sides, in
       if (!rc) rc = make_map(&s->map_xm, s->xm, s->R, s->C, s->ld, TILE_ROWS);
       if (!rc) rc = make_map(&s->map_fm, s->fm, p->r_pad, s->C, s->ld, p->r_pad);
     }
+    if (i == 0 && sides == 1 && planes == 2 && p->rk == 64) {
+      if (!rc) rc = make_map(&s->map_kh, s->fh, p->r_pad, s->C, s->ld, 64);
+      if (!rc) rc = make_map(&s->map_kl, s->fl, p->r_pad, s->C, s->ld, 64);
+    }
     if (rc) { nnfac_nmf_plan_destroy(p); return rc; }
     cudaError_t e = cross_prepare(s, p->r_pad, planes);
     if (e != cudaSuccess) { nnfac_set_error("cudaFuncSetAttribute(smem=%zu): %s", s->smem, cudaGetErrorString(e)); nnfac_nmf_plan_destroy(p); return NNFAC_ERR_CUDA; }
@@ -613,8 +617,9 @@ int nnfac_nmf_plan_create_planes(nnfac_ctx* ctx, int64_t m, int64_t n, int r, in
 // unfolding of the middle axis (ntf.py:309-311 makes a COPY of the tensor for it; here it is a TMA map over the same planes):
 //   right == 1 (last mode):   the planes read as [left x I] hold the unfolding transposed -> MN-major operand (amode 1)
 //   otherwise (middle modes): 3-D map {right, I, left}, contraction index c = l * right + rr (amode 2; right % 64 == 0)
-// A view supports nnfac_nmf_plan_set_krao / _cross(which = 0) / _reduce / _info; its workspace holds only the factor planes
-// and the split-K partials.
+// A view supports nnfac_nmf_plan_set_krao / _cross(which = 0) / _reduce / _info; its workspace holds the factor planes and the
+// split-K partials, and at rank <= 64 also the row planes of factor 0 [I x 64] and the cost partials of the MU passes
+// (nnfac_nmf_plan_set_factor_rows / _fused(mode 1) / _fused_beta / _mu_finish_rows).
 static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, int64_t I, int64_t right, int r, void* buffer,
                       size_t buffer_bytes, cudaStream_t st, nnfac_nmf_plan** out, size_t* bytes_out) {
   NNFAC_ARG(ctx && base && left >= 1 && I >= 1 && right >= 1 && r > 0 && r <= 128, "nnfac_nmf_plan_view: bad argument");
@@ -631,7 +636,7 @@ static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, 
   p->ctx = ctx; p->base = base; p->m = I; p->n = left * right; p->r = r; p->sides = 1; p->planes = 2;
   p->r_pad = (int)round_up(r, 16);
   p->rk = p->r_pad <= 64 ? 64 : 128;
-  p->fused_ok = 0;
+  p->fused_ok = p->rk == 64;
   Side* s = &p->side[0];
   s->R = I; s->C = left * right; s->ld = round_up(s->C, 64);
   choose_partition(ctx->sm_count, s->R, s->C, p->r_pad, 2, s);
@@ -643,6 +648,8 @@ static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, 
   const size_t o_fh = take(fb), o_fl = take(fb);
   const size_t partial_bytes = (size_t)s->cp.splits * p->r_pad * s->cp.ld_partial * sizeof(float);
   const size_t o_partial = take(partial_bytes);
+  const size_t rb = p->fused_ok ? (size_t)I * p->rk * sizeof(bf16) : 0;
+  const size_t o_rh = take(rb), o_rl = take(rb), o_cost = take(p->fused_ok ? sizeof(double) * 1024 : 0);
   if (bytes_out) *bytes_out = off;
   if (!out) { free(p); return NNFAC_OK; }
   if (!buffer || buffer_bytes < off || ((uintptr_t)buffer & 255)) {
@@ -657,11 +664,23 @@ static int view_build(nnfac_ctx* ctx, const nnfac_nmf_plan* base, int64_t left, 
   p->partial = (float*)(mem + o_partial); p->partial_bytes = partial_bytes;
   cudaMemsetAsync(s->fh, 0, fb, st);
   cudaMemsetAsync(s->fl, 0, fb, st);
-  int rc;
-  if (right == 1) {           // planes as [left x I]: box = 64 contraction rows x 64 output rows
+  int rc = NNFAC_OK;
+  if (p->fused_ok) {
+    p->rowp_h[0] = (bf16*)(mem + o_rh); p->rowp_l[0] = (bf16*)(mem + o_rl);
+    cudaMemsetAsync(p->rowp_h[0], 0, rb, st);
+    cudaMemsetAsync(p->rowp_l[0], 0, rb, st);
+    p->cost_part = (double*)(mem + o_cost);
+    cudaMemsetAsync(p->cost_part, 0, sizeof(double) * 1024, st);
+    p->sums = base->sums;     // sum of X: the same tensor
+    rc = make_map(&p->map_row_a_h[0], p->rowp_h[0], I, p->rk, p->rk, TILE_ROWS);
+    if (!rc) rc = make_map(&p->map_row_a_l[0], p->rowp_l[0], I, p->rk, p->rk, TILE_ROWS);
+    if (!rc) rc = make_map(&s->map_kh, s->fh, p->r_pad, s->C, s->ld, 64);
+    if (!rc) rc = make_map(&s->map_kl, s->fl, p->r_pad, s->C, s->ld, 64);
+  }
+  if (!rc && right == 1) {           // planes as [left x I]: box = 64 contraction rows x 64 output rows
     rc = make_map(&s->map_xh, s->xh, left, I, I, 64);
     if (!rc) rc = make_map(&s->map_xl, s->xl, left, I, I, 64);
-  } else {
+  } else if (!rc) {
     rc = make_map_3d(&s->map_xh, s->xh, right, I, left, right, I * right, TILE_ROWS);
     if (!rc) rc = make_map_3d(&s->map_xl, s->xl, right, I, left, right, I * right, TILE_ROWS);
   }

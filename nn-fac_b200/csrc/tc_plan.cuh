@@ -100,6 +100,8 @@ struct Side {           // one orientation of X
   bf16 *fh, *fl;        // factor planes [r_pad x ld]
   bf16 *xm, *fm;        // 3-plane plans: the middle planes (x = xh + xm + xl); NULL otherwise
   CUtensorMap map_xh, map_xl, map_fh, map_fl, map_xm, map_fm;
+  CUtensorMap map_kh, map_kl;   // side 0 of a one-sided plan or view of rank <= 64: fh / fl in 64 x 64 boxes (Khatri-Rao operand of
+                                // the NTF MU pass; ranks beyond r_pad read as zeros)
   CrossParams cp;
   int grid;
   size_t smem;

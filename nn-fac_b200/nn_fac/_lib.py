@@ -93,6 +93,8 @@ SIGNATURES = {
     "nnfac_nmf_plan_fused_beta_bytes": [_P, _c.POINTER(_c.c_size_t)],
     "nnfac_nmf_plan_fused_beta": [_P, _INT, _DBL, _INT, _P, _P, _P],
     "nnfac_nmf_plan_mu_finish_beta": [_P, _INT, _P, _I64, _P, _DBL, _DBL, _P, _I64, _P],
+    "nnfac_nmf_plan_set_factor_rows": [_P, _P, _I64, _P],
+    "nnfac_nmf_plan_mu_finish_rows": [_P, _P, _I64, _P, _P, _DBL, _DBL, _P, _I64, _P],
     "nnfac_nmf_plan_info": [_P, _INT, _c.POINTER(_INT), _c.POINTER(_INT), _c.POINTER(_INT), _c.POINTER(_INT),
                             _c.POINTER(_INT)],
 }

@@ -497,6 +497,20 @@ class NMFPlan:
                                                      float(floor), L.ptr(out), out.stride(0), L.stream_ptr()))
         return out
 
+    def set_factor_rows(self, Ft):
+        """Factor 0 (U^T, r x m) of a one-sided plan or view, installed as its row planes only (the operand of the MU pass)."""
+        L.check(_lib().nnfac_nmf_plan_set_factor_rows(self.handle, L.ptr(Ft), Ft.stride(0), L.stream_ptr()))
+
+    def mu_finish_rows(self, F, floor, den=None, gamma=1.0):
+        """Update of factor 0 (rank-major, r x m) of a one-sided plan or view from its last MU pass over side 0: after
+        fused(0, 1, keep_partials=True) pass `den` (the r column sums of the Khatri-Rao operand), after fused_beta(0, beta) leave it
+        None (the denominator partials of that pass, exponent `gamma`).  The result is installed as the row planes of factor 0."""
+        out = torch.empty_like(F)
+        L.check(_lib().nnfac_nmf_plan_mu_finish_rows(self.handle, L.ptr(F), F.stride(0), L.ptr(den),
+                                                     L.ptr(self._den if den is None else None), float(gamma), float(floor),
+                                                     L.ptr(out), out.stride(0), L.stream_ptr()))
+        return out
+
     def enable_f32(self):
         """fp32 copies of X / X^T for the beta = 1 fused pass (made from the planes on first use)."""
         import ctypes

@@ -90,7 +90,10 @@ class DeviceNTF:
                 torch.cuda.empty_cache()
 
     def direct_cost(self, update_rule, fixed_modes=()):
-        """fp32 HALS on a 3-way tensor with plans: the objective is the DIRECT residual ||T - [[A, B, C]]||^2 of the state an
+        """fp32 on a 3-way tensor with plans (HALS; MU at rank <= 64, see _mu_pass): the objective is formed on chip by a fused
+        pass over the tensor, for the state the iteration started from.
+
+        HALS: the objective is the DIRECT residual ||T - [[A, B, C]]||^2 of the state an
         iteration starts from, formed on chip by the fused pass that also yields the first MTTKRP of that iteration (the model
         tile never reaches HBM) -- instead of the reference's ||T||^2 - 2 <F, rhs> + ||F krao^T||^2 (ntf.py:470), which
         subtracts numbers of the size of ||T||^2 and in fp32 keeps an error of ~7e-7 ||T||^2 (the truncation of the tensor
@@ -99,8 +102,11 @@ class DeviceNTF:
         plan of mode 0, which always is one: one extra pass over the tensor per iteration, its MTTKRP unused
         (_residual_mode)."""
         free = [m for m in range(len(self.shape)) if m not in fixed_modes]
-        return (update_rule == "hals" and self.plans is not None and self.T.dim() == 3 and self.T.dtype == torch.float32
-                and len(free) > 0 and os.environ.get("NNFAC_NTF_DIRECT", "1") != "0")
+        if self.plans is None or self.T.dim() != 3 or self.T.dtype != torch.float32 or not free:
+            return False
+        if update_rule == "mu":
+            return int(self.factors[0].shape[1]) <= 64
+        return update_rule == "hals" and os.environ.get("NNFAC_NTF_DIRECT", "1") != "0"
 
     def _residual_mode(self, fixed_modes):
         """The mode whose fused pass forms the direct residual (the fused pass needs a full plan, a view has no row planes):
@@ -116,9 +122,43 @@ class DeviceNTF:
         plan.set_krao_rows(self.factors_t[others[0]], self.factors_t[others[1]])
         return plan.fused(0, 0)
 
-    def cost_terms_now(self, sparsity, fixed_modes=()):
-        """Device vector [direct residual of the current state, l1 norms for the sparsity terms...] (closing pass of a run)."""
-        _, res = self._residual_pass(self._residual_mode(fixed_modes))
+    def _mu_pass(self, mode, beta, want_cost):
+        """MU pass of the tensor core over unfold(T, mode) for the CURRENT factors (3-way tensor, rank <= 64, beta != 2): the model
+        tile F_mode krao^T is formed on chip, never in HBM, and X is read once from the planes (views: in place).  The numerator
+        partials (beta != 1: the denominator partials too) stay in the plan for _mu_finish; returns d_beta(T | [[F]]) as a device
+        scalar when want_cost."""
+        others = [i for i in range(3) if i != mode]
+        plan = self.plans[mode]
+        plan.set_factor_rows(self.factors_t[mode])
+        plan.set_krao(self.factors_t[others[0]], self.factors_t[others[1]])
+        if beta == 1:
+            return plan.fused(0, 1, want_cost=want_cost, keep_partials=True)[1]
+        return plan.fused_beta(0, beta, want_cost=want_cost)
+
+    def _mu_finish(self, mode, beta):
+        """The update of factor `mode` from its _mu_pass (mu.py:84-97); returns it rank-major (r x I)."""
+        from nn_fac.utils.beta_divergence import gamma_beta
+        plan = self.plans[mode]
+        if beta == 1:
+            # column sums of krao = colsum(F_a) * colsum(F_b)
+            a, b = (self.factors_t[i] for i in range(3) if i != mode)
+            den = ops.hadamard_(ops.row_sums(a), ops.row_sums(b))
+            return plan.mu_finish_rows(self.factors_t[mode], mu.epsilon, den=den)
+        return plan.mu_finish_rows(self.factors_t[mode], mu.epsilon, gamma=gamma_beta(beta))
+
+    def _mu_cost_mode(self, beta, fixed_modes):
+        """The mode whose pass forms the objective of an MU iteration: the first free mode (beta = 2: as for HALS)."""
+        if beta == 2:
+            return self._residual_mode(fixed_modes)
+        return [m for m in range(len(self.shape)) if m not in fixed_modes][0]
+
+    def cost_terms_now(self, sparsity, fixed_modes=(), update_rule="hals", beta=2):
+        """Device vector [direct residual / beta-divergence of the current state, l1 norms for the sparsity terms...] (closing pass
+        of a run)."""
+        if update_rule == "mu" and beta != 2:
+            res = self._mu_pass(self._mu_cost_mode(beta, fixed_modes), beta, True)
+        else:
+            _, res = self._residual_pass(self._residual_mode(fixed_modes))
         terms = [res]
         for idx, sp in enumerate(sparsity):
             if sp:
@@ -188,10 +228,11 @@ class DeviceNTF:
         rhs = krao = cross = None
         mode = None
         direct = self.direct_cost(update_rule, fixed_modes)
+        mu_fused = direct and update_rule == "mu"          # MU on the tensor core: no tensor-sized model (_mu_pass)
         lag_terms = res_mode = None
         if direct:
             lag_terms = []
-            res_mode = self._residual_mode(fixed_modes)
+            res_mode = self._mu_cost_mode(beta, fixed_modes) if mu_fused else self._residual_mode(fixed_modes)
             if res_mode not in modes:
                 # mode 0 is fixed and the first free mode a view: a pass over unfold(T, 0) just for the residual
                 lag_terms.append(self._residual_pass(res_mode)[1])
@@ -201,7 +242,7 @@ class DeviceNTF:
         for mode in modes:
             others = [i for i in range(len(self.factors)) if i != mode]
             fused_krao = update_rule == "hals" and self.plans is not None and len(others) == 2
-            krao = None if fused_krao else self.khatri_rao(mode)
+            krao = None if fused_krao or mu_fused else self.khatri_rao(mode)
             if update_rule == "hals":
                 cross = None
                 for i in others:
@@ -230,6 +271,29 @@ class DeviceNTF:
                 self.factors_t[mode] = Ft
                 self.factors[mode] = ops.transpose(Ft)
                 self._gram_ok[mode] = False
+            elif mu_fused:
+                if beta == 2:
+                    # numerator: the MTTKRP (ntf.py:449); denominator: F krao^T krao = F (Hadamard product of the other Grams)
+                    cross = None
+                    for i in others:
+                        gram = self._gram(i)
+                        cross = gram.clone() if cross is None else ops.hadamard_(cross, gram)
+                    if mode == res_mode:
+                        rhs_t, res_in = self._residual_pass(mode)
+                        lag_terms.insert(0, res_in)
+                    else:
+                        self.plans[mode].set_krao(self.factors_t[others[0]], self.factors_t[others[1]])
+                        rhs_t = self.plans[mode].cross(0, None)
+                    Ft = self.factors_t[mode]
+                    Ft = ops.mu_apply(Ft, rhs_t, den_mat=ops.matmul(cross, Ft), floor=mu.epsilon)
+                else:
+                    cost = self._mu_pass(mode, beta, mode == res_mode)
+                    if mode == res_mode:
+                        lag_terms.insert(0, cost)
+                    Ft = self._mu_finish(mode, beta)
+                self.factors_t[mode] = Ft
+                self.factors[mode] = ops.transpose(Ft)
+                self._gram_ok[mode] = False
             else:
                 F = self.factors[mode]
                 K = self.reconstruct_unfolded(mode, krao)
@@ -255,10 +319,11 @@ class DeviceNTF:
         return torch.cat([t.reshape(1).to(torch.float64) for t in terms])
 
     @staticmethod
-    def finish_cost(terms_host, norm_tensor, update_rule, sparsity, direct=False):
+    def finish_cost(terms_host, norm_tensor, update_rule, sparsity, direct=False, beta=2):
         """ntf.py:463-475 from the device terms of step_async (host float64 arithmetic, as in the reference)."""
         if direct:
-            rec_error = terms_host[0]
+            # MU, beta = 2: the beta-divergence of ntf.py:473 is half the squared residual
+            rec_error = terms_host[0] / 2 if update_rule == "mu" and beta == 2 else terms_host[0]
             rest = terms_host[1:]
         elif update_rule == "hals":
             rec_error = norm_tensor ** 2 - 2 * terms_host[0] + terms_host[1]
@@ -275,8 +340,8 @@ class DeviceNTF:
         terms = self.step_async(rank, norm_tensor, update_rule, beta, sparsity, fixed_modes, normalize)
         direct = self.direct_cost(update_rule, fixed_modes)
         if direct:                                      # the terms of the step describe the state it started from
-            terms = self.cost_terms_now(sparsity, fixed_modes)
-        return self.finish_cost(terms.cpu().numpy(), norm_tensor, update_rule, sparsity, direct)
+            terms = self.cost_terms_now(sparsity, fixed_modes, update_rule, beta)
+        return self.finish_cost(terms.cpu().numpy(), norm_tensor, update_rule, sparsity, direct, beta)
 
     def _mu_factor(self, F, krao, K, mode, beta):
         """mu_betadivmin(F, krao.T, unfold(T, mode), beta) with the unfolding kept implicit."""
@@ -385,7 +450,7 @@ def compute_ntf(tensor_in, rank, factors_in, n_iter_max=100, tol=1e-8,
                     history = (history + [(list(state.factors), list(state.factors_t))])[-2:]
                     terms = step()
             else:
-                terms = state.cost_terms_now(sparsity_coefficients, fixed_modes)
+                terms = state.cost_terms_now(sparsity_coefficients, fixed_modes, update_rule, beta)
             buf = hosts[k & 1]
             buf[:terms.numel()].copy_(terms, non_blocking=True)
             ev = torch.cuda.Event()
@@ -398,7 +463,7 @@ def compute_ntf(tensor_in, rank, factors_in, n_iter_max=100, tol=1e-8,
                 if s_idx == 0:
                     continue                           # objective of the initial factors: the reference never reports it
                 ev_s.synchronize()
-                cost = state.finish_cost(buf_s[:n_s].numpy().copy(), norm_tensor, update_rule, sparsity_coefficients, True)
+                cost = state.finish_cost(buf_s[:n_s].numpy().copy(), norm_tensor, update_rule, sparsity_coefficients, True, beta)
                 if record(cost) and s_idx < n_iter_max:
                     back = min(k + 1, n_iter_max) - s_idx  # iterations launched beyond state s_idx: 2, or 1 in the closing round
                     if graphed is not None:
