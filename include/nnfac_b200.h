@@ -297,8 +297,17 @@ int nnfac_nmf_plan_set_krao(nnfac_nmf_plan* plan, const float* At, int64_t lda, 
  * ||unfold(T, mode) - F krao^T||_F^2 of the CP model (instead of the cancelling ntf.py:470) in one pass over the tensor. */
 int nnfac_nmf_plan_set_krao_rows(nnfac_nmf_plan* plan, const float* At, int64_t lda, int64_t I, const float* Bt, int64_t ldb,
                                  int64_t J, void* stream);
+/* Operand of an NTD unfolding: the r x (left*right) factor V[q][l*right + rr] = B[l][q][rr] of the C-order fp32 array B
+ * (left, r, right), r == the plan's rank, left*right == n, written into the operand planes that nnfac_nmf_plan_cross(which = 0,
+ * F = NULL) and, on one-sided plans and views, the MU passes (fused mode 1, fused_beta) read -- the planes set_krao writes, the
+ * same bits as cross(0, F) with F the unfolded copy.  NNFAC_ERR_UNSUPPORTED for 3-plane plans, NNFAC_ERR_ARG for extents that do
+ * not match the plan; nothing is written then. */
+int nnfac_nmf_plan_set_operand(nnfac_nmf_plan* plan, const float* B, int64_t left, int r, int64_t right, void* stream);
 /* out (r x R of `side`) = sum of the split-K partials of the last X pass over `side` run with out == NULL. */
 int nnfac_nmf_plan_reduce(nnfac_nmf_plan* plan, int side, float* out, int64_t ld_out, void* stream);
+/* The same sum, in the same order, of a caller-owned partial set laid out as the plan's own (e.g. the den_partial buffer of
+ * nnfac_nmf_plan_fused_beta). */
+int nnfac_nmf_plan_reduce_partials(nnfac_nmf_plan* plan, int side, const float* partial, float* out, int64_t ld_out, void* stream);
 /* The same sum in the send layout of a reduce-scatter over `slabs` ranks (column-sharded U side, nn_fac/_fast.py):
  * out = [slabs][r][chunk + tail_cols]; column `row` of the result goes to out[row / chunk][k][row % chunk], and the small
  * matrix `tail` (r x tail_cols, the partial Gram; NULL with tail_cols = 0) is copied behind every chunk. */

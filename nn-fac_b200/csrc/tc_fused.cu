@@ -1211,6 +1211,17 @@ int nnfac_nmf_plan_reduce(nnfac_nmf_plan* p, int side, float* out, int64_t ld_ou
   return NNFAC_OK;
 }
 
+// The same sum of a partial set the caller owns, laid out as the plan's own for `side` ([splits][r_pad][ld_partial]): the
+// denominator partials nnfac_nmf_plan_fused_beta leaves in den_partial, summed as a matrix.
+int nnfac_nmf_plan_reduce_partials(nnfac_nmf_plan* p, int side, const float* partial, float* out, int64_t ld_out, void* stream) {
+  NNFAC_ARG(p && partial && out && (side == 0 || side == 1), "nnfac_nmf_plan_reduce_partials: bad argument");
+  Side* s = &p->side[side];
+  NNFAC_ARG(ld_out >= s->R, "nnfac_nmf_plan_reduce_partials: leading dimension too small");
+  nnfac_reduce_partials(partial, s->cp.splits, p->r, p->r_pad, s->R, s->cp.ld_partial, out, ld_out, p->ctx->sm_count, (cudaStream_t)stream);
+  NNFAC_LAUNCH_CHECK(p->ctx);
+  return NNFAC_OK;
+}
+
 // The sum of nnfac_nmf_plan_reduce, written as the send buffer of a reduce-scatter over `slabs` ranks (see the kernel in
 // tc_nmf.cu): out = [slabs][r][chunk + tail_cols], `tail` (r x tail_cols, may be NULL with tail_cols = 0) copied behind
 // every chunk.  Replaces a reduction + a permuting copy + a broadcast copy by one kernel.

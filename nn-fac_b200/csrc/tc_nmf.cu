@@ -36,6 +36,22 @@ __global__ void split_planes_kernel(const float* __restrict__ in, int64_t ld_in,
   }
 }
 
+// The factor operand read from a strided tensor: B is the C-order array (left, r, right) and plane row q = blockIdx.y holds
+// V[q][l * right + rr] = B[l][q][rr] (right > 1: runs of `right` contiguous values; the last mode, right == 1, takes the tiled
+// transpose below).  The same split as split_planes_kernel<2>, so that for the same values both write the same bits.  The plans
+// keep every extent below 2^31, so the column index is split with 32-bit arithmetic.
+__global__ void split_planes_strided_kernel(const float* __restrict__ B, int cols, int r, int right, bf16* __restrict__ hi,
+                                            bf16* __restrict__ lo, int64_t ld_out) {
+  const int q = blockIdx.y;
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < cols; c += gridDim.x * blockDim.x) {
+    const int l = c / right, rr = c - l * right;
+    bf16 h, l16;
+    tc::split_bf16(B[((int64_t)l * r + q) * right + rr], h, l16);
+    hi[q * ld_out + c] = h;
+    lo[q * ld_out + c] = l16;
+  }
+}
+
 // out planes hold in^T: hiT/loT (/midT) are [cols x rows] with leading dimension ld_out
 template <int PLANES>
 __global__ void split_planes_transposed_kernel(const float* __restrict__ in, int64_t ld_in, int64_t rows, int64_t cols,
@@ -803,6 +819,32 @@ int nnfac_nmf_plan_set_krao(nnfac_nmf_plan* p, const float* At, int64_t lda, int
   const int64_t total = I * J;
   const int grid = (int)(ceil_div64(total, 256) < (int64_t)p->ctx->sm_count * 16 ? ceil_div64(total, 256) : (int64_t)p->ctx->sm_count * 16);
   krao_planes_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(At, lda, I, Bt, ldb, J, p->r, s->fh, s->fl, s->ld);
+  NNFAC_LAUNCH_CHECK(p->ctx);
+  return NNFAC_OK;
+}
+
+// Install the r x (left * right) factor V[q][l * right + rr] = B[l][q][rr] of a C-order fp32 array B (left, r, right) into the
+// K-major planes of side 0 that nnfac_nmf_plan_cross(which = 0, F = NULL) and, on one-sided plans and views, the MU passes read
+// (where nnfac_nmf_plan_set_krao writes): the operand of an NTD unfolding, B = G x_{j != n} F_j, without its unfolded copy.
+int nnfac_nmf_plan_set_operand(nnfac_nmf_plan* p, const float* B, int64_t left, int r, int64_t right, void* stream) {
+  NNFAC_ARG(p && B && left > 0 && r > 0 && right > 0, "nnfac_nmf_plan_set_operand: bad argument");
+  NNFAC_ARG(p->sides & 1, "nnfac_nmf_plan_set_operand: this plan keeps no planes of side 0");
+  if (p->planes != 2) { nnfac_set_error("nnfac_nmf_plan_set_operand: writes two planes, the plan has %d", p->planes); return NNFAC_ERR_UNSUPPORTED; }
+  Side* s = &p->side[0];
+  NNFAC_ARG(r == p->r && left * right == s->C, "nnfac_nmf_plan_set_operand: (%lld, %d, %lld) is not an operand of this %d x %lld plan",
+            (long long)left, r, (long long)right, p->r, (long long)s->C);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (right == 1) {     // V = B^T, B read as [left x r]: grid.y is limited to 65535 blocks of 32 rows, walk the rows in slabs
+    for (int64_t r0 = 0; r0 < left; r0 += 65535ll * 32) {
+      const int64_t nr = left - r0 < 65535ll * 32 ? left - r0 : 65535ll * 32;
+      dim3 g((unsigned)ceil_div64(r, 32), (unsigned)ceil_div64(nr, 32)), b(32, 8);
+      split_planes_transposed_kernel<2><<<g, b, 0, st>>>(B + r0 * r, r, nr, r, s->fh + r0, s->fl + r0, s->ld, nullptr);
+      NNFAC_LAUNCH_CHECK(p->ctx);
+    }
+    return NNFAC_OK;
+  }
+  const int64_t bx = ceil_div64(s->C, 256) < 1024 ? ceil_div64(s->C, 256) : 1024;
+  split_planes_strided_kernel<<<dim3((unsigned)bx, (unsigned)r), 256, 0, st>>>(B, (int)s->C, r, (int)right, s->fh, s->fl, s->ld);
   NNFAC_LAUNCH_CHECK(p->ctx);
   return NNFAC_OK;
 }

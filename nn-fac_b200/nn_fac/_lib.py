@@ -83,7 +83,9 @@ SIGNATURES = {
     "nnfac_nmf_plan_cross": [_P, _INT, _P, _I64, _P, _I64, _P],
     "nnfac_nmf_plan_set_factor": [_P, _INT, _P, _I64, _P],
     "nnfac_nmf_plan_set_factor_gathered": [_P, _INT, _P, _I64, _P, _I64, _P],
+    "nnfac_nmf_plan_set_operand": [_P, _P, _I64, _INT, _I64, _P],
     "nnfac_nmf_plan_reduce": [_P, _INT, _P, _I64, _P],
+    "nnfac_nmf_plan_reduce_partials": [_P, _INT, _P, _P, _I64, _P],
     "nnfac_nmf_plan_reduce_chunked": [_P, _INT, _P, _I64, _INT, _P, _I64, _INT, _P],
     "nnfac_nmf_plan_set_krao": [_P, _P, _I64, _I64, _P, _I64, _I64, _P],
     "nnfac_nmf_plan_set_krao_rows": [_P, _P, _I64, _I64, _P, _I64, _I64, _P],

@@ -380,6 +380,20 @@ class NMFPlan:
         L.check(_lib().nnfac_nmf_plan_reduce(self.handle, side, L.ptr(out), out.stride(0), L.stream_ptr()))
         return out
 
+    def reduce_den(self, side, out=None):
+        """Sum of the denominator partials the last fused_beta(side) left in this object's buffer (r x rows of that side)."""
+        R = self.m if side == 0 else self.n
+        if out is None:
+            out = torch.empty((self.r, R), dtype=torch.float32, device=self.device)
+        L.check(_lib().nnfac_nmf_plan_reduce_partials(self.handle, side, L.ptr(self._den), L.ptr(out), out.stride(0), L.stream_ptr()))
+        return out
+
+    def set_operand(self, B, left, right):
+        """B: contiguous fp32 tensor read as (left, r, right); installs V[q, l * right + rr] = B[l, q, rr] as the operand of
+        cross(0, None) and of the MU passes of a one-sided plan or view (an NTD unfolding without its unfolded copy)."""
+        assert B.is_contiguous() and B.dtype == torch.float32
+        L.check(_lib().nnfac_nmf_plan_set_operand(self.handle, L.ptr(B), left, B.numel() // (left * right), right, L.stream_ptr()))
+
     def reduce_chunked(self, side, slabs, chunk, tail=None):
         """The sum of reduce(side) as the send buffer of a reduce-scatter over `slabs` ranks: [slabs][r][chunk + t] with the small
         matrix `tail` (r x t) copied behind every chunk."""

@@ -72,20 +72,41 @@ class DeviceNTD:
         self.core = L.to_device(core, dtype, device)
         self.factors = [L.to_device(f, dtype, device) for f in factors]
         self.stats = torch.zeros(4, dtype=torch.float64, device=self.T.device)
-        # fp32, every rank <= 64: the beta = 1 factor update of a mode is the NMF update of U for X = unfold(T, mode),
-        # V = unfold(G x_{j != mode} F_j, mode), i.e. one fused tcgen05 pass over the planes of that unfolding
-        # (model tile, ratio and contraction on chip; nothing of the size of the tensor is written).
-        self.plans = None
+        # fp32, every rank <= 64: every pass over the tensor runs on tcgen05 over ONE copy of it as bf16 hi/lo planes (4 bytes per
+        # element).  The factor update of mode n is the update of U for X = unfold(T, n), V = unfold(G x_{j != n} F_j, n) -- one
+        # fused pass (beta = 2: one cross product), model tile and ratios on chip -- on plans[n]: the plan that owns the planes
+        # for mode 0, a view of them (NMFPlan.view) for the other modes, or, where an unfolding cannot be addressed in place, a
+        # one-sided plan on a copy of it.  core_plan reads the same planes as unfold(T, 0)^T (rows: the columns of unfold(T, 0),
+        # contraction over I_0): every contraction of the tensor over mode 0 -- the core update's, HALS's T x_0 F_0^T -- runs
+        # there.  Not enough memory for the plans: the strided CUDA-core route (self.plans None), as NNFAC_NTD_TC=0 selects.
+        self.plans = self.core_plan = None
         self._m0_ready = False                                              # see step_mu_async
         self._pg, self._pg_calls = None, 0                                  # see _core_loop_graphed
         self._m0_den = torch.empty(int(self.factors[0].shape[1]), dtype=dtype, device=self.T.device)
-        if (dtype == torch.float32 and max(int(f.shape[1]) for f in self.factors) <= 64
+        self._m0_num = None
+        if (dtype == torch.float32 and self.T.dim() >= 2 and max(int(f.shape[1]) for f in self.factors) <= 64
                 and os.environ.get("NNFAC_NTD_TC", "1") != "0"):
-            self.plans = []
-            for mode in range(self.T.dim()):
-                Xm = self.T.movedim(mode, 0).reshape(self.T.shape[mode], -1).contiguous()
-                self.plans.append(ops.NMFPlan(Xm).bind_rank(int(self.factors[mode].shape[1])))
-                del Xm
+            try:
+                self._build_plans()
+            except torch.cuda.OutOfMemoryError:
+                self.plans = self.core_plan = None
+                torch.cuda.empty_cache()
+
+    def _build_plans(self):
+        shape = list(self.T.shape)
+        ranks = [int(f.shape[1]) for f in self.factors]
+        base = ops.NMFPlan(self.T.reshape(shape[0], -1)).bind_rank(ranks[0], sides=1)
+        plans = [base]
+        for mode in range(1, len(shape)):
+            left, I, right = ops._split(shape, mode)
+            view = base.view(left, I, right, ranks[mode])
+            if view is None:
+                view = ops.NMFPlan(self._unfold(self.T, mode)).bind_rank(ranks[mode], sides=1)
+            plans.append(view)
+        core = base.view(shape[0], base.n, 1, ranks[0])                    # the last-mode view of (I_0, prod of the others)
+        if core is None:
+            core = ops.NMFPlan(ops.transpose(self.T.reshape(shape[0], -1))).bind_rank(ranks[0], sides=1)
+        self.plans, self.core_plan = plans, core
 
     def invalidate(self):
         """Core / factors were replaced from outside: nothing left in the plans refers to them."""
@@ -101,14 +122,23 @@ class DeviceNTD:
         """mu_betadivmin(F, unfold(G x_{j != mode} F_j, mode), unfold(T, mode), beta), ntd.py:672."""
         F = self.factors[mode]
         B = ops.multi_mode_dot(self.core, self.factors, skip=mode)          # shape of T except R_mode along `mode`
-        if self.plans is not None and beta == 1:
+        if self.plans is not None:
+            # B_(n) = unfold(B, mode) is installed straight from B: the contraction order of the plan of `mode` (view or copy)
+            # is the column order of unfold(T, mode), which is that of unfold(B, mode)
             plan = self.plans[mode]
-            Vm = B.movedim(mode, 0).reshape(B.shape[mode], -1).contiguous()  # unfold(B, mode): r_mode x rest
+            left, _, right = ops._split(list(self.T.shape), mode)
             Ft = ops.transpose(F)
-            plan.set_factor(0, Ft)
-            plan.set_factor(1, Vm)
-            plan.fused(0, 1, want_cost=False, keep_partials=True)           # (X / (F Vm)) Vm^T, mu.py:82-85
-            return ops.transpose(plan.mu_finish(0, Ft, ops.row_sums(Vm), mu.epsilon))   # mu.py:86-88
+            plan.set_operand(B, left, right)
+            if beta == 2:
+                return self._mu_finish(mode, beta, Ft, plan.cross(0, None))
+            plan.set_factor_rows(Ft)
+            if beta == 1:
+                plan.fused(0, 1, want_cost=False, keep_partials=True)       # (X / (F B_(n))) B_(n)^T, mu.py:82-85
+                # row sums of B_(n) (mu.py:86) = G x_{j != n} (column sums of F_j): B_n is not read again
+                sums = [None if j == mode else ops.row_sums(ops.transpose(f)).reshape(1, -1) for j, f in enumerate(self.factors)]
+                return self._mu_finish(mode, beta, Ft, ops.multi_mode_dot(self.core, sums, skip=mode).reshape(-1))
+            plan.fused_beta(0, beta, want_cost=False)
+            return self._mu_finish(mode, beta, Ft)
         K = ops.mode_dot(B, F, mode)                                        # = F @ unfold(B, mode), folded (mu.py:82)
         g = gamma_beta(beta)
         if beta == 2:
@@ -124,26 +154,43 @@ class DeviceNTD:
             return ops.mu_apply(F, num, den_vec=den_vec, vec_per_row=False, gamma=g, floor=mu.epsilon)
         return ops.mu_apply(F, num, den_mat=ops.unfold_times(Q, B, mode), gamma=g, floor=mu.epsilon)
 
+    def _mu_finish(self, mode, beta, Ft, extra=None):
+        """The update of factor `mode` (given as F^T) from the last pass over its plan, mu.py:84-97: beta = 2, `extra` is the
+        numerator B_(n) unfold(T, mode)^T and the denominator (B_(n) B_(n)^T) F^T; beta = 1, `extra` = the row sums of B_(n);
+        any other beta, both partial sets of the plan's fused_beta pass."""
+        if beta == 2:
+            return ops.transpose(ops.mu_apply(Ft, extra, den_mat=ops.matmul(self._bbt(mode), Ft), floor=mu.epsilon))
+        if beta == 1:
+            return ops.transpose(self.plans[mode].mu_finish_rows(Ft, mu.epsilon, den=extra))
+        return ops.transpose(self.plans[mode].mu_finish_rows(Ft, mu.epsilon, gamma=gamma_beta(beta)))
+
+    def _bbt(self, mode):
+        """B_(n) B_(n)^T = unfold(G x_{j != n} F_j^T F_j, n) unfold(G, n)^T (r_n x r_n), from the Grams: B_n is never read."""
+        grams = [None if j == mode else mu.gram(F) for j, F in enumerate(self.factors)]
+        return ops.matmul(self._unfold(ops.multi_mode_dot(self.core, grams, skip=mode), mode), self._unfold(self.core, mode).T)
+
     # ---- HALS factor updates + projected-gradient core update (ntd.py:436-645) ------------------------------
     @staticmethod
     def _unfold(t, mode):
         return t.movedim(mode, 0).reshape(t.shape[mode], -1).contiguous()
 
-    def _project_all_but(self, mode):
-        """T x_{j != mode} F_j^T (ntd.py:550).  With the tcgen05 plans (fp32, ranks <= 64) the first contraction -- the only
-        one that reads the whole tensor -- is the cross product F_j^T unfold(T, j) over the bf16 planes of that unfolding;
-        the remaining ones act on a tensor r_j / I_j times smaller."""
-        nm = self.T.dim()
-        if self.plans is None or nm < 2:
+    def _project_all_but(self, mode, P0=None):
+        """T x_{j != mode} F_j^T (ntd.py:550); mode None: every mode.  With the tcgen05 plans (fp32, ranks <= 64), for a mode
+        other than 0, the first contraction -- the only one that reads the whole tensor -- is T x_0 F_0^T = F_0^T unfold(T, 0),
+        one cross product on core_plan (P0 when the caller already has it: it depends on F_0 only); the remaining ones act on a
+        tensor r_0 / I_0 times smaller."""
+        if self.plans is None or mode == 0:
             return ops.multi_mode_dot(self.T, self.factors, skip=mode, transpose=True)
-        j = 0 if mode != 0 else 1
-        rest = [d for d in range(nm) if d != j]
-        P = self.plans[j].cross(1, ops.transpose(self.factors[j]))         # r_j x prod(rest), mode j in front
-        P = P.reshape([P.shape[0]] + [self.T.shape[d] for d in rest])
-        for pos, d in enumerate(rest):
+        P = P0 if P0 is not None else self._project_mode0()
+        for d in range(1, self.T.dim()):
             if d != mode:
-                P = ops.mode_dot(P, self.factors[d], pos + 1, transpose=True)
-        return P.movedim(0, j).contiguous()
+                P = ops.mode_dot(P, self.factors[d], d, transpose=True)
+        return P
+
+    def _project_mode0(self):
+        """T x_0 F_0^T on core_plan: r_0 x I_1 x ... """
+        P = self.core_plan.cross(0, ops.transpose(self.factors[0]))
+        return P.reshape([P.shape[0]] + list(self.T.shape[1:]))
 
     def step_hals_async(self, norm_tensor, sparsity, fixed_modes, normalize, mode_core_norm, delta=0.01):
         """One outer iteration of one_ntd_step (deterministic inner rule); returns the device vector of cost terms
@@ -151,7 +198,7 @@ class DeviceNTD:
         import nn_fac.update_rules.nnls as nnls
         nm = self.T.dim()
         modes = [m for m in range(nm) if m not in fixed_modes]
-        temp = elemprod = None
+        temp = elemprod = P0 = None                                          # P0: T x_0 F_0^T for the current F_0 (plans only)
         for mode in modes:
             elemprod = list(self.factors)                                    # ntd.py:534-537
             for i, f in enumerate(self.factors):
@@ -160,15 +207,26 @@ class DeviceNTD:
                     elemprod[i] = ops.gemm(f, (1, r_i), f, (r_i, 1), r_i, r_i, f.shape[0])
             core_u = self._unfold(self.core, mode)
             UtU = ops.matmul(self._unfold(ops.multi_mode_dot(self.core, elemprod, skip=mode), mode), core_u.T.contiguous())   # ntd.py:539-544
-            temp = self._project_all_but(mode)                                                                                # ntd.py:550
-            UtM = ops.matmul(core_u, self._unfold(temp, mode).T.contiguous())                                                 # ntd.py:555-557 (transposed)
+            if self.plans is not None and mode == 0:
+                # ntd.py:555-557 in another association: UtM = B_(0) unfold(T, 0)^T, B_0 = G x_{j>0} F_j, one cross product
+                B0 = ops.multi_mode_dot(self.core, self.factors, skip=0)
+                UtM = self.plans[0].cross(0, B0.reshape(B0.shape[0], -1))
+                temp = None
+            else:
+                if self.plans is not None and P0 is None:
+                    P0 = self._project_mode0()                              # one pass serves every mode >= 1 of the iteration
+                temp = self._project_all_but(mode, P0)                                                                        # ntd.py:550
+                UtM = ops.matmul(core_u, self._unfold(temp, mode).T.contiguous())                                             # ntd.py:555-557 (transposed)
             Ft = ops.transpose(self.factors[mode])
             nnls.hals_nnls_device(UtM, UtU, Ft, Ft.shape[0], maxiter=100, delta=delta, sparsity_coefficient=sparsity[mode],
                                   normalize=normalize[mode], nonzero=False, result=self.stats)   # ntd.py:571-573
             self.factors[mode] = ops.transpose(Ft)
         last = modes[-1]
         F_last = self.factors[last]
-        all_MtX = ops.mode_dot(temp, F_last, last, transpose=True)           # ntd.py:581
+        if temp is not None:
+            all_MtX = ops.mode_dot(temp, F_last, last, transpose=True)       # ntd.py:581
+        else:
+            all_MtX = self._project_all_but(None)                           # the last free mode was mode 0
         all_MtM = list(elemprod)                                             # ntd.py:582-583
         r_l = F_last.shape[1]
         all_MtM[last] = ops.gemm(F_last, (1, r_l), F_last, (r_l, 1), r_l, r_l, F_last.shape[0])
@@ -274,40 +332,51 @@ class DeviceNTD:
 
     def step_mu_async(self, beta, fixed_modes, normalize, mode_core_norm):
         """One outer iteration; returns the cost as a device scalar (no synchronisation)."""
-        tc = self.plans is not None and beta == 1
         for mode in [m for m in range(self.T.dim()) if m not in fixed_modes]:
-            if mode == 0 and tc and self._m0_ready:
+            if mode == 0 and self._m0_ready:
                 # the pass this update needs already ran: it is the cost pass that ended the previous iteration (same core,
-                # same factors), which left its numerator partials in the plan and the row sums of V in _m0_den
-                self.factors[0] = ops.transpose(self.plans[0].mu_finish(0, ops.transpose(self.factors[0]), self._m0_den,
-                                                                        mu.epsilon))            # mu.py:86-88
+                # same factors), which left what the update needs in the plan of mode 0, _m0_den or _m0_num
+                self.factors[0] = self._mu_finish(0, beta, ops.transpose(self.factors[0]), self._m0_num if beta == 2 else self._m0_den)
             else:
                 self.factors[mode] = self.factor_update(mode, beta)
         self._m0_ready = False
-        plan0 = self.plans[0] if (self.plans is not None and beta == 1) else None
-        self.core = mu.mu_tensorial_device(self.core, self.factors, self.T, beta, plan0)   # ntd.py:674
+        self.core = mu.mu_tensorial_device(self.core, self.factors, self.T, beta, self.core_plan)   # ntd.py:674
         if normalize[-1]:                                                    # ntd.py:676-681
             moved = self.core.movedim(mode_core_norm, 0).contiguous()
             flat = moved.reshape(moved.shape[0], -1)
             ops.normalize_rows_(flat)
             self.core = moved.movedim(0, mode_core_norm).contiguous()
-        if self.plans is not None and beta == 1:
-            # beta_divergence(T, G x_n F_n, 1) without forming the reconstruction: it is the cost output of a fused pass
-            # over unfold(T, last) with U = F_last, V = unfold(G x_{j != last} F_j, last)
-            # (any mode's unfolding gives the same number; mode 0 is used because the same pass, with the same operands, is
-            # the first factor update of the NEXT iteration: its numerator partials stay in the plan for it)
-            plan = self.plans[0]
-            B = ops.multi_mode_dot(self.core, self.factors, skip=0)
-            Vm = B.reshape(B.shape[0], -1)
-            plan.set_factor(1, Vm)                                          # (factor 0's planes: installed by the core update)
-            keep = 0 not in fixed_modes
-            _, cost = plan.fused(0, 1, want_cost=True, keep_partials=keep)
+        if self.plans is None:
+            K = ops.multi_mode_dot(self.core, self.factors)
+            return ops.beta_divergence(self.T, K, beta)                     # ntd.py:694-696 (not normalised)
+        # beta_divergence(T, G x_n F_n, beta) without forming the reconstruction: the cost output of a pass over unfold(T, 0)
+        # with U = F_0, V = B_(0) = unfold(G x_{j > 0} F_j, 0) (any mode's unfolding gives the same number; mode 0 is used because
+        # the same pass, with the same operands, is the first factor update of the NEXT iteration: what it leaves serves it)
+        plan = self.plans[0]
+        B = ops.multi_mode_dot(self.core, self.factors, skip=0)
+        Vm = B.reshape(B.shape[0], -1)
+        keep = 0 not in fixed_modes
+        if beta == 2:
+            # half the direct residual ||unfold(T, 0) - F_0 B_(0)||^2 of one fused pass, whose cross product B_(0) unfold(T, 0)^T
+            # is the next mode-0 numerator
+            plan.set_factor(0, ops.transpose(self.factors[0]))
+            plan.set_factor(1, Vm)
+            if self._m0_num is None:
+                self._m0_num = torch.empty((plan.r, plan.m), dtype=torch.float32, device=self.T.device)
+            _, res = plan.fused(0, 0, out=self._m0_num)
+            self._m0_ready = keep
+            return ops.axpby(0.5, res, 0.0, res)                            # ntd.py:694-696 (not normalised)
+        if not keep:                                                        # a free mode 0 was installed by its update (mu_finish_rows)
+            plan.set_factor_rows(ops.transpose(self.factors[0]))
+        plan.set_operand(B, 1, Vm.shape[1])
+        if beta == 1:
+            _, cost = plan.fused(0, 1, want_cost=True, keep_partials=True)
             if keep:
                 ops.row_sums(Vm, out=self._m0_den)
-                self._m0_ready = True
-            return cost                                                     # ntd.py:694-696 (not normalised)
-        K = ops.multi_mode_dot(self.core, self.factors)
-        return ops.beta_divergence(self.T, K, beta)                         # ntd.py:694-696 (not normalised)
+        else:
+            cost = plan.fused_beta(0, beta, want_cost=True)
+        self._m0_ready = keep
+        return cost                                                         # ntd.py:694-696 (not normalised)
 
 
 def compute_ntd(tensor_in, ranks, core_in, factors_in, n_iter_max=100, tol=1e-6,

@@ -89,19 +89,39 @@ def _ones_contracted(factors):
     return dn.contiguous()
 
 
-def mu_tensorial_device(G, factors, T, beta, plan0=None):
+def gram(F):
+    """F^T F of a factor (I x r)."""
+    r = F.shape[1]
+    return ops.gemm(F, (1, r), F, (r, 1), r, r, F.shape[0])
+
+
+def mu_tensorial_device(G, factors, T, beta, plan=None):
     """Tucker-core multiplicative update on device tensors (mu.py:138-159).
 
-    plan0 (beta = 1, fp32, ranks <= 64): the NMF plan of unfold(T, 0).  The first contraction of the numerator,
-    F_0^T unfold(T / K, 0), is then the V-side numerator of one fused tcgen05 pass over the planes of that unfolding
-    with U = F_0 and V = unfold(G x_{j>0} F_j, 0): neither K nor T / K is ever written."""
-    if beta == 1 and plan0 is not None:
-        B0 = ops.multi_mode_dot(G, factors, skip=0)                         # r_0 x I_1 x ... (K = F_0 x_0 B0, mu.py:141)
-        plan0.set_factor(0, ops.transpose(factors[0]))
-        plan0.set_factor(1, B0.reshape(B0.shape[0], -1))
-        P, _ = plan0.fused(1, 1, want_cost=False)                           # F_0^T unfold(T / K, 0): r_0 x (I_1 ...)
-        up = ops.multi_mode_dot(P.reshape(B0.shape), factors, skip=0, transpose=True)
-        dn = _ones_contracted(factors)
+    plan (fp32, ranks <= 64): the one-sided plan of unfold(T, 0)^T (rows: the columns of unfold(T, 0); contraction over I_0),
+    DeviceNTD.core_plan.  The one contraction that reads the whole tensor, over mode 0, then runs there and yields r_0 x (I_1 ...):
+    beta = 2, F_0^T unfold(T, 0) (cross product; the denominator is G x_n F_n^T F_n); any other beta, F_0^T unfold(K^(beta-2) T, 0)
+    and F_0^T unfold(K^(beta-1), 0) from one fused pass with U = unfold(G x_{j>0} F_j, 0)^T and V = F_0^T, so that neither K nor
+    the ratio tensors are ever written.  The remaining mode products act on tensors r_0 / I_0 the size of T."""
+    if plan is not None:
+        F0t = ops.transpose(factors[0])
+        shape = [G.shape[0]] + list(T.shape[1:])
+        if beta == 2:
+            up = ops.multi_mode_dot(plan.cross(0, F0t).reshape(shape), factors, skip=0, transpose=True)
+            dn = ops.multi_mode_dot(G, [gram(F) for F in factors])                                      # K x_n F_n^T
+        else:
+            B0 = ops.multi_mode_dot(G, factors, skip=0)                     # r_0 x I_1 x ... (K = F_0 x_0 B0, mu.py:141)
+            plan.set_factor_rows(B0.reshape(B0.shape[0], -1))
+            plan.set_operand(F0t, 1, F0t.shape[1])
+            del B0
+            if beta == 1:
+                P, _ = plan.fused(0, 1, want_cost=False)
+                dn = _ones_contracted(factors)
+            else:
+                plan.fused_beta(0, beta, want_cost=False)
+                P = plan.reduce(0)
+                dn = ops.multi_mode_dot(plan.reduce_den(0).reshape(shape), factors, skip=0, transpose=True)
+            up = ops.multi_mode_dot(P.reshape(shape), factors, skip=0, transpose=True)
         return ops.mu_apply(G.reshape(G.shape[0], -1), up.reshape(G.shape[0], -1), den_mat=dn.reshape(G.shape[0], -1),
                             gamma=gamma_beta(beta), floor=epsilon).reshape(G.shape)
     K = ops.multi_mode_dot(G, factors)                                     # mu.py:141
